@@ -3,7 +3,7 @@
 round trip, input GB/s, on the synthetic mixed CSV/log/binary corpus, chunk 4096, repo-native
 methods only.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--size-mib M]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--size-mib M] [--dump-outputs DIR]
 
 N = 1 : configs[1], 1 GiB on one B200.  N > 1 (torchrun): configs[3] -- every rank takes a contiguous
 4 GiB chunk-range shard of a 4 N GiB corpus (weak scaling; 32 GiB at 8 GPUs), compresses it, the 16-byte
@@ -313,6 +313,28 @@ def full_size_parity(args, engine, t_in, n, threads):
             "oracle": "C port, indexed match search (lz_fast), %d threads" % threads}
 
 
+DUMP_SEED = 0xA3BC0D00
+DUMP_MAX_ELEMS = 6 << 20  # per array: two float32 samples of this size plus the counters stay under 64 MB
+
+
+def dump_outputs(out_dir, body, decoded, res):
+    """write what the last timed step returned, as float32 / float64 .npy files: the compressed body, the decoded
+    output and the CompressResult counters.  An array longer than DUMP_MAX_ELEMS is written as the values at
+    DUMP_MAX_ELEMS sorted positions drawn uniformly with numpy's default_rng(DUMP_SEED) (with replacement), so two
+    runs whose arrays have the same length are sampled at the same positions."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("body", body), ("decoded", decoded)):
+        n = t.numel()
+        if n > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.default_rng(DUMP_SEED).integers(0, n, DUMP_MAX_ELEMS))
+            t = t[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float32))
+    counters = [res.body_len, res.n_chunks, res.first_raw, res.n_packages, res.payload_bytes] + list(res.usage)
+    np.save(os.path.join(out_dir, "compress_result.npy"), np.array(counters, dtype=np.float64))
+
+
 def bind_to_gpu_numa_node(index):
     """Pin this rank (and with it the first-touch placement of its pinned host buffers and the helper
     threads of the host package walk) to the CPUs of its GPU's NUMA node: with 8 ranks on one host the
@@ -446,7 +468,7 @@ def run_b200(args):
     with ClockSampler(local) as clocks:
         for s in range(args.steps):
             ev[3 * s].record()
-            compress()
+            g_body = compress()
             ev[3 * s + 1].record()
             decompress()
             ev[3 * s + 2].record()
@@ -463,6 +485,8 @@ def run_b200(args):
     if world > 1:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
     tc_m, td_m, tstep = tt.cpu().tolist()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, g_body if world > 1 else t_out[:res.body_len], t_dec, res)
 
     # e2e through the C-ABI host calls (pinned buffers)
     e2e_steps = max(1, args.steps)
@@ -661,7 +685,14 @@ def main():
     ap.add_argument("--no-full-parity", action="store_true", help="skip the CPU body of the whole shard (indexed oracle)")
     ap.add_argument("--traffic", type=float, default=None,
                     help="dram bytes per k_select launch from the committed ncu capture (profiles/)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's body, decoded output and counters as DIR/<name>.npy "
+                         "(float32 / float64, a seeded sample of arrays longer than %d elements)" % DUMP_MAX_ELEMS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":

@@ -91,9 +91,7 @@ _SIGS = {
     "ambc_last_timing": (C.c_int, [C.POINTER(C.c_float)]),
     "ambc_host_alloc": (C.c_void_p, [C.c_uint64]),
     "ambc_host_free": (None, [C.c_void_p]),
-    # test and experiment hooks (include/ambc.h, last section)
-    "ambc_set_lz_levels": (C.c_int, [C.c_void_p, C.c_int]),
-    "ambc_set_lz_coop_threshold": (C.c_int, [C.c_int]),
+    # test hooks (include/ambc.h, last section)
     "ambc_set_lz_force_buckets": (C.c_int, [C.c_int]),
     "ambc_set_walk_threads": (None, [C.c_uint64, C.c_uint]),
     "ambc_scan_state_bytes": (C.c_uint64, []),

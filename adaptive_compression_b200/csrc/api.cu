@@ -47,27 +47,9 @@ extern "C" int ambc_last_timing(float *ms4)
     return AMBC_OK;
 }
 
-int ambc_lz_levels_compress(const int *levels, int n);
-int ambc_lz_levels_codec(const int *levels, int n);
-// experiment knob (not part of include/ambc.h): n-gram levels of the Dictionary match search
-extern "C" int ambc_set_lz_levels(const int *levels, int n)
-{
-    if (ambc_lz_levels_compress(levels, n) || ambc_lz_levels_codec(levels, n))
-        return ambc_fail(AMBC_E_ARG, "ambc_set_lz_levels: need ascending levels starting at 3, each <= 16, at most 8");
-    return AMBC_OK;
-}
-
-int ambc_lz_coop_compress(int t);
-int ambc_lz_coop_codec(int t);
-extern "C" int ambc_set_lz_coop_threshold(int t) { return (ambc_lz_coop_compress(t) || ambc_lz_coop_codec(t)) ? AMBC_E_CUDA : AMBC_OK; }
-
-int ambc_lz_force_buckets_compress(int on);
 int ambc_lz_force_buckets_codec(int on);
-// test knob (not part of include/ambc.h): force the window-aware bucket search for every chunk size
-extern "C" int ambc_set_lz_force_buckets(int on)
-{
-    return (ambc_lz_force_buckets_compress(on) || ambc_lz_force_buckets_codec(on)) ? AMBC_E_CUDA : AMBC_OK;
-}
+// test knob: force the window-aware bucket search of the plug-in Dictionary encoder for every chunk size
+extern "C" int ambc_set_lz_force_buckets(int on) { return ambc_lz_force_buckets_codec(on) ? AMBC_E_CUDA : AMBC_OK; }
 
 // fold of the all-gathered placement records (see include/ambc.h; mirrors distributed.fold_placement)
 extern "C" int ambc_shard_place(const ambc_shard_rec *recs, uint32_t n_ranks, const uint64_t *first_byte, uint32_t chunk,

@@ -10,23 +10,6 @@
 #pragma once
 #include "common.cuh"
 
-// dev-only phase timeline (build with -DAMBC_PHASE_TIMING): thread 0 of every CTA adds the
-// clock64() delta since the previous mark to g_phase[id]
-#ifdef AMBC_PHASE_TIMING
-__device__ unsigned long long g_phase[32];
-__device__ __forceinline__ void phase_mark(long long &t, int id)
-{
-    if (threadIdx.x == 0) { long long now = clock64(); atomicAdd(&g_phase[id], (unsigned long long)(now - t)); t = now; }
-}
-#define PHASE_DECL long long ph_t = clock64();
-#define PHASE(id) phase_mark(ph_t, id)
-#define PHASE_SYNC(id) do { __syncthreads(); phase_mark(ph_t, id); } while (0)
-#else
-#define PHASE_DECL
-#define PHASE(id)
-#define PHASE_SYNC(id)
-#endif
-
 struct ChunkCtx {
     uint8_t *sd;       // chunk bytes, 16-byte aligned, followed by AMBC_PAD zero bytes
     int n;             // chunk length (<= AMBC_NMAX)
@@ -42,7 +25,7 @@ struct ChunkCtx {
     uint32_t *reach;   // token-start bitmap, ceil(n/32) words
     uint8_t *estart;   // per 32-block chain entry offset
     int *red;          // 32 ints of reduction scratch (8-byte aligned)
-    // names-based match search (lz_names.cuh), chunks of at most LZ2_NMAX bytes; T == nullptr: absent
+    // names-based match search (lz_names.cuh), chunks of at most LZ2_NMAX bytes
     uint32_t *T;       // LZ2_TSLOTS hash slots (32 KiB)
     uint16_t *nameA;   // LZ2_NMAX first-occurrence names (two buffers, alternating levels)
     uint16_t *nameB;
@@ -112,48 +95,6 @@ __device__ inline void chunkctx_carve(ChunkCtx &c, uint8_t *base, int N, int pca
     c.n = 0;
 }
 
-// Compact layout for the chunk kernel at N <= LZ2_NMAX, payload capacity N: everything that is
-// dead while the names search runs (trigram set / Huffman scratch / fallback-search counters X,
-// Huffman bit words `sorted`, the payload buffer, the bucket starts of the fallback search)
-// overlays the hash table and the two name buffers.
-__host__ __device__ inline size_t chunkctx_fast_smem_bytes(int N)
-{
-    size_t nb = (size_t)(N + 31) / 32;
-    return r16((size_t)N) + AMBC_PAD + LZ2_TSLOTS * 4 + 2 * LZ2_NMAX * 2 + LZ2_LBYTES
-           + r16((size_t)N) + r16(2 * (size_t)N) + 1024 + r16(nb * 4) * 2 + r16(nb) + 128 + AMBC_HTAB_BYTES;
-}
-__device__ inline void chunkctx_carve_fast(ChunkCtx &c, uint8_t *base, int N)
-{
-    size_t nb = (size_t)(N + 31) / 32;
-    uint8_t *p = base;
-    c.sd = p; p += r16((size_t)N) + AMBC_PAD;
-    c.T = (uint32_t *)p;
-    {   // overlays of the table + names region (48 KiB): X | sorted | pay | bstart
-        uint8_t *q = p;
-        c.X = q; q += AMBC_XBYTES + 64;
-        c.sorted = (uint16_t *)q; q += r16(2 * (size_t)(N + 2) > (size_t)N + 16 ? 2 * (size_t)(N + 2) : (size_t)N + 16);
-        c.pay = q; q += r16((size_t)N) + 16;
-        c.bstart = (uint16_t *)q;
-    }
-    p += LZ2_TSLOTS * 4;
-    c.nameA = (uint16_t *)p; p += LZ2_NMAX * 2;
-    c.nameB = (uint16_t *)p; p += LZ2_NMAX * 2;
-    c.L = p; p += LZ2_LBYTES;
-    c.mlen = p; p += r16((size_t)N);
-    c.mpos = (uint16_t *)p; p += r16(2 * (size_t)N);
-    c.hist = (uint32_t *)p; p += 1024;
-    c.bmask = (uint32_t *)p; p += r16(nb * 4);
-    c.reach = (uint32_t *)p; p += r16(nb * 4);
-    c.estart = p; p += r16(nb);
-    c.red = (int *)p; p += 128;
-    c.hcode = (uint32_t *)p; c.hlen = p + 1024;
-    c.pcap = N;
-    c.n = 0;
-}
-static_assert(AMBC_XBYTES + 64 + ((2 * (LZ2_NMAX + 2) + 15) & ~15) + LZ2_NMAX + 16 + 2 * (AMBC_NBUCKET + 1) <=
-                  LZ2_TSLOTS * 4 + 2 * LZ2_NMAX * 2,
-              "overlays must fit the table + names region");
-
 // Stage chunk [src, src+n) in c.sd and zero the pad.  Ends with __syncthreads().
 __device__ inline void chunk_load(ChunkCtx &c, const uint8_t *__restrict__ src, int n)
 {
@@ -196,7 +137,6 @@ __device__ inline void chunk_features(ChunkCtx &c, ChunkFeatures &f)
     for (int i = tid; i < 256; i += AMBC_BLOCK) c.hist[i] = 0;
     for (int i = tid; i < 2048 / 4; i += AMBC_BLOCK) ((uint4 *)tri)[i] = make_uint4(0, 0, 0, 0);
     __syncthreads();
-    PHASE_DECL
 
     // histogram (run-aggregated shared atomics) + run-boundary bitmap
     for (int s = tid; s < nsl; s += AMBC_BLOCK) {
@@ -220,7 +160,6 @@ __device__ inline void chunk_features(ChunkCtx &c, ChunkFeatures &f)
         c.bmask[s] = mask;
     }
 
-    PHASE_SYNC(21);
     // sampled gates: RLE (:165-180) and Delta (:651-667) share the sample positions
     int rep = 0, small = 0;
     if (n >= 4) {
@@ -232,7 +171,6 @@ __device__ inline void chunk_features(ChunkCtx &c, ChunkFeatures &f)
             small += (abs(x - y) < 32);
         }
     }
-    PHASE_SYNC(22);
     // distinct trigrams (:326-343)
     int ins = 0;
     if (n >= 100) {
@@ -248,7 +186,6 @@ __device__ inline void chunk_features(ChunkCtx &c, ChunkFeatures &f)
             }
         }
     }
-    PHASE_SYNC(23);
     // one block reduction for the three gate counters (also orders hist / bmask writes before the reads below)
     int *redx = (int *)(c.X + 8192); // 4 x AMBC_WARPS ints behind the trigram set
     {
@@ -262,7 +199,6 @@ __device__ inline void chunk_features(ChunkCtx &c, ChunkFeatures &f)
         __syncthreads();
     }
 
-    PHASE(24);
     // RLE pair count: a run of R bytes -> ceil(R/255) pairs (:95-109).  Only needed (and only
     // defined) when the RLE gate holds (:177-180), which is rare outside run-heavy data.
     int pairs = 0;
@@ -287,7 +223,6 @@ __device__ inline void chunk_features(ChunkCtx &c, ChunkFeatures &f)
             }
         }
     }
-    PHASE(25);
 
     // entropy (:566-574) in fp32; the caller resolves near-threshold cases in fp64, in the reference's order
     float hsum = 0.0f;
@@ -317,7 +252,6 @@ __device__ inline void chunk_features(ChunkCtx &c, ChunkFeatures &f)
         f.H = rh;
         __syncthreads();
     }
-    PHASE(26);
 }
 
 // first-occurrence order of the byte values (Counter insertion order, :368-370 / :566).
@@ -475,29 +409,11 @@ __device__ inline int chunk_delta_encode(ChunkCtx &c)
 // LZ_LEVELS[k+1]-gram, so its longest match is at most LZ_LEVELS[k+1]-1 bytes and the ascending
 // scan can stop at the first candidate of that length.  Any level set starting at 3 is exact;
 // the set only changes how many candidates are visited.
-// (tunable at run time for experiments: ambc_set_lz_levels / env AMBC_LZ_LEVELS)
 #define LZ_MAX_LEVELS 8
 static __device__ __constant__ int LZ_LEVELS[LZ_MAX_LEVELS] = {3, 4, 6, 10, 0, 0, 0, 0};
 static __device__ __constant__ int LZ_NLEVELS = 4;
 static __device__ __constant__ int LZ_COOP_T = 24; // buckets with more candidates are scanned by a whole warp
 static __device__ __constant__ int LZ_FORCE_BUCKETS = 0; // test knob: always use the bucket search
-// per-translation-unit setter (the constants are TU-local without relocatable device code)
-static inline int lz_levels_upload(const int *levels, int n)
-{
-    int buf[LZ_MAX_LEVELS] = {0};
-    if (n < 1 || n > LZ_MAX_LEVELS || levels[0] != 3) return -1;
-    for (int i = 0; i < n; i++) {
-        if (levels[i] > 16 || (i && levels[i] <= levels[i - 1])) return -1;
-        buf[i] = levels[i];
-    }
-    if (cudaMemcpyToSymbol(LZ_LEVELS, buf, sizeof buf) != cudaSuccess) return -1;
-    if (cudaMemcpyToSymbol(LZ_NLEVELS, &n, sizeof n) != cudaSuccess) return -1;
-    return 0;
-}
-static inline int lz_coop_upload(int t)
-{
-    return cudaMemcpyToSymbol(LZ_COOP_T, &t, sizeof t) == cudaSuccess ? 0 : -1;
-}
 static inline int lz_force_buckets_upload(int on)
 {
     return cudaMemcpyToSymbol(LZ_FORCE_BUCKETS, &on, sizeof on) == cudaSuccess ? 0 : -1;
@@ -522,15 +438,6 @@ __device__ __forceinline__ uint32_t lz_hash_l(const uint8_t *s, int L)
         w1 = w2; k++; rem -= 4;
     }
     return (h ^ (h >> 13)) * 3266489917u >> (32 - AMBC_HB);
-}
-
-// Lower bound of the Dictionary payload for n bytes: the first token is a literal, every
-// other token covers at most 32 bytes (lookahead_size) for at least 2 bytes of output.
-__host__ __device__ inline int lz_lower_bound(int n)
-{
-    if (n <= 0) return 0;
-    int r = (n - 1) % 32;
-    return 2 + 4 * ((n - 1) / 32) + (2 * r < 4 ? 2 * r : 4);
 }
 
 // Stable bucket sort of positions [0, P) by the hash of their L-gram: c.sorted (ascending
@@ -762,26 +669,20 @@ __device__ __forceinline__ void lz_zero_mlen(ChunkCtx &c)
     __syncthreads();
 }
 
-// Payload -> c.pay (as far as pcap allows).  Returns the exact payload length, or LZ_ABORTED when the
-// match search proved early that the length cannot stay below `cutoff` (the caller already holds a
-// payload that short).  Collective.
-#define LZ_ABORTED 0x7fffffff
-__device__ inline int chunk_lz_encode(ChunkCtx &c, int cutoff = LZ_ABORTED)
+// Payload -> c.pay (as far as pcap allows).  Returns the exact payload length.  Collective.
+__device__ inline int chunk_lz_encode(ChunkCtx &c)
 {
     const int n = c.n, tid = threadIdx.x;
     lz_zero_mlen(c);
     bool done = false;
-    if (c.T && n <= LZ2_NMAX && !LZ_FORCE_BUCKETS) {
-        const int r = lz2_match_all(c, cutoff);
-        if (r == 2) return LZ_ABORTED;
-        done = r == 0;
+    if (n <= LZ2_NMAX && !LZ_FORCE_BUCKETS) {
+        done = lz2_match_all(c) == 0;
         if (!done) lz_zero_mlen(c); // a table overflowed (pathological key skew): redo with the bucket search
     }
     if (!done) lz_match_all_buckets(c);
     __syncthreads();
 
     // ---- token chain: pos -> pos + (len>2 ? len : 1) (:211-232), resolved per 32-block ---
-    PHASE_DECL
     const int nb = (n + 31) >> 5;
     uint8_t *fexit = c.X; // fexit[q * nb + b]: where a chain entering block b at offset q leaves it
     for (int b = tid; b < nb; b += AMBC_BLOCK) {
@@ -799,7 +700,6 @@ __device__ inline int chunk_lz_encode(ChunkCtx &c, int cutoff = LZ_ABORTED)
         }
     }
     __syncthreads();
-    PHASE(27);
     {   // entry offset of every block on the chain from position 0: groups of 32 blocks are composed
         // for all 32 entry offsets at once (one warp per group, lane = entry offset), then the few
         // groups are chained and every group is walked from its true entry
@@ -832,7 +732,6 @@ __device__ inline int chunk_lz_encode(ChunkCtx &c, int cutoff = LZ_ABORTED)
         }
     }
     __syncthreads();
-    PHASE(28);
     // per block: token-start mask, match mask, payload bytes; then every position emits its own token
     uint32_t *mmask = (uint32_t *)(c.X + 8192);        // behind fexit (32 * nb <= 8 KiB)
     uint32_t *boff = (uint32_t *)(c.X + 8192 + 1024);  // payload offset of the block's first token
@@ -854,7 +753,6 @@ __device__ inline int chunk_lz_encode(ChunkCtx &c, int cutoff = LZ_ABORTED)
     const int off0 = block_excl_scan(tbytes, c.red, &total);
     for (int b = tid * bpt; b < min(nb, (tid + 1) * bpt); b++) boff[b] += (uint32_t)off0;
     __syncthreads();
-    PHASE(29);
     uint16_t *pay16 = (uint16_t *)c.pay; // token offsets are even
     for (int p = tid; p < n; p += AMBC_BLOCK) {
         const int b = p >> 5;
@@ -872,7 +770,6 @@ __device__ inline int chunk_lz_encode(ChunkCtx &c, int cutoff = LZ_ABORTED)
         }
     }
     __syncthreads();
-    PHASE(30);
     return total;
 }
 
@@ -917,7 +814,6 @@ __device__ inline HuffScratch huff_scratch(ChunkCtx &c)
 __device__ inline int chunk_huff_build(ChunkCtx &c, HuffScratch &h, int K)
 {
     const int tid = threadIdx.x;
-    PHASE_DECL
     for (int b = tid; b < 256; b += AMBC_BLOCK) {
         uint32_t cnt = c.hist[b];
         h.key[b] = cnt ? ((cnt << 8) | (uint32_t)b) : 0xFFFFFFFFu;
@@ -929,7 +825,6 @@ __device__ inline int chunk_huff_build(ChunkCtx &c, HuffScratch &h, int K)
     rank_present(h.key, (uint32_t *)(c.X + 3072), c.X + 8448, (int *)(c.X + 8704),
                  [&](int r, int sym, uint32_t k) { h.nodeW[r] = k; h.leafsym[r] = (uint8_t)sym; });
     __syncthreads();
-    PHASE(31);
     if (tid == 0) {
         // two-queue merge, both queue heads cached in registers: one reload per pick.  Weights stay
         // below 2^24 (chunks of at most 8192 bytes), leaders are byte values.
@@ -963,7 +858,6 @@ __device__ inline int chunk_huff_build(ChunkCtx &c, HuffScratch &h, int K)
         }
     }
     __syncthreads();
-    PHASE(0);
     const int root = 2 * K - 2;
     int bits = 0;
     for (int j = tid; j < K; j += AMBC_BLOCK) {
@@ -987,9 +881,7 @@ __device__ inline int chunk_huff_build(ChunkCtx &c, HuffScratch &h, int K)
 __device__ inline int chunk_huff_emit(ChunkCtx &c, HuffScratch &h, int K, int total_bits)
 {
     const int n = c.n, tid = threadIdx.x;
-    PHASE_DECL
     chunk_first_order(c, h.firstpos, h.order);
-    PHASE(14);
     const int hdr = 1 + 5 * K + 4;
     const int nbytes = (total_bits + 7) >> 3;
     if (tid == 0 && c.pcap >= 1) c.pay[0] = (uint8_t)K;
@@ -1019,7 +911,6 @@ __device__ inline int chunk_huff_emit(ChunkCtx &c, HuffScratch &h, int K, int to
     }
     int tot;
     int g = block_excl_scan(mybits, c.red, &tot); // includes the barrier after zeroing bw
-    PHASE(15);
     {
         int w = g >> 5, used = g & 31;
         uint32_t cur = 0;
@@ -1052,11 +943,9 @@ __device__ inline int chunk_huff_emit(ChunkCtx &c, HuffScratch &h, int K, int to
         if (used && w < wcap) atomicOr(&bw[w], cur);
     }
     __syncthreads();
-    PHASE(16);
     for (int k = tid; k < nbytes; k += AMBC_BLOCK) {
         if (hdr + k < c.pcap) c.pay[hdr + k] = (uint8_t)(bw[k >> 2] >> (24 - 8 * (k & 3)));
     }
     __syncthreads();
-    PHASE(17);
     return hdr + nbytes;
 }

@@ -127,6 +127,4 @@ extern "C" int ambc_should_use_batch(const void *in_dev, const uint64_t *in_off_
     return AMBC_OK;
 }
 
-int ambc_lz_levels_codec(const int *levels, int n) { return lz_levels_upload(levels, n); }
-int ambc_lz_coop_codec(int t) { return lz_coop_upload(t); }
 int ambc_lz_force_buckets_codec(int on) { return lz_force_buckets_upload(on); }

@@ -1,198 +1,23 @@
-// compress.cu -- chunk trial / select / pack kernels and the ambc_compress_* entry points.
+// compress.cu -- chunk select / scan / pack kernels and the ambc_compress_* entry points.
 //
 // Replaces AdaptiveCompressor._adaptive_compress and its helpers
-// (adaptive_compressor.py:363-394, 537-590, 595-700) in fixed-candidate mode.
+// (adaptive_compressor.py:363-394, 537-590, 595-700).
 //
-//   k_select   one CTA per grid chunk: stage 4 KiB in shared memory, evaluate the gates,
-//              compute every enabled candidate's exact size, pick the argmin in list order
-//              with the benefit test len+overhead < n, encode the winner into its slot.
-//   k_sizes / k_scan_blocks / k_offsets
-//              exclusive scan of package sizes with the "rest of file raw" rule: everything
-//              from the first chunk without a winner onward is ONE raw package.
-//   k_pack     one CTA per chunk: 18-byte package header + payload to the final offset.
-#define AMBC_BLOCK 512 // encoder CTAs: 16 warps per chunk, 2 CTAs per SM (100 KB of shared memory each)
+//   k_select_fast      one CTA per grid chunk (select_fast.cuh): gates, the exact size of every enabled
+//                      candidate, the argmin in list order with the benefit test len+overhead < n, the
+//                      winner's payload into its slot.
+//   k_sizes / k_scan_tiles / k_offsets
+//                      exclusive scan of package sizes with the "rest of file raw" rule: everything
+//                      from the first chunk without a winner onward is ONE raw package.
+//   k_pack             one CTA per chunk: 18-byte package header + payload to the final offset.
+//   k_dynamic_walk     multi-candidate mode: the chain of chosen chunk sizes, walked segment by segment;
+//                      k_select_span_fast / k_pack_span then encode and frame the chosen chunks.
 #include "ambc_internal.h"
 #include <vector>
-#include "chunk_codec.cuh"
 #include "select_fast.cuh"
-#include <cstdlib>
 
 
-// per-chunk decision ------------------------------------------------------------------------
-struct SelectOut { int type; int len; };
-
-// size-range eligibility (adaptive_compressor.py:114-127, tested on the clamped size :565-567)
-__device__ __forceinline__ bool eligible(int id, int n)
-{
-    switch (id) {
-    case 1: return n >= 32 && n <= 4096;
-    case 2: return n >= 128 && n <= 8192;
-    case 3: return n >= 32 && n <= 8192;
-    case 4: return n >= 32 && n <= 4096;
-    }
-    return false;
-}
-
-// Evaluate one chunk already staged in c; leaves the winner's payload in c.pay.
-__device__ SelectOut select_chunk(ChunkCtx &c, uint32_t mask, int ovh, unsigned int *trial = nullptr)
-{
-    const int n = c.n;
-    ChunkFeatures f;
-    PHASE_DECL
-    chunk_features(c, f);
-    PHASE(1);
-    HuffScratch hs = huff_scratch(c);
-
-    // gates (compression_methods.py:154-180, 315-343, 551-574)
-    // (the fp64 quotients rep / (s - 1) > 0.3 and distinct / s < 0.8 as exact integer compares: the
-    // operands are below 1000, so a quotient that is not exactly 3/10 or 8/10 is at least 1e-4 away
-    // from it, and the exact ones round to the very doubles the literals denote)
-    bool rle_ok = (mask & 2u) && eligible(1, n) && n >= 4 && 10 * f.rep > 3 * (min(1000, n) - 1);
-    bool lz_ok = (mask & 4u) && eligible(2, n) && n >= 100 && 10 * f.distinct3 < 8 * min(1000, n);
-    bool hf_ok = (mask & 8u) && eligible(3, n) && n >= 100 && f.K >= 2 && f.K <= 255;
-    if (hf_ok) {
-        if (fabsf(f.H - 7.0f) < 0.02f) { // near the threshold: fp64, in the reference's summation order (:566-574)
-            chunk_first_order(c, hs.firstpos, hs.order);
-            hf_ok = chunk_entropy_ordered(c, f.K, hs.order) < 7.0;
-        } else hf_ok = f.H < 7.0f;
-    }
-    // Delta (id 4) always produces n bytes, so (n + overhead)/n > 1 never wins (:574-577).
-
-    // The reference tries the methods in id order and keeps the first strictly smaller payload (:575).
-    // The order of evaluation below differs, the outcome does not: a method's trial is skipped or cut
-    // short only when its payload provably cannot end up as the winner.
-    int best_type = 255, best_len = 0x7fffffff;
-    if (rle_ok) {
-        int len = 2 * f.rle_pairs;
-        if (len + ovh < n) { best_type = 1; best_len = len; }
-    }
-    // Huffman lower bound from the entropy: bits >= max(n, n*H)
-    int hf_lb = 0x7fffffff;
-    // (f.H is within 3e-4 of the entropy: 0.002 and the 0.01 keep the bound below n * H whatever fp32 rounds to)
-    if (hf_ok) hf_lb = 1 + 5 * f.K + 4 + (int)ceilf(fmaxf((float)n, (float)n * (f.H - 0.002f) - 0.01f) * 0.125f);
-    // Huffman first when the Dictionary method looks weak (many distinct trigrams): its size then cuts
-    // the match search short (lz2_match_all).  Its code table survives the search in c.hcode / c.hlen.
-    // Chunks above LZ2_NMAX bytes always go Huffman first: their Dictionary trial is the window-aware
-    // bucket search, twenty times the cost of a prefix trial with the names search (below).
-    const bool big = n > LZ2_NMAX;
-    const bool hf_first = hf_ok && lz_ok && (big || 100 * f.distinct3 >= 34 * min(1000, n));
-    const bool lz_weak = !big && 100 * f.distinct3 >= 43 * min(1000, n);
-    int hf_len = 0x7fffffff, hf_bits = 0; // hf_len: built, and a candidate against RLE
-    if (hf_first && hf_lb < best_len && hf_lb + ovh < n) {
-        hf_bits = chunk_huff_build(c, hs, f.K);
-        const int len = 1 + 5 * f.K + 4 + ((hf_bits + 7) >> 3);
-        if (len < best_len && len + ovh < n) hf_len = len;
-    }
-    if (lz_ok) {
-        // a Dictionary payload can never be shorter than lz_lower_bound(n): skip the trial when it cannot
-        // win.  It ends up as the winner only if it is < the RLE payload and <= the Huffman payload.
-        const int cutoff = hf_len == 0x7fffffff ? best_len : min(best_len, hf_len + 1);
-        int lb = lz_lower_bound(n);
-        if (lb < cutoff && lb + ovh < n) {
-            PHASE(10);
-            // Prefix trial (a gamble on speed, never on the outcome): with a Huffman payload in hand and a
-            // fair share of distinct trigrams the Dictionary method usually loses clearly.  The exact parse
-            // of the first 5/8 of the chunk (positions below n1 see the same 32-byte look-ahead as in the
-            // whole chunk, so their tokens are the real ones) then already costs more than the cutoff:
-            // tokens starting below n1 cost at least lenp - 62 (the prefix parse may end with <= 31 bytes
-            // of tokens starting at or after n1, <= 2 payload bytes per byte), and the n - np bytes behind
-            // the prefix need at least 4 bytes per 32.  When the bound does not reach the cutoff the whole
-            // chunk is parsed as usual; `trial` counts attempts / aborts per launch and switches the gamble
-            // off where it keeps failing.
-            bool aborted = false;
-            if (hf_first && !lz_weak && hf_len != 0x7fffffff && n >= 2048 && (trial || big) && c.T) {
-                // one thread reads the counters (other CTAs update them all the time): the whole block must
-                // take the same branch, the calls below are collective.  Big chunks always try: the prefix
-                // (the first LZ2_NMAX - 1 bytes, all inside the window of every position) costs a twentieth
-                // of their bucket search.
-                if (threadIdx.x == 0) {
-                    int go = 1;
-                    if (!big) {
-                        const unsigned int att = ((volatile unsigned int *)trial)[0], hit = ((volatile unsigned int *)trial)[1];
-                        go = (att < 64u || 4u * hit >= 3u * att) ? 1 : 0;
-                    }
-                    c.red[25] = go;
-                }
-                __syncthreads();
-                const bool go = c.red[25] != 0;
-                if (go) {
-                    const int np = big ? LZ2_NMAX - 1 : ((5 * n / 8) & ~31) + 31;
-                    c.n = np;
-                    const int lenp = chunk_lz_encode(c);
-                    c.n = n;
-                    const int r = n - np;
-                    aborted = lenp - 62 + 4 * (r >> 5) + min(4, 2 * (r & 31)) >= cutoff;
-                    if (threadIdx.x == 0 && !big) {
-                        atomicAdd(&trial[0], 1u);
-                        if (aborted) atomicAdd(&trial[1], 1u);
-                    }
-                }
-            }
-            if (!aborted) {
-                int len = chunk_lz_encode(c, (hf_first && lz_weak) ? cutoff : LZ_ABORTED);
-                PHASE(11);
-                if (len < best_len && len + ovh < n) { best_type = 2; best_len = len; }
-            }
-        }
-    }
-    if (hf_first) {
-        if (hf_len < best_len) {
-            best_type = 3; best_len = hf_len;
-            chunk_huff_emit(c, hs, f.K, hf_bits);
-        }
-    } else if (hf_ok) {
-        if (hf_lb < best_len && hf_lb + ovh < n) {
-            int bits = chunk_huff_build(c, hs, f.K);
-            int len = 1 + 5 * f.K + 4 + ((bits + 7) >> 3);
-            if (len < best_len && len + ovh < n) {
-                best_type = 3; best_len = len;
-                chunk_huff_emit(c, hs, f.K, bits);
-            }
-        }
-    }
-    PHASE(12);
-    if (best_type == 1) chunk_rle_encode(c);
-    PHASE(13);
-    SelectOut o;
-    o.type = best_type;
-    o.len = best_type == 255 ? n : best_len;
-    return o;
-}
-
-#ifndef KSEL_MINB
-#define KSEL_MINB 2
-#endif
-__global__ void __launch_bounds__(AMBC_BLOCK, KSEL_MINB)
-k_select(const uint8_t *__restrict__ in, uint64_t total, uint32_t N, uint32_t mask, uint32_t ovh,
-         uint8_t *__restrict__ slots, uint64_t slot_stride, uint8_t *__restrict__ type,
-         uint32_t *__restrict__ comp, unsigned long long *first_raw, uint64_t chunk_begin, uint64_t n_chunks,
-         unsigned int *trial)
-{
-    extern __shared__ uint4 smem4[];
-    ChunkCtx c;
-    if (N <= LZ2_NMAX) chunkctx_carve_fast(c, (uint8_t *)smem4, (int)N);
-    else chunkctx_carve(c, (uint8_t *)smem4, (int)N, (int)N);
-    for (uint64_t i = chunk_begin + blockIdx.x; i < n_chunks; i += gridDim.x) {
-        uint64_t off = i * (uint64_t)N;
-        int n = (int)min((uint64_t)N, total - off);
-        chunk_load(c, in + off, n);
-        SelectOut o = select_chunk(c, mask, (int)ovh, trial);
-        __syncthreads();
-        if (o.type != 255) {
-            uint8_t *dst = slots + i * slot_stride; // 16-byte aligned
-            int nv = (o.len + 15) >> 4;
-            for (int k = threadIdx.x; k < nv; k += AMBC_BLOCK) ((uint4 *)dst)[k] = ((const uint4 *)c.pay)[k];
-        }
-        if (threadIdx.x == 0) {
-            type[i] = (uint8_t)o.type;
-            comp[i] = (uint32_t)o.len;
-            if (o.type == 255) atomicMin(first_raw, (unsigned long long)i);
-        }
-        __syncthreads();
-    }
-}
-
-// round-2 kernel (select_fast.cuh): 128 threads and ~38 KB of shared memory per chunk, five CTAs per SM
+// select_fast.cuh: 128 threads and ~38 KB of shared memory per chunk, five CTAs per SM
 template <int NMAX>
 __global__ void __launch_bounds__(SF_T, NMAX <= 4096 ? 6 : 3)
 k_select_fast(const uint8_t *__restrict__ in, uint64_t total, uint32_t N, uint32_t mask, uint32_t ovh,
@@ -235,16 +60,8 @@ k_select_fast(const uint8_t *__restrict__ in, uint64_t total, uint32_t N, uint32
         __syncthreads();
     }
 }
-// dev knob: AMBC_SELECT=old keeps the round-1 kernel (A/B timing)
-static bool use_fast_select(uint32_t chunk)
-{
-    static int mode = -1;
-    if (mode < 0) { const char *e = getenv("AMBC_SELECT"); mode = (e && !strcmp(e, "old")) ? 0 : 1; }
-    return mode == 1 && chunk <= AMBC_NMAX;
-}
 
-// span mode (multi-candidate path, see k_select_span below) with the round-2 chunk code
-struct ChunkSpan;
+// span mode (multi-candidate path, see the span section below): chunks given by position and size
 template <int NMAX>
 __global__ void __launch_bounds__(SF_T, NMAX <= 4096 ? 6 : 3)
 k_select_span_fast(const uint8_t *__restrict__ in, uint64_t total, uint32_t N, uint32_t mask, uint32_t ovh, uint32_t stride,
@@ -253,6 +70,7 @@ k_select_span_fast(const uint8_t *__restrict__ in, uint64_t total, uint32_t N, u
 {
     // list == nullptr: item i = [i * stride, i * stride + min(N, total - i * stride)), no payload kept;
     // else item i = (pos, size) = (list[2 i], low half of list[2 i + 1]) and its payload goes to slots + pos
+    // (payloads are shorter than their chunks, so the chunk's own offset is a collision-free slot)
     extern __shared__ uint4 smem4[];
     SfCtx<NMAX> c;
     sf_carve<NMAX>(c, (uint8_t *)smem4);
@@ -292,7 +110,6 @@ struct ScanState {
     unsigned long long payload_bytes;
     unsigned long long usage[5];
     unsigned long long carry;      // body bytes before the chunks not yet scanned (piece-wise runs)
-    unsigned int trial[2];         // prefix trials of k_select in this run: attempts, aborts (speed heuristic only)
 };
 
 __device__ __forceinline__ uint64_t pkg_size(uint64_t i, const uint8_t *type, const uint32_t *comp, uint32_t N,
@@ -496,68 +313,23 @@ k_pack(const uint8_t *__restrict__ in, uint64_t total, uint32_t N, const uint8_t
 }
 
 // ---- span mode: chunks given by (position, size) instead of the fixed grid ---------------------
-// Used by the multi-candidate ("dynamic chunk size") path, adaptive_compressor.py:537-590: first as a
-// trial at every stride-aligned position for one candidate size (sizes only), then on the chosen
-// chunk chain (payloads).  Separate kernels so that the fixed-grid hot path stays untouched.
+// Used by the multi-candidate ("dynamic chunk size") path, adaptive_compressor.py:537-590, on the chosen
+// chunk chain.  Separate kernels so that the fixed-grid hot path stays untouched.
 struct ChunkSpan { unsigned long long pos; uint32_t size; uint32_t pad; };
 
-template <int MINB> // 2: sizes up to LZ2_NMAX (two CTAs per SM like k_select), 1: larger chunks
-__global__ void __launch_bounds__(AMBC_BLOCK, MINB)
-k_select_span(const uint8_t *__restrict__ in, uint64_t total, uint32_t N, uint32_t mask, uint32_t ovh,
-              uint32_t stride, const ChunkSpan *__restrict__ list, uint8_t *__restrict__ slots,
-              uint8_t *__restrict__ type, uint32_t *__restrict__ comp, uint64_t n_items)
-{
-    // list == nullptr: item i = [i * stride, i * stride + min(N, total - i * stride)), no payload kept;
-    // else item i = list[i] and its payload goes to slots + list[i].pos (payloads are shorter than
-    // their chunks, so the chunk's own offset is a collision-free slot)
-    extern __shared__ uint4 smem4[];
-    ChunkCtx c;
-    if (N <= LZ2_NMAX) chunkctx_carve_fast(c, (uint8_t *)smem4, (int)N);
-    else chunkctx_carve(c, (uint8_t *)smem4, (int)N, (int)N);
-    for (uint64_t i = blockIdx.x; i < n_items; i += gridDim.x) {
-        uint64_t off;
-        int n;
-        if (list) { off = list[i].pos; n = (int)list[i].size; }
-        else { off = i * (uint64_t)stride; n = (int)min((uint64_t)N, total - off); }
-        chunk_load(c, in + off, n);
-        SelectOut o = select_chunk(c, mask, (int)ovh);
-        __syncthreads();
-        if (slots && o.type != 255) {
-            uint8_t *dst = slots + off;
-            if ((((uintptr_t)dst) & 15) == 0) {
-                int nv = (o.len + 15) >> 4;
-                for (int k = threadIdx.x; k < nv; k += AMBC_BLOCK) ((uint4 *)dst)[k] = ((const uint4 *)c.pay)[k];
-            } else {
-                for (int k = threadIdx.x; k < o.len; k += AMBC_BLOCK) dst[k] = c.pay[k];
-            }
-        }
-        if (threadIdx.x == 0) {
-            type[i] = (uint8_t)o.type;
-            comp[i] = (uint32_t)o.len;
-        }
-        __syncthreads();
-    }
-}
-
-static int launch_select_span(unsigned grid, size_t smem, cudaStream_t stream, const uint8_t *in, uint64_t total, uint32_t N,
+static int launch_select_span(unsigned grid, cudaStream_t stream, const uint8_t *in, uint64_t total, uint32_t N,
                               uint32_t mask, uint32_t ovh, uint32_t stride, const ChunkSpan *list, uint8_t *slots,
                               uint8_t *type, uint32_t *comp, uint64_t n_items)
 {
     static_assert(sizeof(ChunkSpan) == 16, "k_select_span_fast reads spans as two 64-bit words");
-    if (use_fast_select(N) && N <= 4096) {
+    if (N <= 4096) {
         CUDA_TRY(cudaFuncSetAttribute(k_select_span_fast<4096>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SfCfg<4096>::SMEM));
         k_select_span_fast<4096><<<grid, SF_T, SfCfg<4096>::SMEM, stream>>>(in, total, N, mask, ovh, stride, (const unsigned long long *)list,
                                                                             slots, type, comp, n_items);
-    } else if (use_fast_select(N)) {
+    } else {
         CUDA_TRY(cudaFuncSetAttribute(k_select_span_fast<8192>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SfCfg<8192>::SMEM));
         k_select_span_fast<8192><<<grid, SF_T, SfCfg<8192>::SMEM, stream>>>(in, total, N, mask, ovh, stride, (const unsigned long long *)list,
                                                                             slots, type, comp, n_items);
-    } else if (N <= LZ2_NMAX) {
-        CUDA_TRY(cudaFuncSetAttribute(k_select_span<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_select_span<2><<<grid, AMBC_BLOCK, smem, stream>>>(in, total, N, mask, ovh, stride, list, slots, type, comp, n_items);
-    } else {
-        CUDA_TRY(cudaFuncSetAttribute(k_select_span<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_select_span<1><<<grid, AMBC_BLOCK, smem, stream>>>(in, total, N, mask, ovh, stride, list, slots, type, comp, n_items);
     }
     ambc_count_launch();
     CUDA_TRY(cudaGetLastError());
@@ -696,9 +468,7 @@ int ambc_compress_dev_impl(const void *in_dev, uint64_t n, uint32_t chunk, uint3
     unsigned grid_chunks = (unsigned)min<uint64_t>(L.n_chunks, 0x7fffffffull);
 
     if (native) {
-        size_t smem = chunk <= LZ2_NMAX ? chunkctx_fast_smem_bytes((int)chunk) : chunkctx_smem_bytes((int)chunk, (int)chunk);
         size_t psmem = 32 + (((size_t)chunk + 15) & ~(size_t)15) + 32;
-        CUDA_TRY(cudaFuncSetAttribute(k_select, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         CUDA_TRY(cudaFuncSetAttribute(k_pack, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem));
         CUDA_TRY(cudaFuncSetAttribute(k_select_fast<4096>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SfCfg<4096>::SMEM));
         CUDA_TRY(cudaFuncSetAttribute(k_select_fast<8192>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SfCfg<8192>::SMEM));
@@ -721,17 +491,14 @@ int ambc_compress_dev_impl(const void *in_dev, uint64_t n, uint32_t chunk, uint3
             const unsigned gt = (unsigned)((c1 - c0 + SCAN_TILE - 1) / SCAN_TILE);
             if (pieces) CUDA_TRY(cudaStreamWaitEvent(stream, piece_ready[k], 0));
             if (k == 0) ambc_timing_mark(0, stream);
-            if (use_fast_select(chunk) && chunk <= 4096)
+            if (chunk <= 4096)
                 k_select_fast<4096><<<gch, SF_T, SfCfg<4096>::SMEM, stream>>>((const uint8_t *)in_dev, n, chunk, method_mask, ovh,
                                                                              W + L.slots, L.slot_stride, type, comp,
                                                                              &st->first_raw, c0, c1, (flags & AMBC_F_PER_CHUNK_RAW) ? 0u : 1u);
-            else if (use_fast_select(chunk))
+            else
                 k_select_fast<8192><<<gch, SF_T, SfCfg<8192>::SMEM, stream>>>((const uint8_t *)in_dev, n, chunk, method_mask, ovh,
                                                                              W + L.slots, L.slot_stride, type, comp,
                                                                              &st->first_raw, c0, c1, (flags & AMBC_F_PER_CHUNK_RAW) ? 0u : 1u);
-            else
-                k_select<<<gch, AMBC_BLOCK, smem, stream>>>((const uint8_t *)in_dev, n, chunk, method_mask, ovh, W + L.slots,
-                                                            L.slot_stride, type, comp, &st->first_raw, c0, c1, st->trial);
             ambc_count_launch();
             if (last) ambc_timing_mark(1, stream);
             // scan + pack of piece k run on their own stream so that k_select of piece k + 1 follows at once
@@ -840,32 +607,24 @@ extern "C" int ambc_sf_phase_read(unsigned long long *out48, int reset)
     if (reset) { unsigned long long z[48] = {0}; cudaMemcpyToSymbol(g_sf, z, sizeof z); }
     return 0;
 }
-extern "C" int ambc_phase_read(unsigned long long *out32, int reset)
-{
-    cudaMemcpyFromSymbol(out32, g_phase, sizeof(unsigned long long) * 32);
-    if (reset) { unsigned long long z[32] = {0}; cudaMemcpyToSymbol(g_phase, z, sizeof z); }
-    return 0;
-}
 #endif
 // ---- multi-candidate ("dynamic chunk size") mode ------------------------------------------------
 // adaptive_compressor.py:537-590 with several CHUNK_SIZE_CANDIDATES: at every position each candidate
 // size (clamped to the remaining bytes) is tried, the smallest ratio (len + overhead) / size wins,
 // larger candidates win ties; no winner -> the rest of the file is one raw package.
-// Every reachable position is a multiple of g = gcd(candidates), so each distinct size min(cand, 8192)
-// is tried at every multiple of g on the GPU (sizes only), the chain is resolved on the host (it is a
-// serial walk over <= n / g table entries), and the chosen chunks are encoded and framed in span mode.
+// Every reachable position is a multiple of g = gcd(candidates).  The chain is walked on the GPU
+// (k_dynamic_walk, below), and the chosen chunks are encoded and framed in span mode.
 static uint64_t gcd64(uint64_t a, uint64_t b) { while (b) { uint64_t t = a % b; a = b; b = t; } return a; }
 
 // ---- the chain of the multi-candidate mode on the GPU ---------------------------------------------------------
 // The reference walks the file once: at every position it tries every candidate size and moves on by the winner's
 // size (adaptive_compressor.py:363-394, 537-590).  Only the positions on that chain matter, about one in six of
-// the multiples of g -- round 1 tried every size at EVERY multiple of g and walked the tables on the host.  Here
-// the file is cut into segments of DYN_SEGU * g bytes; one CTA walks the chain of a segment from its first byte,
-// evaluating the candidates at the positions it actually visits (speculative: the true chain may enter the segment
-// elsewhere).  Chains that enter a segment at different positions meet after a few packages (the winner at a
-// position is a function of the position), so the host stitches the true chain from the speculative ones and
-// re-enters (a second launch, same kernel) only the segments whose true entry differs, each until it meets the
-// segment's speculative chain.
+// the multiples of g.  The file is cut into segments of DYN_SEGU * g bytes; one CTA walks the chain of a segment
+// from its first byte, evaluating the candidates at the positions it actually visits (speculative: the true chain
+// may enter the segment elsewhere).  Chains that enter a segment at different positions meet after a few packages
+// (the winner at a position is a function of the position), so the host stitches the true chain from the
+// speculative ones and re-enters (a second launch, same kernel) only the segments whose true entry differs, each
+// until it meets the segment's speculative chain.
 #define DYN_SEGU 64
 struct WalkRec { unsigned long long pos; uint32_t size; uint32_t type_len; };   // type << 24 | payload length
 struct WalkSeg { unsigned long long exit; unsigned long long stop; uint32_t count; uint32_t merged; uint32_t pad[2]; };
@@ -948,10 +707,8 @@ k_dynamic_walk(const uint8_t *__restrict__ in, uint64_t total, WalkCands cands, 
 }
 
 struct DynLayout {
-    uint64_t slots, spans, type, comp, offs, tiles, state, trial_type, trial_len, walk_recs, walk_segs, walk_list, total;
-    uint64_t n_pos, n_tiles, n_pass, g, n_seg;
-    uint32_t pass_size[16];
-    int cand_pass[32];
+    uint64_t slots, spans, type, comp, offs, tiles, state, walk_recs, walk_segs, walk_list, total;
+    uint64_t n_pos, n_tiles, g, n_seg;
 };
 static int dyn_layout(uint64_t n, const uint32_t *cands, uint32_t n_cands, DynLayout &L)
 {
@@ -965,14 +722,11 @@ static int dyn_layout(uint64_t n, const uint32_t *cands, uint32_t n_cands, DynLa
     if (g < 256 || g % 16) return ambc_fail(AMBC_E_ARG, "candidate sizes need a common divisor that is a multiple of 16 and >= 256");
     L.g = g;
     L.n_pos = (n + g - 1) / g;
-    L.n_pass = 0;
-    for (uint32_t i = 0; i < n_cands; i++) {
-        uint32_t sz = cands[i] < AMBC_NMAX ? cands[i] : AMBC_NMAX;
-        int found = -1;
-        for (uint64_t j = 0; j < L.n_pass; j++) if (L.pass_size[j] == sz) found = (int)j;
-        if (found < 0) { if (L.n_pass >= 16) return ambc_fail(AMBC_E_ARG, "too many distinct candidate sizes"); found = (int)L.n_pass; L.pass_size[L.n_pass++] = sz; }
-        L.cand_pass[i] = found;
-    }
+    // sizes clamped to 8192 (candidates are strictly descending, so equal clamped sizes are adjacent)
+    uint32_t n_sizes = 0;
+    for (uint32_t i = 0; i < n_cands; i++)
+        if (!i || min(cands[i], (uint32_t)AMBC_NMAX) != min(cands[i - 1], (uint32_t)AMBC_NMAX)) n_sizes++;
+    if (n_sizes > 16) return ambc_fail(AMBC_E_ARG, "too many distinct candidate sizes");
     L.n_tiles = (L.n_pos + SCAN_TILE - 1) / SCAN_TILE;
     uint64_t o = 0;
     auto take = [&](uint64_t bytes) { uint64_t r = o; o += (bytes + 255) & ~255ull; return r; };
@@ -983,8 +737,6 @@ static int dyn_layout(uint64_t n, const uint32_t *cands, uint32_t n_cands, DynLa
     L.offs = take(L.n_pos * 8 + 16);
     L.tiles = take(L.n_tiles * 8 + 16);
     L.state = take(sizeof(ScanState));
-    L.trial_type = take(L.n_pass * (L.n_pos + 16));
-    L.trial_len = take(L.n_pass * (L.n_pos * 4 + 16));
     L.n_seg = (L.n_pos + DYN_SEGU - 1) / DYN_SEGU;
     L.walk_recs = take(2 * L.n_pos * sizeof(WalkRec) + 64);   // speculative chains | re-entered chains
     L.walk_segs = take(2 * L.n_seg * sizeof(WalkSeg) + 64);
@@ -1029,9 +781,7 @@ extern "C" int ambc_compress_dynamic_dev(const void *in_dev, uint64_t n, const u
     std::vector<uint8_t> s_type;
     std::vector<uint32_t> s_len;
     uint64_t raw_from = n; // raw_from < n: one raw package [raw_from, n)
-    static int dyn_mode = -1; // dev knob: AMBC_DYNAMIC=trial keeps the round-1 path (every size at every multiple of g)
-    if (dyn_mode < 0) { const char *e = getenv("AMBC_DYNAMIC"); dyn_mode = (e && !strcmp(e, "trial")) ? 0 : 1; }
-    if (n && native && dyn_mode == 1) {
+    if (n && native) {
         // ---- the chain, walked on the GPU segment by segment (k_dynamic_walk) ------------------------------------
         WalkCands wc;
         wc.n = n_cands;
@@ -1121,51 +871,14 @@ extern "C" int ambc_compress_dynamic_dev(const void *in_dev, uint64_t n, const u
                 e = h_sseg[sg].exit;
             }
         }
+    } else if (!pcr) {
+        raw_from = 0; // no native method: the whole file is one raw package (:586-590)
     } else {
-        // ---- trial passes: sizes only, every multiple of g, one pass per distinct size ----------------
-        std::vector<uint8_t> h_type(L.n_pass * L.n_pos);
-        std::vector<uint32_t> h_len(L.n_pass * L.n_pos);
-        if (n && native) {
-            for (uint64_t j = 0; j < L.n_pass; j++) {
-                const uint32_t S = L.pass_size[j];
-                size_t smem = S <= LZ2_NMAX ? chunkctx_fast_smem_bytes((int)S) : chunkctx_smem_bytes((int)S, (int)S);
-                uint8_t *tt = W + L.trial_type + j * (L.n_pos + 16);
-                uint32_t *tl = (uint32_t *)(W + L.trial_len + j * (L.n_pos * 4 + 16));
-                unsigned grid = (unsigned)min<uint64_t>(L.n_pos, 0x7fffffffull);
-                if ((rc = launch_select_span(grid, smem, stream, (const uint8_t *)in_dev, n, S, method_mask, ovh, (uint32_t)L.g,
-                                             nullptr, nullptr, tt, tl, L.n_pos))) return rc;
-                CUDA_TRY(cudaMemcpyAsync(h_type.data() + j * L.n_pos, tt, L.n_pos, cudaMemcpyDeviceToHost, stream));
-                CUDA_TRY(cudaMemcpyAsync(h_len.data() + j * L.n_pos, tl, L.n_pos * 4, cudaMemcpyDeviceToHost, stream));
-            }
-            CUDA_TRY(cudaStreamSynchronize(stream));
-        }
-
-        // ---- the chain (adaptive_compressor.py:363-394 + 537-590) -------------------------------------
-        uint64_t pos = 0;
-        while (pos < n) {
-            const uint64_t remain = n - pos, i = pos / L.g;
-            double best_ratio = 1.0;
-            uint64_t best_c = remain;
-            int best_t = 255;
-            uint32_t best_len = 0;
-            for (uint32_t ci = 0; ci < n_cands && native; ci++) {
-                const uint64_t c = cands[ci] < remain ? cands[ci] : remain;
-                if (c > AMBC_NMAX) continue; // no native method is eligible (:114-127)
-                const uint64_t j = (uint64_t)L.cand_pass[ci];
-                const int t = h_type[j * L.n_pos + i];
-                if (t == 255) continue;
-                const uint32_t len = h_len[j * L.n_pos + i];
-                const double ratio = (double)((uint64_t)len + ovh) / (double)c; // (:573-574)
-                if (ratio < best_ratio) { best_ratio = ratio; best_c = c; best_t = t; best_len = len; }
-            }
-            if (best_t == 255) {
-                if (!pcr) { raw_from = pos; break; }                       // rest of the file raw (:586-590)
-                best_c = cands[n_cands - 1] < remain ? cands[n_cands - 1] : remain; // labelled extension
-                best_len = (uint32_t)best_c;
-            }
-            ChunkSpan sp; sp.pos = pos; sp.size = (uint32_t)best_c; sp.pad = 0;
-            spans.push_back(sp); s_type.push_back((uint8_t)best_t); s_len.push_back(best_len);
-            pos += best_c;
+        // per-chunk-raw extension without a native method: raw pieces of the smallest candidate size
+        for (uint64_t pos = 0; pos < n;) {
+            ChunkSpan sp; sp.pos = pos; sp.size = (uint32_t)min<uint64_t>(cands[n_cands - 1], n - pos); sp.pad = 0;
+            spans.push_back(sp); s_type.push_back(255); s_len.push_back(sp.size);
+            pos += sp.size;
         }
     }
     const uint64_t n_list = spans.size();
@@ -1195,9 +908,8 @@ extern "C" int ambc_compress_dynamic_dev(const void *in_dev, uint64_t n, const u
         if (maxsz > AMBC_NMAX) { // only per-chunk-raw pieces can be this large
             return ambc_fail(AMBC_E_ARG, "per-chunk-raw pieces larger than 8192 bytes are not supported");
         }
-        size_t smem = maxsz <= LZ2_NMAX ? chunkctx_fast_smem_bytes((int)maxsz) : chunkctx_smem_bytes((int)maxsz, (int)maxsz);
         unsigned grid = (unsigned)min<uint64_t>(n_list, 0x7fffffffull);
-        if ((rc = launch_select_span(grid, smem, stream, (const uint8_t *)in_dev, n, maxsz, method_mask, ovh, 0, d_spans,
+        if ((rc = launch_select_span(grid, stream, (const uint8_t *)in_dev, n, maxsz, method_mask, ovh, 0, d_spans,
                                      W + L.slots, type, comp, n_list))) return rc;
         const unsigned gt = (unsigned)((n_list + SCAN_TILE - 1) / SCAN_TILE);
         const uint32_t sflags = 1u | 2u; // every entry is a package; no END (appended below)
@@ -1256,7 +968,3 @@ extern "C" int ambc_compress_dynamic_dev(const void *in_dev, uint64_t n, const u
     }
     return AMBC_OK;
 }
-
-int ambc_lz_levels_compress(const int *levels, int n) { return lz_levels_upload(levels, n); }
-int ambc_lz_coop_compress(int t) { return lz_coop_upload(t); }
-int ambc_lz_force_buckets_compress(int on) { return lz_force_buckets_upload(on); }

@@ -138,11 +138,11 @@ __device__ __forceinline__ uint32_t lz2_insert_pair(ChunkCtx &c, uint32_t mask, 
 }
 
 // name_4 (D) for every position, matches of length 4.  Returns "any match".
-__device__ inline int lz2_level4(ChunkCtx &c, uint16_t *D, bool count)
+__device__ inline int lz2_level4(ChunkCtx &c, uint16_t *D)
 {
     const int n = c.n, tid = threadIdx.x;
     lz2_clear(c, LZ2_TSLOTS);
-    if (tid == 0) { c.red[30] = 0; c.red[27] = 0; c.red[26] = 0; } // level-3 list length; match counts at 4 / 8
+    if (tid == 0) c.red[30] = 0; // level-3 list length
     __syncthreads();
     const int P = n - 3;
     for (int p = tid; p < n; p += AMBC_BLOCK) {
@@ -175,10 +175,6 @@ __device__ inline int lz2_level4(ChunkCtx &c, uint16_t *D, bool count)
             if (head3) list3[base + __popc(m & ((1u << lane) - 1))] = (uint16_t)p;
         }
     }
-    if (count) { // number of positions with a match of >= 4 bytes (early-abort bound of lz2_match_all)
-        const int w = warp_sum(nonhead);
-        if (lane == 0 && w) atomicAdd(c.red + 27, w);
-    }
     return __syncthreads_or(nonhead);
 }
 
@@ -210,7 +206,7 @@ __device__ inline void lz2_level3(ChunkCtx &c, uint16_t *tmp)
 // heads by construction and do not enter the table.  Also lists the participants of the bracket
 // (k, 2k) in c.L: heads of their 2k-gram whose k-gram occurs elsewhere, with room for k+1 bytes
 // (count in c.red[30]).  Returns "any match of 2k bytes".
-__device__ inline int lz2_double(ChunkCtx &c, const uint16_t *S, uint16_t *D, int k, bool count = false)
+__device__ inline int lz2_double(ChunkCtx &c, const uint16_t *S, uint16_t *D, int k)
 {
     const int n = c.n, tid = threadIdx.x, lane = tid & 31;
     lz2_clear(c, LZ2_TSLOTS);
@@ -254,10 +250,6 @@ __device__ inline int lz2_double(ChunkCtx &c, const uint16_t *S, uint16_t *D, in
             base = __shfl_sync(FULL_MASK, base, 0);
             if (part) plist[base + __popc(m & ((1u << lane) - 1))] = (uint16_t)p;
         }
-    }
-    if (count) {
-        const int w = warp_sum(nonhead);
-        if (lane == 0 && w) atomicAdd(c.red + 26, w);
     }
     return __syncthreads_or(nonhead);
 }
@@ -333,7 +325,6 @@ __device__ inline int lz2_refine_binary_dense(ChunkCtx &c, const uint16_t *S, in
     const int n = c.n, tid = threadIdx.x, lane = tid & 31;
     uint16_t *A = (uint16_t *)c.L, *B = A + LZ2_LISTCAP, *islot = B + LZ2_LISTCAP;
     int E = np, dummy = 0, round = 0;
-    PHASE_DECL
     for (int step = k >> 1; step >= 1; step >>= 1, round++) {
         // two alternating counters: the one of this round was last read two rounds ago
         volatile int *cntB = c.red + 28 + (round & 1);
@@ -344,7 +335,6 @@ __device__ inline int lz2_refine_binary_dense(ChunkCtx &c, const uint16_t *S, in
         lz2_clear(c, 1 << tbits);
         if (tid == 0) *cntB = 0;
         __syncthreads();
-        PHASE(16);
         for (int i = tid; i < E; i += AMBC_BLOCK) {
             const uint32_t item = A[i];
             const int p = item & 0xFFFu, t = item >> 12;
@@ -360,7 +350,6 @@ __device__ inline int lz2_refine_binary_dense(ChunkCtx &c, const uint16_t *S, in
             islot[i] = (uint16_t)slot;
         }
         __syncthreads();
-        PHASE(17);
         bool overflow = false;
         for (int ib = 0; ib < E; ib += AMBC_BLOCK) {
             const int i = ib + tid;
@@ -399,7 +388,6 @@ __device__ inline int lz2_refine_binary_dense(ChunkCtx &c, const uint16_t *S, in
             }
         }
         const int ov = __syncthreads_or(overflow);
-        PHASE(18);
         if (ov) return 1;
         E = *cntB;
         uint16_t *tmp = A; A = B; B = tmp;
@@ -438,54 +426,22 @@ __device__ inline bool lz2_refine(ChunkCtx &c, const uint16_t *S, const uint16_t
     return lz2_refine_flat(c, S, k, c.red[30], plist, (uint16_t *)(c.L + 8192));
 }
 
-// Lower bound on the Dictionary payload of ANY parse of n bytes in which at most `a` tokens start at a
-// position with a match of >= 8 bytes (they cover at most 32 bytes for 4 payload bytes), at most `b` at a
-// position whose longest match has 4..7 bytes (at most 7 bytes for 4), and every other token covers at most
-// 3 bytes for 4 or 1 byte for 2 (compression_methods.py:211-232).  Tokens may be cut short, so the bound
-// holds for the greedy parse whatever it turns out to be.
-__device__ __forceinline__ int lz2_small_cost(int r) { return 4 * (r / 3) + 2 * (r % 3); }
-__device__ inline int lz2_count_bound(int n, int a_avail, int b_avail)
-{
-    const int a = min(a_avail, n >> 5);
-    int rem = n - 32 * a;
-    if (a < a_avail) return 4 * a + min(4, lz2_small_cost(rem));
-    const int b = min(b_avail, rem / 7);
-    rem -= 7 * b;
-    if (b < b_avail) return 4 * a + 4 * b + min(4, lz2_small_cost(rem));
-    return 4 * a + 4 * b + lz2_small_cost(rem);
-}
-
 // mlen / mpos for every position of the chunk (c.mlen zeroed by the caller).  n <= LZ2_NMAX.
-// Returns 0 = done, 1 = a table overflowed (run the bucket search), 2 = given up: after the 8-byte level
-// the counts of positions with matches of >= 4 and >= 8 bytes prove a payload of at least `cutoff` bytes.
-__device__ inline int lz2_match_all(ChunkCtx &c, int cutoff)
+// Returns 0 = done, 1 = a table overflowed (run the bucket search).
+__device__ inline int lz2_match_all(ChunkCtx &c)
 {
     uint16_t *A = c.nameA, *B = c.nameB;
     if (c.n < 3) return 0;
-    const bool bounded = cutoff < 0x7fffffff;
-    PHASE_DECL // (dev-only phase timeline, see chunk_codec.cuh)
-    const int any4 = lz2_level4(c, A, bounded);
-    PHASE(2);
+    const int any4 = lz2_level4(c, A);
     lz2_level3(c, B);
-    PHASE(3);
     if (!any4) return 0;
-    const int any8 = lz2_double(c, A, B, 4, bounded);
-    PHASE(4);
-    if (bounded) { // (the counters were complete at the barrier that ended lz2_double)
-        const int n4 = c.red[27], n8 = c.red[26];
-        if (lz2_count_bound(c.n, n8, n4 - n8) >= cutoff) return 2;
-    }
+    const int any8 = lz2_double(c, A, B, 4);
     if (!lz2_refine(c, A, B, 4)) return 1;
-    PHASE(5);
     if (!any8) return 0;
     const int any16 = lz2_double(c, B, A, 8);
-    PHASE(6);
     if (!lz2_refine(c, B, A, 8)) return 1;
-    PHASE(7);
     if (!any16) return 0;
     lz2_double(c, A, B, 16);
-    PHASE(8);
     const bool ok = lz2_refine(c, A, B, 16);
-    PHASE(9);
     return ok ? 0 : 1;
 }

@@ -9,28 +9,10 @@ from . import _lib as L
 FIXED_MARKER = b"\xff\xff\x00\x00"  # adaptive_compressor.py:303-310 (_find_marker is a stub)
 
 
-_levels_done = False
-
-
 def require_cuda():
-    global _levels_done
     if not torch.cuda.is_available():
         raise RuntimeError("adaptive_compression_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
-    lib = L.lib()
-    if not _levels_done:
-        _levels_done = True
-        import os
-        env = os.environ.get("AMBC_LZ_LEVELS")  # experiment knob, e.g. "3,4,6,10"; results are identical
-        if env:
-            set_lz_levels([int(x) for x in env.split(",")])
-    return lib
-
-
-def set_lz_levels(levels):
-    lib = L.lib()
-    arr = (C.c_int * len(levels))(*levels)
-    lib.ambc_set_lz_levels.restype = C.c_int
-    L.check(lib.ambc_set_lz_levels(arr, len(levels)))
+    return L.lib()
 
 
 def _stream_ptr():

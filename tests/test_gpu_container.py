@@ -82,7 +82,7 @@ def test_body_fuzz_vs_oracle(eng, chunk):
 
 
 def test_selection_small_alphabets_vs_oracle(eng):
-    """the Huffman-first order of k_select and its early stop of a Dictionary trial that cannot win
+    """the Huffman-first order of k_select_fast and its early stop of a Dictionary trial that cannot win
     (small alphabets, varying skew, sprinkled repeats and runs) never change the outcome: body and
     method map equal to the oracle's in-order trial of every method (adaptive_compressor.py:537-590)"""
     r = np.random.RandomState(77)
@@ -232,16 +232,22 @@ def test_dynamic_candidates_golden_and_oracle(eng, golden):
 @pytest.mark.parametrize("cands", [(131072, 65536, 32768, 16384, 8192, 4096, 2048, 1024), (4096, 1024), (8192, 2048, 512)])
 def test_dynamic_candidates_fuzz_vs_oracle(eng, cands):
     r = np.random.RandomState(sum(cands) % 1000)
-    for i in range(6):
+    for i in range(7):
         kinds = ("text", "csv", "log", "runs", "lowcard", "binrec", "periodic", "rand")
         parts = [inputs.make(kinds[r.randint(len(kinds) - (0 if i % 3 == 2 else 1))], int(r.choice([700, 1024, 2048, 3000, 4096, 9000])), 6000 + 100 * i + j)
                  for j in range(int(r.randint(3, 9)))]
         data = b"".join(parts)
+        # the last input allows no method at all: strict mode sends the whole file to one raw package, per-chunk-raw
+        # mode cuts it into raw pieces of the smallest candidate size
+        methods = () if i == 6 else (1, 2, 3, 4)
         for pcr in (False, True):
             from adaptive_compression_b200 import _lib as L
-            o = eng.compress_dynamic_device(eng.to_device(data), cands, flags=L.F_PER_CHUNK_RAW if pcr else 0)
-            wbody, wpm = O.compress_body(data, cands, per_chunk_raw=pcr)
+            o = eng.compress_dynamic_device(eng.to_device(data), cands, mask=eng.method_mask(methods),
+                                            flags=L.F_PER_CHUNK_RAW if pcr else 0)
+            wbody, wpm = O.compress_body(data, cands, methods, per_chunk_raw=pcr)
             assert o.body.cpu().numpy().tobytes() == wbody, (cands, i, pcr)
             assert [list(p) for p in o.packages] == [list(p) for p in wpm]
+            if i == 6:
+                assert {p[0] for p in wpm} == {255} and len(wpm) == (-(-len(data) // cands[-1]) if pcr else 1)
             out, status = eng.decompress_device(o.body, len(data))
             assert status == [0, 0] and out.cpu().numpy().tobytes() == data

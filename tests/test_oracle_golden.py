@@ -116,51 +116,3 @@ def test_container_dynamic_kat(golden):
         assert len(f) == row["ambc_len"] and sha(f) == row["ambc_sha256"], row["name"]
         assert [list(p) for p in pm] == row["packages"], row["name"]
         assert O.decompress_file(f) == data
-
-
-def test_dictionary_lower_bounds_hold():
-    """the two lower bounds that let k_select stop a Dictionary trial early (compress.cu select_chunk,
-    lz_names.cuh lz2_count_bound) never exceed the oracle's Dictionary payload: (1) the counting bound from
-    the numbers of positions with a match of >= 8 / of 4..7 bytes, (2) the prefix bound from the exact parse
-    of the first 5/8 of the chunk"""
-    def small_cost(r):
-        return 4 * (r // 3) + 2 * (r % 3)
-
-    def count_bound(n, a_avail, b_avail):
-        a = min(a_avail, n >> 5)
-        rem = n - 32 * a
-        if a < a_avail:
-            return 4 * a + min(4, small_cost(rem))
-        b = min(b_avail, rem // 7)
-        rem -= 7 * b
-        if b < b_avail:
-            return 4 * a + 4 * b + min(4, small_cost(rem))
-        return 4 * a + 4 * b + small_cost(rem)
-
-    def matched(d, L):  # positions whose L-gram occurred earlier
-        seen, k = set(), 0
-        for p in range(len(d) - L + 1):
-            g = d[p:p + L]
-            k += g in seen
-            seen.add(g)
-        return k
-
-    import numpy as np
-    r = np.random.RandomState(3)
-    for it in range(40):
-        n = int(r.choice([2048, 3000, 4096]))
-        K = int(r.choice([2, 3, 5, 8, 12, 20, 40]))
-        a = r.randint(0, K, size=n).astype(np.uint8)
-        for _ in range(int(r.choice([0, 10, 100, 400]))):
-            L = int(r.choice([4, 6, 8, 12, 20, 32]))
-            s_, d_ = int(r.randint(0, n - L)), int(r.randint(0, n - L))
-            a[d_:d_ + L] = a[s_:s_ + L].copy()
-        d = a.tobytes()
-        lz = O.compress(2, d)
-        assert not isinstance(lz, int)
-        n8, n4 = matched(d, 8), matched(d, 4)
-        assert count_bound(n, n8, n4 - n8) <= len(lz), (it, n, K)
-        npre = ((5 * n // 8) & ~31) + 31
-        lenp = len(O.compress(2, d[:npre]))
-        rest = n - npre
-        assert lenp - 62 + 4 * (rest >> 5) + min(4, 2 * (rest & 31)) <= len(lz), (it, n, K)

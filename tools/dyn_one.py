@@ -1,4 +1,4 @@
-"""dev tool: one dynamic-mode compress of 32 MiB (for an ncu launch list of the trial passes)"""
+"""dev tool: one dynamic-mode compress of 32 MiB (for an ncu launch list of the chain walk)"""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch

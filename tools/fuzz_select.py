@@ -1,5 +1,5 @@
-"""dev tool: randomized parity fuzz of the chunk selection (k_select) against the oracle, aimed at the
-Huffman-first / early-abort path: small alphabets with varying skew, repeated fragments of varying
+"""dev tool: randomized parity fuzz of the chunk selection (k_select_fast) against the oracle, aimed at
+the Huffman-first / early-abort path: small alphabets with varying skew, repeated fragments of varying
 length and density (so that the Dictionary method wins, loses narrowly, or loses clearly), runs."""
 import sys, os, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))

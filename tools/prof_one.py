@@ -1,4 +1,4 @@
-"""dev tool: run k_select on one corpus kind (for ncu)"""
+"""dev tool: run k_select_fast on one corpus kind (for ncu)"""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from adaptive_compression_b200 import engine

@@ -1,4 +1,4 @@
-"""dev tool: k_select time per corpus kind for one library variant (AMBC_LIB_PATH)"""
+"""dev tool: k_select_fast time per corpus kind for one library variant (AMBC_LIB_PATH)"""
 import ctypes as C, sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from adaptive_compression_b200 import engine, _lib as L

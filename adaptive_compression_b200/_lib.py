@@ -9,6 +9,7 @@ LIB_PATH = os.environ.get("AMBC_LIB_PATH") or os.path.join(_HERE, "libambc.so") 
 OK, E_CUDA, E_ARG, E_CAPACITY, E_MARKER, E_TOO_LARGE, E_NO_MARKER = 0, -1, -2, -3, -4, -5, -6
 RLE, DICT, HUFFMAN, DELTA, RAW = 1, 2, 3, 4, 255
 DEFLATE = 5  # zlib streams (advanced_compression.py:71-107): a plug-in codec and a decodable package type, not a trial candidate
+BZIP2, LZMA = 6, 7  # bz2 / lzma streams: decode-only plug-in codecs and decodable package types
 NATIVE_MASK = (1 << 1) | (1 << 2) | (1 << 3) | (1 << 4)
 MAX_CODEC_CHUNK = 8192
 F_PER_CHUNK_RAW = 1
@@ -70,6 +71,8 @@ _SIGS = {
                                  C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_void_p]),
     "ambc_decompress_dev": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64,
                                       C.c_void_p, C.c_void_p]),
+    "ambc_decompress_dev_mask": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64,
+                                           C.c_uint32, C.c_void_p, C.c_void_p]),
     "ambc_decompress_host": (C.c_int, [C.c_void_p, C.c_uint64, C.c_char_p, C.c_uint32, C.c_uint32, C.c_void_p,
                                        C.c_uint64, C.c_void_p]),
     "ambc_codec_bound": (C.c_uint64, [C.c_int, C.c_uint32]),

@@ -12,8 +12,9 @@ What differs, on purpose:
     tried at every position on the GPU).  chunk_size=N selects ONE size -- the fixed grid of the benchmarked
     path (--chunk-size 4096 in BASELINE.json's configs), an order of magnitude faster.  Candidate lists are
     searched largest first (the reference honours the list order on ratio ties; its own list is descending).
-  * only the repo-native methods 1-4 (+255) are loaded by default; DEFLATE (id 5) on request (methods=[..., 5]): decoded
-    on the GPU, not a trial candidate; the other third-party codecs 6-11 are out of scope.
+  * only the repo-native methods 1-4 (+255) are loaded by default; DEFLATE (id 5), BZIP2 (id 6) and LZMA (id 7) on
+    request (methods=[..., 5, 6, 7]): decoded on the GPU, not trial candidates; the other third-party codecs 8-11 are
+    out of scope.
   * per_chunk_raw=True and use_marker_search=True are labelled extensions (files stay readable by
     the reference decoder)."""
 import hashlib
@@ -27,8 +28,8 @@ import torch
 
 from . import _lib as L
 from . import engine
-from .compression_methods import (DeflateCompression, DeltaCompression, DictionaryCompression, HuffmanCompression, NoCompression,
-                                  RLECompression)
+from .compression_methods import (BZip2Compression, DeflateCompression, DeltaCompression, DictionaryCompression,
+                                  HuffmanCompression, LZMACompression, NoCompression, RLECompression)
 from .marker_finder import MarkerFinder
 
 METHOD_NAMES = {1: "RLE", 2: "Dictionary", 3: "Huffman", 4: "Delta", 5: "DEFLATE", 6: "BZIP2", 7: "LZMA",
@@ -73,10 +74,10 @@ class AdaptiveCompressor:
                                     DeltaCompression(), NoCompression()]
         if methods is not None:
             keep = set(int(m) for m in methods) | {255}
-            if 5 in keep:
-                # DEFLATE on request (advanced_compression.py:71-107): packages of type 5 decode on the GPU; the
-                # chunk trial of compress() stays with methods 1-4, see _method_mask
-                self.compression_methods.insert(4, DeflateCompression())
+            # DEFLATE, BZIP2 and LZMA on request (the stdlib codecs of advanced_compression.py): packages of these
+            # types decode on the GPU; the chunk trial of compress() stays with methods 1-4, see _method_mask
+            self.compression_methods[4:4] = [cls() for mid, cls in ((5, DeflateCompression), (6, BZip2Compression),
+                                                                     (7, LZMACompression)) if mid in keep]
             self.compression_methods = [m for m in self.compression_methods if m.type_id in keep]
         if disable_methods:
             drop = set(int(m) for m in disable_methods) - {255}
@@ -153,14 +154,17 @@ class AdaptiveCompressor:
 
     def _method_mask(self):
         ids = [m.type_id for m in self.compression_methods if m.type_id != 255]
-        foreign = [i for i in ids if i not in (1, 2, 3, 4, 5)]
+        foreign = [i for i in ids if i not in (1, 2, 3, 4, 5, 6, 7)]
         if foreign:
             raise NotImplementedError("only the repo-native methods 1-4 run on the B200 path; got %s" % foreign)
         if 5 in ids:
             # the GPU DEFLATE encoder does not write zlib.compress(level=9)'s bytes, so a trial with it could
             # not reproduce the reference's choices: it is a plug-in (DeflateCompression) and a decodable type
             print("DEFLATE (id 5) is decoded but takes no part in the chunk trial on the B200 path")
-        return engine.method_mask([i for i in ids if i != 5])
+        for i in (6, 7):
+            if i in ids:  # decode-only: there is no GPU encoder whose bytes would be libbzip2's / liblzma's
+                print("%s (id %d) is decoded but takes no part in the chunk trial on the B200 path" % (METHOD_NAMES[i], i))
+        return engine.method_mask([i for i in ids if i not in (5, 6, 7)])
 
     # ---- compress (adaptive_compressor.py:221-255) ----
     @staticmethod

@@ -140,6 +140,51 @@ class DeflateCompression(CompressionMethod):
         return not ent[0] >= 8.0
 
 
+class _StdlibDecoder(CompressionMethod):
+    """a codec the reference takes from the Python stdlib, decoded on the GPU only"""
+    _id = 0
+    _stock = ""
+
+    @property
+    def type_id(self):
+        return self._id
+
+    def compress(self, data):
+        raise NotImplementedError("%s streams are decoded on the GPU but not written there: a GPU encoder's bytes "
+                                  "would not be stock %s's, so they could not reproduce the reference's files"
+                                  % (type(self).__name__, self._stock))
+
+    def decompress(self, data, original_length):
+        if not data:
+            return b""
+        out = engine.codec_decode_batch(self._id, [bytes(data)], [int(original_length)])[0]
+        if isinstance(out, int):
+            raise L.AmbcError(out, "%s decode failed" % type(self).__name__)
+        return out
+
+    def should_use(self, data, threshold=0.9):
+        return False  # decode-only: never a candidate for compressing a chunk
+
+
+class BZip2Compression(_StdlibDecoder):
+    """method id 6, where the reference calls the stdlib's bz2.  decompress() has the semantics of
+    bz2.decompress(data) -- BZh1..BZh9 streams, randomised blocks, concatenated streams, trailing bytes
+    that do not start a stream ignored -- padded / truncated to original_length, and original_length zero
+    bytes where bz2.decompress raises (bad data, CRC mismatch, truncated stream).  Decode only."""
+    _id = L.BZIP2
+    _stock = "libbzip2"
+
+
+class LZMACompression(_StdlibDecoder):
+    """method id 7, where the reference calls the stdlib's lzma.  decompress() has the semantics of
+    lzma.decompress(data) with FORMAT_AUTO -- .xz streams with one LZMA2 filter and a None / CRC32 / CRC64
+    check, stream padding, concatenated streams, the legacy .lzma header -- padded / truncated to
+    original_length, and original_length zero bytes where lzma.decompress raises.  Other filter chains and the
+    SHA-256 check are not implemented and count as errors.  Decode only."""
+    _id = L.LZMA
+    _stock = "liblzma"
+
+
 class NoCompression(CompressionMethod):
     """identity (compression_methods.py:670-713)"""
 

@@ -240,7 +240,7 @@ int ambc_index_stream(const uint8_t *body, uint64_t body_len, const uint8_t *mar
                       uint32_t known_mask, void (*sink)(void *, const ambc_pkg &), void *user, uint64_t *n_entries,
                       uint64_t *out_bytes);
 int ambc_decode_launch(const void *body_dev, const ambc_pkg *table_dev, uint64_t n_entries, void *out_dev,
-                       uint32_t *status_dev, cudaStream_t stream);
+                       uint32_t *status_dev, cudaStream_t stream, uint32_t known_mask);
 
 // state of the piece-wise decode that runs while the host walks the package chain
 struct DecPipe {
@@ -250,6 +250,7 @@ struct DecPipe {
     uint64_t body_len, uploaded = 0; // body bytes whose upload has been queued on the copy stream
     uint64_t filled = 0, flushed_entries = 0;
     uint64_t piece_entries = 2048; // ramps up to DEC_PIECE_ENTRIES so the first download starts early
+    uint32_t known_mask = 0;       // packages of types 6 / 7 are decoded when their bits are set
     int rc = AMBC_OK;
     int ev = 0, ring = 0, up = 0;
 };
@@ -291,7 +292,7 @@ static void decpipe_flush(DecPipe &d)
     cudaStreamWaitEvent(c->stream, up, 0);
     decpipe_upload(d, need + DEC_BODY_AHEAD);
     if (d.rc) return;
-    d.rc = ambc_decode_launch(c->in.p, tab_dev, d.filled, c->out.p, (uint32_t *)c->status.p, c->stream);
+    d.rc = ambc_decode_launch(c->in.p, tab_dev, d.filled, c->out.p, (uint32_t *)c->status.p, c->stream, d.known_mask);
     if (d.rc) return;
     // results of this piece go home on the download stream while the walk and the next kernels continue
     const uint64_t d0 = src[0].dst_off, d1 = src[d.filled - 1].dst_off + src[d.filled - 1].out_len;
@@ -344,6 +345,7 @@ extern "C" int ambc_decompress_host(const void *body_host, uint64_t body_len, co
     CUDA_TRY(cudaMemsetAsync(c->status.p, 0, 8, c->stream));
     DecPipe d;
     d.c = c; d.body_host = (const uint8_t *)body_host; d.out_host = (uint8_t *)out_host; d.body_len = body_len;
+    d.known_mask = known_mask;
     decpipe_upload(d, DEC_BODY_AHEAD);
     if (d.rc) return d.rc;
     rc = ambc_index_stream((const uint8_t *)body_host, body_len, marker, marker_bytes, orig_size, known_mask,

@@ -328,7 +328,7 @@ k_decode(const uint8_t *__restrict__ body, const ambc_pkg *__restrict__ table, u
         bool want = false;
         if (mine < n_entries) {
             const ambc_pkg e = table[mine];
-            want = !dlz_eligible(e) && !dw_eligible(e, 8192);
+            want = !dlz_eligible(e) && !dw_eligible(e, 8192) && e.type != 6 && e.type != 7; // (6, 7: stdcodec.cu)
         }
         const uint32_t bal = __ballot_sync(FULL_MASK, want);
         if ((threadIdx.x & 31) == 0) s_mask[threadIdx.x >> 5] = bal;
@@ -417,9 +417,13 @@ __global__ void k_zero_tail(const ambc_pkg *__restrict__ table, uint64_t n_entri
         out[i] = 0;
 }
 
-// launch the decoders for table[0 .. n_entries) (no tail zeroing)
+int ambc_stdcodec_decode_table(const void *body_dev, const ambc_pkg *table_dev, uint64_t n_entries, void *out_dev,
+                               uint32_t *status_dev, uint32_t known_mask, cudaStream_t stream);
+
+// launch the decoders for table[0 .. n_entries) (no tail zeroing).  Packages of types 6 and 7 are decoded when
+// their bits are set in known_mask; without them the launches are exactly those of a table of native packages.
 int ambc_decode_launch(const void *body_dev, const ambc_pkg *table_dev, uint64_t n_entries, void *out_dev,
-                       uint32_t *status_dev, cudaStream_t stream)
+                       uint32_t *status_dev, cudaStream_t stream, uint32_t known_mask)
 {
     if (n_entries == 0) return AMBC_OK;
     const int in_cap = DEC_OUT_CAP; // payloads the reference's encoder emits are < orig_len <= 8192
@@ -468,14 +472,18 @@ int ambc_decode_launch(const void *body_dev, const ambc_pkg *table_dev, uint64_t
     k_decode<<<grid, AMBC_BLOCK, smem, stream>>>((const uint8_t *)body_dev, table_dev, n_entries, (uint8_t *)out_dev,
                                                  in_cap, status_dev);
     ambc_count_launch();
+    if (known_mask & (AMBC_METHOD_BIT(AMBC_BZIP2) | AMBC_METHOD_BIT(AMBC_LZMA))) {
+        const int rc = ambc_stdcodec_decode_table(body_dev, table_dev, n_entries, out_dev, status_dev, known_mask, stream);
+        if (rc) return rc;
+    }
     CUDA_TRY(cudaStreamWaitEvent(stream, ev_join[dev], 0));
     CUDA_TRY(cudaGetLastError());
     return AMBC_OK;
 }
 
-extern "C" int ambc_decompress_dev(const void *body_dev, uint64_t body_len, const ambc_pkg *table_dev,
-                                   uint64_t n_entries, void *out_dev, uint64_t orig_size, uint32_t *status_dev,
-                                   void *stream_)
+extern "C" int ambc_decompress_dev_mask(const void *body_dev, uint64_t body_len, const ambc_pkg *table_dev,
+                                        uint64_t n_entries, void *out_dev, uint64_t orig_size, uint32_t known_mask,
+                                        uint32_t *status_dev, void *stream_)
 {
     cudaStream_t stream = (cudaStream_t)stream_;
     (void)body_len;
@@ -488,15 +496,24 @@ extern "C" int ambc_decompress_dev(const void *body_dev, uint64_t body_len, cons
     ambc_timing_mark(4, stream);
     k_zero_tail<<<148, 256, 0, stream>>>(table_dev, n_entries, (uint8_t *)out_dev, orig_size);
     ambc_count_launch();
-    int rc = ambc_decode_launch(body_dev, table_dev, n_entries, out_dev, status_dev, stream);
+    int rc = ambc_decode_launch(body_dev, table_dev, n_entries, out_dev, status_dev, stream, known_mask);
     if (rc) return rc;
     ambc_timing_mark(5, stream);
     ambc_timing().pending_d = ambc_timing().on;
     return AMBC_OK;
 }
 
+extern "C" int ambc_decompress_dev(const void *body_dev, uint64_t body_len, const ambc_pkg *table_dev,
+                                   uint64_t n_entries, void *out_dev, uint64_t orig_size, uint32_t *status_dev,
+                                   void *stream_)
+{
+    return ambc_decompress_dev_mask(body_dev, body_len, table_dev, n_entries, out_dev, orig_size, 0u, status_dev, stream_);
+}
+
 int ambc_inflate_batch(const void *in_dev, const uint64_t *in_off_dev, const uint32_t *orig_len_dev, uint32_t n_items,
                        void *out_dev, uint64_t out_stride, int32_t *out_len_dev, cudaStream_t stream);
+int ambc_stdcodec_decode_batch(int method, const void *in_dev, const uint64_t *in_off_dev, const uint32_t *orig_len_dev,
+                               uint32_t n_items, void *out_dev, uint64_t out_stride, int32_t *out_len_dev, cudaStream_t stream);
 
 // ---- codec plug-in batch kernels (CompressionMethod API parity) -------------------------------
 // items the warp decoders take (the same code as the container path, so the codec-level fixtures hold it too)
@@ -561,11 +578,13 @@ extern "C" int ambc_codec_decode_batch(int method, const void *in_dev, const uin
                                        uint64_t out_stride, int32_t *out_len_dev, void *stream_)
 {
     cudaStream_t stream = (cudaStream_t)stream_;
-    if (!(method == 1 || method == 2 || method == 3 || method == 4 || method == 5 || method == 255))
+    if (!((method >= 1 && method <= 7) || method == 255))
         return ambc_fail(AMBC_E_ARG, "ambc_codec_decode_batch: unknown method %d", method);
     if (n_items == 0) return AMBC_OK;
     if (!in_off_dev || !orig_len_dev || !out_dev || !out_len_dev) return ambc_fail(AMBC_E_ARG, "null buffer");
     if (method == 5) return ambc_inflate_batch(in_dev, in_off_dev, orig_len_dev, n_items, out_dev, out_stride, out_len_dev, stream);
+    if (method == 6 || method == 7)
+        return ambc_stdcodec_decode_batch(method, in_dev, in_off_dev, orig_len_dev, n_items, out_dev, out_stride, out_len_dev, stream);
     const int in_cap = 2 * AMBC_NMAX + 2048; // any payload the encoders can emit for <= 8192 bytes
     size_t smem = decctx_smem_bytes(in_cap);
     CUDA_TRY(cudaFuncSetAttribute(k_codec_decode, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));

@@ -172,10 +172,10 @@ def decompress_device(t_body, orig_size, marker=FIXED_MARKER, known_mask=L.NATIV
         table, _ = index_host(body_host, orig_size, marker, known_mask)
         t_table = torch.from_numpy(table.view(np.uint8).reshape(-1).copy()).to("cuda") if len(table) else \
             torch.empty(0, dtype=torch.uint8, device="cuda")
-    L.check(lib.ambc_decompress_dev(C.c_void_p(t_body.data_ptr() if t_body.numel() else 0), t_body.numel(),
-                                    C.c_void_p(t_table.data_ptr() if len(table) else 0), len(table),
-                                    C.c_void_p(out.data_ptr()), orig_size, C.c_void_p(status.data_ptr()),
-                                    _stream_ptr()))
+    L.check(lib.ambc_decompress_dev_mask(C.c_void_p(t_body.data_ptr() if t_body.numel() else 0), t_body.numel(),
+                                         C.c_void_p(t_table.data_ptr() if len(table) else 0), len(table),
+                                         C.c_void_p(out.data_ptr()), orig_size, known_mask, C.c_void_p(status.data_ptr()),
+                                         _stream_ptr()))
     torch.cuda.current_stream().synchronize()
     return out[:orig_size], status.cpu().tolist()
 
@@ -212,13 +212,30 @@ def codec_encode_batch(method, items):
 
 def codec_decode_batch(method, items, orig_lens):
     """items: payloads; -> list of bytes | int error code (what the reference's decompress returns)"""
-    lib = require_cuda()
+    require_cuda()
     if not items:
         return []
-    blob, offs = _pack_items(items)
     stride = (max(max(orig_lens), 1) + 512 + 15) & ~15
     if method == L.DEFLATE:
         stride += 32768  # window of a stream that runs past original_length (it is checked to its end, then truncated)
+    elif method == L.LZMA:
+        stride += 65536  # the whole stride is the dictionary: a stream is decoded (and its check verified) to its end
+    out = _codec_decode(method, items, orig_lens, stride)
+    # LZMA streams that decode past the stride: again, one at a time, with room for them
+    for i, o in enumerate(out):
+        room = stride
+        while o == L.E_CAPACITY:
+            room *= 4
+            if room > (1 << 34):
+                raise L.AmbcError(L.E_CAPACITY, "stream %d decodes to more than %d bytes" % (i, 1 << 34))
+            o = _codec_decode(method, [items[i]], [orig_lens[i]], room)[0]
+        out[i] = o
+    return out
+
+
+def _codec_decode(method, items, orig_lens, stride):
+    lib = L.lib()
+    blob, offs = _pack_items(items)
     t_in = to_device(blob)
     t_off = torch.from_numpy(offs.view(np.int64)).to("cuda")
     t_orig = torch.tensor(list(orig_lens), dtype=torch.int32, device="cuda")

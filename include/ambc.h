@@ -39,6 +39,9 @@ extern "C" {
 #define AMBC_DICT 2
 #define AMBC_HUFFMAN 3
 #define AMBC_DELTA 4
+#define AMBC_DEFLATE 5 /* third-party codecs the reference loads from the Python stdlib: decoded only */
+#define AMBC_BZIP2 6
+#define AMBC_LZMA 7
 #define AMBC_RAW 255
 #define AMBC_METHOD_BIT(id) (1u << (id))
 #define AMBC_NATIVE_MASK (AMBC_METHOD_BIT(1) | AMBC_METHOD_BIT(2) | AMBC_METHOD_BIT(3) | AMBC_METHOD_BIT(4))
@@ -147,7 +150,8 @@ typedef struct {
  * Walk the package chain on the host (adaptive_compressor.py:399-430 and the stop
  * rule :444-445): validates markers, stops at END / truncated header / truncated
  * payload.  Raw packages are split into entries of at most 64 KiB.  `known_mask`
- * = method ids present in method_lookup (others are copied through, :432-435).
+ * = method ids present in method_lookup (others are copied through, :432-435):
+ * bits 1-4 the native methods, bit 5 DEFLATE, bit 6 BZIP2, bit 7 LZMA.
  * Pass table=NULL to count entries.  Returns AMBC_E_MARKER on a marker mismatch.
  */
 int ambc_index_host(const uint8_t *body, uint64_t body_len, const uint8_t *marker, uint32_t marker_bytes,
@@ -170,11 +174,22 @@ int ambc_index_dev(const void *body_dev, uint64_t body_len, const uint8_t *marke
  * as adaptive_compressor.py:447-452).  status_dev (optional, uint32[2]):
  * [0] = entries whose codec raised (output zero-filled, :440-442),
  * [1] = entries whose decoded length differed from out_len (malformed stream).
+ * Entries of types 6 (BZIP2) and 7 (LZMA) are left to ambc_decompress_dev_mask.
  */
 int ambc_decompress_dev(const void *body_dev, uint64_t body_len, const ambc_pkg *table_dev, uint64_t n_entries,
                         void *out_dev, uint64_t orig_size, uint32_t *status_dev, void *stream);
+/*
+ * The same, and entries of types 6 / 7 are decoded when known_mask has bit 6 / 7 (pass the
+ * known_mask the table was built with).  Without those bits it is ambc_decompress_dev: the same
+ * kernels, launches and device memory.  The first call with bit 6 allocates 1 GiB of bzip2 block
+ * scratch on the device, kept for later calls.
+ */
+int ambc_decompress_dev_mask(const void *body_dev, uint64_t body_len, const ambc_pkg *table_dev, uint64_t n_entries,
+                             void *out_dev, uint64_t orig_size, uint32_t known_mask, uint32_t *status_dev,
+                             void *stream);
 
-/* host buffers: index walk + H2D + kernels + D2H.  status (optional) as above. */
+/* host buffers: index walk + H2D + kernels + D2H.  status (optional) as above.  Packages of
+ * every type whose bit is in known_mask are decoded, 6 and 7 included. */
 int ambc_decompress_host(const void *body_host, uint64_t body_len, const uint8_t *marker, uint32_t marker_bytes,
                          uint32_t known_mask, void *out_host, uint64_t orig_size, uint32_t *status);
 
@@ -190,6 +205,14 @@ int ambc_decompress_host(const void *body_host, uint64_t body_len, const uint8_t
 /*   zlib stream, pads / truncates to original_length, and returns        */
 /*   original_length zero bytes where zlib.decompress raises (:93-97).    */
 /*   known_mask bit 5 makes packages of type 5 decodable in a body.       */
+/*   methods 6 = BZip2Compression and 7 = LZMACompression, where the      */
+/*   reference calls the stdlib's bz2 / lzma: decode only, with the       */
+/*   semantics of bz2.decompress / lzma.decompress (FORMAT_AUTO: .xz     */
+/*   with a lone LZMA2 filter and a None / CRC32 / CRC64 check, or the    */
+/*   legacy .lzma header; concatenated streams, trailing bytes as the     */
+/*   stdlib treats them); pad / truncate to original_length, zeros where  */
+/*   the stdlib raises.  No encoder: its bytes would not be libbzip2's or */
+/*   liblzma's.  known_mask bits 6 / 7 make such packages decodable.      */
 /* ------------------------------------------------------------------ */
 
 /*
@@ -204,6 +227,11 @@ int ambc_codec_encode_batch(int method, const void *in_dev, const uint64_t *in_o
  * Item i = payload in_dev[in_off[i] .. in_off[i+1]) with original_length
  * orig_len[i]; decoded bytes at out_dev + i*out_stride, out_len[i] = number of
  * bytes the reference's decompress() returns, or AMBC_CODEC_INDEX_ERROR.
+ * Methods 5-7 take payloads and original lengths of any size the stride holds.
+ * Method 7 uses the whole stride as its dictionary: a stream that decodes past
+ * out_stride bytes gets out_len[i] = AMBC_E_CAPACITY (call again with a larger
+ * stride; the bytes behind original_length must be decoded to verify the check).
+ * Method 6 verifies every CRC whatever the stride.
  */
 int ambc_codec_decode_batch(int method, const void *in_dev, const uint64_t *in_off_dev,
                             const uint32_t *orig_len_dev, uint32_t n_items, void *out_dev, uint64_t out_stride,

@@ -11,7 +11,7 @@ import time
 METHOD_TOKENS = {"rle": 1, "dictionary": 2, "dict": 2, "huffman": 3, "delta": 4, "deflate": 5, "bzip2": 6, "lzma": 7,
                  "zstandard": 8, "zstd": 8, "lz4": 9, "brotli": 10, "lzham": 11, "none": 255, "raw": 255}
 METHOD_LABELS = {1: "Run-Length Encoding (RLE)", 2: "Dictionary-Based", 3: "Huffman Coding", 4: "Delta Encoding",
-                 5: "DEFLATE", 255: "No Compression"}
+                 5: "DEFLATE", 6: "BZIP2", 7: "LZMA", 255: "No Compression"}
 
 
 def parse_methods(text):
@@ -116,7 +116,8 @@ def decompress_file(args):
     from adaptive_compression_b200 import AdaptiveCompressor
     print(f"Decompressing {args.input} to {args.output}...")
     try:
-        stats = AdaptiveCompressor().decompress(args.input, args.output)
+        methods = parse_methods(args.methods) if args.methods else None
+        stats = AdaptiveCompressor(methods=methods).decompress(args.input, args.output)
         print("\nDecompression Statistics:")
         print(f"  Compressed size: {stats['compressed_size']} bytes")
         print(f"  Decompressed size: {stats['decompressed_size']} bytes")
@@ -140,7 +141,7 @@ def parse_chunk_size(text):
     return int(t)
 
 
-def main(argv=None):
+def build_parser():
     p = argparse.ArgumentParser(description="Adaptive Marker-Based Compression (B200 chunk path)")
     sub = p.add_subparsers(dest="command", help="Command to execute")
     c = sub.add_parser("compress", help="Compress a file")
@@ -160,8 +161,16 @@ def main(argv=None):
     d.add_argument("input")
     d.add_argument("output")
     d.add_argument("--show-progress", action="store_true")
+    d.add_argument("--methods", default=None,
+                   help="Comma-separated list of the methods the file's packages may use (same tokens as compress; "
+                        "default: the native methods 1-4); e.g. rle,dictionary,huffman,delta,deflate,bzip2,lzma")
     sub.add_parser("analyze", help="(out of scope in this build: plotting)")
     sub.add_parser("gui", help="(out of scope in this build: UI)")
+    return p
+
+
+def main(argv=None):
+    p = build_parser()
     args = p.parse_args(argv)
     if args.command == "compress":
         return compress_file(args)

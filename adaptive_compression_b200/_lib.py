@@ -95,7 +95,6 @@ _SIGS = {
     "ambc_host_alloc": (C.c_void_p, [C.c_uint64]),
     "ambc_host_free": (None, [C.c_void_p]),
     # test hooks (include/ambc.h, last section)
-    "ambc_set_lz_force_buckets": (C.c_int, [C.c_int]),
     "ambc_set_walk_threads": (None, [C.c_uint64, C.c_uint]),
     "ambc_scan_state_bytes": (C.c_uint64, []),
 }

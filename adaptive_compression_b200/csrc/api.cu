@@ -47,10 +47,6 @@ extern "C" int ambc_last_timing(float *ms4)
     return AMBC_OK;
 }
 
-int ambc_lz_force_buckets_codec(int on);
-// test knob: force the window-aware bucket search of the plug-in Dictionary encoder for every chunk size
-extern "C" int ambc_set_lz_force_buckets(int on) { return ambc_lz_force_buckets_codec(on) ? AMBC_E_CUDA : AMBC_OK; }
-
 // fold of the all-gathered placement records (see include/ambc.h; mirrors distributed.fold_placement)
 extern "C" int ambc_shard_place(const ambc_shard_rec *recs, uint32_t n_ranks, const uint64_t *first_byte, uint32_t chunk,
                                 uint32_t marker_bytes, ambc_shard_slot *out)

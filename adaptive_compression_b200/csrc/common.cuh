@@ -7,12 +7,7 @@
 #define AMBC_BLOCK 256              // threads per CTA in the chunk kernels
 #endif
 #define AMBC_WARPS (AMBC_BLOCK / 32)
-#ifndef AMBC_HB
-#define AMBC_HB 10                  // LZ n-gram hash bits
-#endif
-#define AMBC_NBUCKET (1 << AMBC_HB)
 #define AMBC_NMAX 8192              // largest chunk a native method accepts (adaptive_compressor.py:114-127)
-#define AMBC_PAD 64                 // zeroed bytes after the chunk in shared memory
 
 #define FULL_MASK 0xffffffffu
 
@@ -66,20 +61,6 @@ __device__ __forceinline__ int block_sum(int v, volatile int *red)
     if (lane == 0) red[w] = v;
     __syncthreads();
     return warp_sum(lane < AMBC_WARPS ? red[lane] : 0);
-}
-
-__device__ __forceinline__ double block_sum_f64(double v, volatile double *red)
-{
-    int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(FULL_MASK, v, d);
-    __syncthreads();
-    if (lane == 0) red[w] = v;
-    __syncthreads();
-    double tot = 0.0;
-#pragma unroll
-    for (int i = 0; i < AMBC_WARPS; i++) tot += red[i]; // fixed order: the same sum in every thread
-    return tot;
 }
 
 // 16 bytes starting Q words + r bits into the eight words of two consecutive aligned 16-byte loads

@@ -1,7 +1,8 @@
 // select_fast.cuh -- the chunk trial / select step (adaptive_compressor.py:537-590) for chunks of at most
-// NMAX bytes, round-2 design: one CTA of 128 threads per chunk, ~38 KB of shared memory, five CTAs per SM.
+// NMAX bytes: one CTA of 128 threads per chunk, ~38 KB of shared memory, five CTAs per SM.  The plug-in batch
+// kernels (codec_batch.cu) run the same encoders and gates on items of any size up to NMAX.
 //
-// What changed against chunk_codec.cuh / lz_names.cuh (round 1), and why:
+// Design choices, and why:
 //   * The Dictionary trial (compression_methods.py:195-234, 283-313) no longer computes the longest match of
 //     all n positions.  The greedy parse visits a few hundred of them, so the match search is LAZY:
 //       1. positions are bucket-sorted by a hash of their 3 bytes (stable, ascending inside a bucket): one
@@ -69,6 +70,11 @@ template <int NMAX> struct SfCfg {
     static constexpr int OFF_A = OFF_SD + NMAX + SF_PAD;
     static constexpr int OFF_ORD = OFF_A + A_BYTES;           // ord (u16 per position) | payload buffer
     static constexpr int OFF_BSTART = OFF_ORD + NMAX * 2;
+    // payload capacity.  Any payload of n <= NMAX bytes fits: RLE emits at most a 2-byte pair per byte (2n), the
+    // Dictionary 2 bytes per literal or 4 per match of >= 3 bytes (2n), Huffman at most 1 + 5 * 255 + 4 + n bytes
+    // (K <= 255, and the reference's tree is optimal, so it is no longer than a flat 8-bit code).
+    static constexpr int PAY_BYTES = 2 * NMAX;
+    static_assert(PAY_BYTES == OFF_BSTART - OFF_ORD, "the payload overlays ord");
     static constexpr int OFF_BITS = OFF_BSTART + (((NB + 1) * 2 + 15) & ~15);
     static constexpr int OFF_HIST = OFF_BITS + NWORDS * 4; // (only the run-boundary bitmap lives outside region A)
     static constexpr int OFF_HCODE = OFF_HIST + 1024;
@@ -312,7 +318,7 @@ template <int NMAX> __device__ inline int sf_rle_emit(SfCtx<NMAX> &c)
             const uint8_t v = c.sd[p];
             while (R > 0) {
                 const int cnt = R > 255 ? 255 : R;
-                if (off + 2 <= NMAX) { c.pay[off] = v; c.pay[off + 1] = (uint8_t)cnt; }
+                if (off + 2 <= SfCfg<NMAX>::PAY_BYTES) { c.pay[off] = v; c.pay[off + 1] = (uint8_t)cnt; }
                 off += 2;
                 R -= cnt;
             }
@@ -561,13 +567,13 @@ template <int NMAX> __device__ inline int sf_huff_emit(SfCtx<NMAX> &c, SfHuff &h
     if (tid == 0) c.pay[0] = (uint8_t)K;
     for (int r = tid; r < K; r += SF_T) {
         const int o = 1 + 5 * r;
-        if (o + 5 <= NMAX) {
+        if (o + 5 <= SfCfg<NMAX>::PAY_BYTES) {
             const int sym = h.order[r];
             c.pay[o] = (uint8_t)sym;
             store_u32le(c.pay + o + 1, c.hist[sym]);
         }
     }
-    if (tid == 0 && hdr <= NMAX) store_u32le(c.pay + hdr - 4, (uint32_t)total_bits);
+    if (tid == 0 && hdr <= SfCfg<NMAX>::PAY_BYTES) store_u32le(c.pay + hdr - 4, (uint32_t)total_bits);
     const int nwords = (total_bits + 31) >> 5;
     const int wcap = min(nwords, NMAX / 4 + 1);
     for (int i = tid; i < wcap; i += SF_T) h.bw[i] = 0;
@@ -620,7 +626,7 @@ template <int NMAX> __device__ inline int sf_huff_emit(SfCtx<NMAX> &c, SfHuff &h
     }
     __syncthreads();
     for (int k = tid; k < nbytes; k += SF_T)
-        if (hdr + k < NMAX) c.pay[hdr + k] = (uint8_t)(h.bw[k >> 2] >> (24 - 8 * (k & 3)));
+        if (hdr + k < SfCfg<NMAX>::PAY_BYTES) c.pay[hdr + k] = (uint8_t)(h.bw[k >> 2] >> (24 - 8 * (k & 3)));
     __syncthreads();
     return hdr + nbytes;
 }
@@ -1139,7 +1145,7 @@ template <int NMAX> __device__ inline void sf_lz_emit(SfCtx<NMAX> &c)
             reach &= reach - 1;
             const int p = 32 * wd + bit;
             if ((mm >> bit) & 1u) {
-                if (off + 4 <= NMAX) {
+                if (off + 4 <= C::PAY_BYTES) {
                     const uint32_t v = mm16[p];
                     const int d = (int)(v & 0xFFFu) + 1;
                     const int L = 3 + (int)(v >> 12) + (((c.lenhi[wd] >> bit) & 1u) ? 16 : 0);
@@ -1148,12 +1154,11 @@ template <int NMAX> __device__ inline void sf_lz_emit(SfCtx<NMAX> &c)
                 }
                 off += 4;
             } else {
-                if (off + 2 <= NMAX) pay16[off >> 1] = (uint16_t)((uint32_t)c.sd[p] << 8);
+                if (off + 2 <= C::PAY_BYTES) pay16[off >> 1] = (uint16_t)((uint32_t)c.sd[p] << 8);
                 off += 2;
             }
         }
     }
-    (void)C::NB;
     __syncthreads();
 }
 

@@ -315,13 +315,10 @@ int ambc_shard_place(const ambc_shard_rec *recs, uint32_t n_ranks, const uint64_
  * time (different devices may be driven concurrently, one thread each). */
 
 /* ---- test hooks (exported, not part of the reference-facing surface) ----------------------------------
- * ambc_set_lz_force_buckets(1) makes the Dictionary encoder of ambc_codec_encode_batch use its window-aware
- * bucket search for every item size (otherwise it serves items above 4096 bytes and overflowed name tables),
- * so that tests reach that search with small inputs; ambc_set_walk_threads lets small bodies exercise the helper threads of
- * ambc_index_host (min_bytes = body size from which helpers start, threads = 0 for the host cores divided by
- * LOCAL_WORLD_SIZE, at most 8); ambc_scan_state_bytes = size of the per-piece state record ambc_compress_host
- * downloads.  None of them changes any result. */
-int ambc_set_lz_force_buckets(int on);
+ * ambc_set_walk_threads lets small bodies exercise the helper threads of ambc_index_host (min_bytes = body size
+ * from which helpers start, threads = 0 for the host cores divided by LOCAL_WORLD_SIZE, at most 8);
+ * ambc_scan_state_bytes = size of the per-piece state record ambc_compress_host downloads.  None of them changes
+ * any result. */
 void ambc_set_walk_threads(uint64_t min_bytes, unsigned threads);
 uint64_t ambc_scan_state_bytes(void);
 

@@ -70,9 +70,21 @@ def test_gates_codec_cases(eng, golden):
     assert not bad, bad
 
 
+def _capacity_case(mid, n):
+    """an input whose payload reaches the top of the encoders' payload capacity (2 * 8192 bytes)"""
+    r = np.random.RandomState(n)
+    if mid == 1:  # no two equal neighbours: one pair per byte, 2n bytes
+        a = np.cumsum(r.randint(1, 256, size=n)) % 256
+    elif mid == 2:  # random bytes: (almost) only literals, about 2n bytes
+        a = r.randint(0, 256, size=n)
+    else:  # exactly 255 values, near uniform: an 8-bit code, about 1280 + n bytes
+        a = r.permutation(np.arange(n) % 255)
+    return bytes(a.astype(np.uint8))
+
+
 @pytest.mark.parametrize("mid", [1, 2, 3, 4])
 def test_encode_fuzz_vs_oracle(eng, mid):
-    """seeded inputs of every kind and many sizes: CUDA payload == oracle payload"""
+    """seeded inputs of every kind and many sizes, and the largest payloads: CUDA payload == oracle payload"""
     r = np.random.RandomState(100 + mid)
     kinds = sorted(inputs.KINDS)
     datas = []
@@ -87,6 +99,7 @@ def test_encode_fuzz_vs_oracle(eng, mid):
             a[m] = r.randint(0, 256, size=int(m.sum()))
             d = a.tobytes()
         datas.append(d)
+    datas += [_capacity_case(mid, n) for n in (4096, 4097, 8192)]
     got = eng.codec_encode_batch(mid, datas)
     bad = []
     for i, (d, g) in enumerate(zip(datas, got)):
@@ -166,19 +179,12 @@ def test_decode_corrupted_fuzz(eng):
     assert not bad, bad[:20]
 
 
-def test_encode_lz_bucket_search_fallback(eng):
-    """the window-aware bucket search (chunks > 4096 bytes, and the fallback of the names search)
-    forced for every size: same payloads as the oracle"""
-    from adaptive_compression_b200 import _lib as L
-    lib = L.lib()
+def test_encode_dictionary_seeded_sizes(eng):
+    """Dictionary items of 3, 100, 1000 and 4096 bytes of every kind: same payloads as the oracle"""
     r = np.random.RandomState(555)
     kinds = sorted(inputs.KINDS)
     datas = [inputs.make(kinds[r.randint(len(kinds))], int(r.choice([3, 100, 1000, 4096])), 50000 + i) for i in range(60)]
-    assert lib.ambc_set_lz_force_buckets(1) == 0
-    try:
-        got = eng.codec_encode_batch(2, datas)
-    finally:
-        assert lib.ambc_set_lz_force_buckets(0) == 0
+    got = eng.codec_encode_batch(2, datas)
     bad = [(i, len(d)) for i, (d, g) in enumerate(zip(datas, got)) if g != O.compress(2, d, lz_fast=True)]
     assert not bad, bad
 

@@ -46,6 +46,22 @@ class Pkg(C.Structure):
                 ("orig_len", C.c_uint32), ("type", C.c_uint32), ("out_len", C.c_uint32)]
 
 
+class RangeState(C.Structure):
+    """ambc_range_state: the walk's state handed from one body range to the next"""
+    _fields_ = [("next_pos", C.c_uint64), ("out_before", C.c_uint64), ("pkg_pos", C.c_uint64), ("pkg_out", C.c_uint64),
+                ("pkg_type", C.c_uint32), ("pkg_orig", C.c_uint32), ("pkg_comp", C.c_uint32), ("status", C.c_uint32)]
+
+
+class Range(C.Structure):
+    """ambc_range: what one rank holds after ambc_range_index"""
+    _fields_ = [("lo", C.c_uint64), ("hi", C.c_uint64), ("body_len", C.c_uint64), ("orig_size", C.c_uint64),
+                ("n_cand", C.c_uint64), ("work_bytes", C.c_uint64), ("work_dev", C.c_void_p),
+                ("marker_bytes", C.c_uint32), ("known_mask", C.c_uint32), ("levels", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+RANGE_NO_PKG = (1 << 64) - 1
+RANGE_RUNNING, RANGE_END, RANGE_TRUNCATED, RANGE_COMPLETE, RANGE_MARKER = 0, 1, 2, 3, 4
+
 _lib = None
 
 _SIGS = {
@@ -69,6 +85,14 @@ _SIGS = {
                                   C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "ambc_index_dev": (C.c_int, [C.c_void_p, C.c_uint64, C.c_char_p, C.c_uint32, C.c_uint64, C.c_uint32,
                                  C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_void_p]),
+    "ambc_range_workspace_bytes": (C.c_uint64, [C.c_uint64, C.c_uint64]),
+    "ambc_range_index": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_char_p, C.c_uint32,
+                                   C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint64, C.POINTER(Range), C.c_void_p]),
+    "ambc_range_fold": (C.c_int, [C.POINTER(Range), C.POINTER(RangeState), C.POINTER(RangeState), C.c_void_p]),
+    "ambc_range_table": (C.c_int, [C.POINTER(Range), C.POINTER(RangeState), C.c_void_p, C.c_uint64,
+                                   C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64),
+                                   C.POINTER(C.c_uint64), C.c_void_p]),
+    "ambc_range_out_offset": (C.c_uint64, [C.POINTER(RangeState), C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32]),
     "ambc_decompress_dev": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64,
                                       C.c_void_p, C.c_void_p]),
     "ambc_decompress_dev_mask": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64,

@@ -449,3 +449,420 @@ extern "C" int ambc_index_dev(const void *body_dev, uint64_t body_len, const uin
     }
     return AMBC_OK;
 }
+
+// ==== range-local index (ambc_range_*): one rank's byte range [lo, hi) of the body ============================
+// The walk above, split across ranks.  Candidates are the marker occurrences that start in [lo, hi); nodes
+// M (stop) and M + 1 (marker mismatch) are those of k_idx_link, node M + 2 is an exit: the successor lies at
+// or beyond hi, in a later range.  Next to J[k] = succ^(2^k) the range keeps S[k][i] = output bytes of the
+// 2^k packages from node i on (the k_idx_nominal rule), so that one lifting pass from any candidate finds
+// where the chain leaves the range or where the walk ends (the stop rule :444-445 included), and how many
+// output bytes lie on the way.  The fold (k_rng_fold) runs that pass from the state the previous range
+// handed on; ambc_range_table lists the chain from there and places every entry with global output offsets.
+#define RNG_EXIT(M) ((uint32_t)(M) + 2u)
+
+struct RngGeo { // body positions are global
+    uint64_t lo, hi, body_len, orig_size;
+    uint32_t mb, known_mask;
+};
+struct RngShare { uint64_t a, b; };
+
+__host__ __device__ __forceinline__ uint64_t rng_min(uint64_t x, uint64_t y) { return x < y ? x : y; }
+__host__ __device__ __forceinline__ uint64_t rng_nominal(uint32_t type, uint32_t known_mask, uint32_t comp, uint32_t orig)
+{
+    const bool known = type == 255 || (type < 32 && ((known_mask >> type) & 1u));
+    if (!known) return comp;
+    if (type == 255) return orig;
+    if (type == 4) return comp == 0 ? 0 : (comp < orig ? comp : orig);
+    return comp == 0 ? 0 : orig;
+}
+__host__ __device__ __forceinline__ bool rng_copied(uint32_t type, uint32_t known_mask)
+{
+    return type == 255 || !(type < 32 && ((known_mask >> type) & 1u));
+}
+// bytes the walk emits for a package with `nominal` output bytes at output offset o
+__host__ __device__ __forceinline__ uint64_t rng_emit(uint64_t nominal, uint64_t o, uint64_t orig_size)
+{
+    return rng_min(nominal, orig_size > o ? orig_size - o : 0);
+}
+// the output bytes [a, b) of a copied-through package (payload at body position pay) that the range [lo, hi)
+// owns: the payload bytes it holds, plus the zero pad when it holds the payload's last byte; the range that
+// holds the header owns everything before its end.
+__host__ __device__ __forceinline__ RngShare rng_share(uint64_t pay, uint64_t comp, uint64_t emit, uint64_t lo, uint64_t hi,
+                                                       bool header_here)
+{
+    RngShare s;
+    s.a = s.b = 0;
+    if (!header_here && pay + comp <= lo) return s; // the payload ended in an earlier range
+    s.a = header_here ? 0 : rng_min(lo > pay ? lo - pay : 0, emit);
+    s.b = pay + comp <= hi ? emit : rng_min(hi > pay ? hi - pay : 0, emit);
+    if (s.b < s.a) s.b = s.a;
+    return s;
+}
+// first output byte owned by the range starting at body position lo, given the state handed to it
+static uint64_t rng_out_offset(const ambc_range_state &s, uint64_t lo, uint64_t orig_size, uint32_t mb, uint32_t known_mask)
+{
+    if (s.pkg_pos != AMBC_RANGE_NO_PKG && rng_copied(s.pkg_type, known_mask)) {
+        const uint64_t pay = s.pkg_pos + mb + 14;
+        if (pay + s.pkg_comp > lo) {
+            const uint64_t emit = rng_emit(rng_nominal(s.pkg_type, known_mask, s.pkg_comp, s.pkg_orig), s.pkg_out, orig_size);
+            return rng_min(s.pkg_out + rng_share(pay, s.pkg_comp, emit, lo, ~0ull, false).a, orig_size);
+        }
+    }
+    return rng_min(s.out_before, orig_size);
+}
+
+__global__ void __launch_bounds__(256)
+k_rng_link(const uint8_t *__restrict__ buf, RngGeo g, const unsigned long long *__restrict__ cand, uint32_t M, IdxRec *rec,
+           uint32_t *succ, unsigned long long *sum)
+{
+    const uint32_t i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= M + 3) return;
+    if (i >= M) { succ[i] = i; sum[i] = 0; return; } // absorbing
+    const uint64_t hdr = g.mb + 14, p = cand[i], pos = g.lo + p;
+    IdxRec r;
+    r.orig = r.comp = 0; r.type = 0; r.kind = 0; r.pad = 0;
+    uint32_t sx = IDX_STOP(M);
+    if (pos + hdr > g.body_len) r.kind = 2;                           // :400-403
+    else {
+        r.type = buf[p + g.mb];
+        uint32_t o = 0, c = 0;
+        for (int k = 0; k < 4; k++) { o |= (uint32_t)buf[p + g.mb + 6 + k] << (8 * k); c |= (uint32_t)buf[p + g.mb + 10 + k] << (8 * k); }
+        r.orig = o; r.comp = c;
+        const uint64_t nxt = pos + hdr + c;
+        if (r.type == 0) r.kind = 1;                                    // :422-424
+        else if (nxt > g.body_len) r.kind = 3;                          // :425-427
+        else if (nxt + hdr > g.body_len) sx = IDX_STOP(M);              // the next iteration stops at :400-403
+        else if (nxt >= g.hi) sx = RNG_EXIT(M);                         // a later range continues
+        else {
+            const uint64_t want = nxt - g.lo;
+            uint32_t lo = i + 1, hi = M;
+            while (lo < hi) { const uint32_t mid = lo + (hi - lo) / 2; if (cand[mid] < want) lo = mid + 1; else hi = mid; }
+            sx = (lo < M && cand[lo] == want) ? lo : IDX_ERR(M);        // :405-407
+        }
+    }
+    rec[i] = r;
+    succ[i] = sx;
+    sum[i] = r.kind == 0 ? rng_nominal(r.type, g.known_mask, r.comp, r.orig) : 0;
+}
+__global__ void __launch_bounds__(256)
+k_rng_jump(const uint32_t *__restrict__ pj, const unsigned long long *__restrict__ ps, uint32_t *nj, unsigned long long *ns, uint32_t n)
+{
+    const uint32_t i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t a = pj[i];
+    nj[i] = pj[a];
+    ns[i] = ps[i] + ps[a];
+}
+// one fold step.  walk[0] = chain length in this range from the entry (0: the walk does not pass here),
+// walk[1] = entry node, walk[2] = last node, walk[3] = output offset of the last node
+__global__ void k_rng_fold(const unsigned long long *__restrict__ cand, const IdxRec *__restrict__ rec, const uint32_t *__restrict__ J,
+                           const unsigned long long *__restrict__ S, uint32_t n, int K, uint32_t M, RngGeo g,
+                           const ambc_range_state *in, ambc_range_state *out, unsigned long long *walk)
+{
+    if (threadIdx.x || blockIdx.x) return;
+    ambc_range_state s = *in;
+    walk[0] = 0; walk[1] = walk[2] = M; walk[3] = 0;
+    if (s.status != AMBC_RANGE_RUNNING || s.next_pos < g.lo || s.next_pos >= g.hi) { *out = s; return; }
+    const uint64_t hdr = g.mb + 14, x = s.next_pos - g.lo;
+    uint32_t a = 0, b = M;
+    while (a < b) { const uint32_t mid = a + (b - a) / 2; if (cand[mid] < x) a = mid + 1; else b = mid; }
+    s.pkg_pos = AMBC_RANGE_NO_PKG;
+    if (a == M || cand[a] != x) { // no marker here: the walk stops (:400-403) or raises (:405-407)
+        s.status = s.next_pos + hdr > g.body_len ? AMBC_RANGE_TRUNCATED : AMBC_RANGE_MARKER;
+        *out = s;
+        return;
+    }
+    uint32_t node = a;
+    unsigned long long acc = s.out_before, steps = 0;
+    for (int k = K - 1; k >= 0; k--) {
+        const uint64_t at = (uint64_t)k * n + node;
+        if (J[at] < M && acc + S[at] < g.orig_size) { acc += S[at]; node = J[at]; steps += 1ull << k; }
+    }
+    walk[0] = steps + 1; walk[1] = a; walk[2] = node; walk[3] = acc;
+    const IdxRec r = rec[node];
+    s.out_before = acc + S[node];
+    if (r.kind == 1) s.status = AMBC_RANGE_END;
+    else if (r.kind != 0) s.status = AMBC_RANGE_TRUNCATED;
+    else {
+        const uint64_t pos = g.lo + cand[node], end = pos + hdr + r.comp;
+        if (end > g.hi) { s.pkg_pos = pos; s.pkg_out = acc; s.pkg_type = r.type; s.pkg_orig = r.orig; s.pkg_comp = r.comp; }
+        const uint32_t sx = J[node];
+        if (s.out_before >= g.orig_size) s.status = AMBC_RANGE_COMPLETE; // :444-445 before the next header is read
+        else if (sx == IDX_STOP(M)) s.status = AMBC_RANGE_TRUNCATED;
+        else if (sx == IDX_ERR(M)) s.status = AMBC_RANGE_MARKER;
+        else s.next_pos = end;                                            // exit: a later range holds it
+    }
+    *out = s;
+}
+__global__ void __launch_bounds__(256)
+k_rng_chain(const uint32_t *__restrict__ J, uint32_t n, int K, uint32_t entry, uint64_t chain_len, uint32_t *chain)
+{
+    const uint64_t r = (uint64_t)blockIdx.x * 256 + threadIdx.x;
+    if (r >= chain_len) return;
+    uint32_t node = entry;
+    for (int k = 0; k < K; k++)
+        if ((r >> k) & 1) node = J[(uint64_t)k * n + node];
+    chain[r] = node;
+}
+__device__ __forceinline__ void rng_put_pieces(ambc_pkg *table, uint64_t at, uint64_t pay, uint32_t comp, RngShare sh, uint64_t o,
+                                               uint64_t lo, uint64_t out_lo)
+{
+    for (uint64_t done = sh.a; done < sh.b; done += IDX_RAW_PIECE, at++) {
+        const uint64_t piece = rng_min(sh.b - done, IDX_RAW_PIECE), have = comp > done ? comp - done : 0;
+        ambc_pkg e;
+        e.src_off = pay - lo + done; e.dst_off = o + done - out_lo;
+        e.comp_len = (uint32_t)rng_min(have, piece);
+        e.orig_len = (uint32_t)piece; e.type = 255; e.out_len = (uint32_t)piece;
+        table[at] = e;
+    }
+}
+// WRITE == false: ecount[r] = entries of chain node r; WRITE == true: write them at base + ebase[r]
+template <bool WRITE>
+__global__ void __launch_bounds__(256)
+k_rng_entries(const IdxRec *__restrict__ rec, const uint32_t *__restrict__ chain, const unsigned long long *__restrict__ cand,
+              const unsigned long long *__restrict__ nominal, const unsigned long long *__restrict__ obefore, uint64_t chain_len,
+              uint64_t out0, RngGeo g, unsigned long long *ecount, const unsigned long long *__restrict__ ebase, uint64_t base,
+              uint64_t out_lo, ambc_pkg *table)
+{
+    const uint64_t r = (uint64_t)blockIdx.x * 256 + threadIdx.x;
+    if (r >= chain_len) return;
+    const IdxRec x = rec[chain[r]];
+    const uint64_t o = out0 + obefore[r], emit = x.kind == 0 ? rng_emit(nominal[r], o, g.orig_size) : 0;
+    const uint64_t pay = g.lo + cand[chain[r]] + g.mb + 14;
+    const bool copied = rng_copied(x.type, g.known_mask);
+    const RngShare sh = rng_share(pay, x.comp, emit, g.lo, g.hi, true);
+    if (!WRITE) {
+        ecount[r] = emit == 0 ? 0 : copied ? (sh.b - sh.a + IDX_RAW_PIECE - 1) / IDX_RAW_PIECE : 1;
+        return;
+    }
+    if (emit == 0) return;
+    if (copied) {
+        rng_put_pieces(table, base + ebase[r], pay, x.comp, sh, o, g.lo, out_lo);
+    } else {
+        ambc_pkg e;
+        e.src_off = pay - g.lo; e.dst_off = o - out_lo; e.comp_len = x.comp; e.orig_len = x.orig; e.type = x.type;
+        e.out_len = (uint32_t)emit;
+        table[base + ebase[r]] = e;
+    }
+}
+// the pieces of a copied-through package whose header lies in an earlier range
+__global__ void __launch_bounds__(256)
+k_rng_inbound(uint64_t pay, uint32_t comp, RngShare sh, uint64_t o, uint64_t lo, uint64_t out_lo, ambc_pkg *table)
+{
+    const uint64_t j = (uint64_t)blockIdx.x * 256 + threadIdx.x;
+    const uint64_t a = sh.a + j * IDX_RAW_PIECE;
+    if (a >= sh.b) return;
+    RngShare one;
+    one.a = a; one.b = rng_min(sh.b, a + IDX_RAW_PIECE);
+    rng_put_pieces(table, j, pay, comp, one, o, lo, out_lo);
+}
+
+struct RngLayout {
+    uint64_t tile_cnt, tile_base, sc, total, cand, rec, J, S, chain, nom, ob, ec, eb, sct, info, bytes;
+    uint32_t n;
+    int K;
+};
+static RngLayout rng_layout(uint64_t range_len, uint64_t M)
+{
+    RngLayout l;
+    const uint64_t n_tiles = (range_len + 3 + IDX_TILE - 1) / IDX_TILE; // the scan covers at most range_len + 3 bytes
+    l.n = (uint32_t)(M + 3);
+    l.K = 1;
+    while ((1ull << l.K) <= M) l.K++;
+    uint64_t off = 0;
+    auto take = [&](uint64_t bytes) { uint64_t r = off; off += (bytes + 255) & ~255ull; return r; };
+    l.tile_cnt = take((n_tiles + 1) * 8); l.tile_base = take((n_tiles + 1) * 8);
+    l.sc = take(((n_tiles + SC_TILE) / SC_TILE + 1) * 8); l.total = take(8);
+    l.cand = take(M * 8); l.rec = take(M * sizeof(IdxRec)); l.J = take((uint64_t)l.K * l.n * 4); l.S = take((uint64_t)l.K * l.n * 8);
+    l.chain = take(M * 4); l.nom = take(M * 8); l.ob = take(M * 8); l.ec = take(M * 8); l.eb = take(M * 8);
+    l.sct = take(((M + SC_TILE) / SC_TILE + 2) * 8); l.info = take(256);
+    l.bytes = off;
+    return l;
+}
+// info area: [0, 48) state in, [64, 112) state out, [128, 160) walk, [160, 192) scan totals
+#define RNG_IN 0
+#define RNG_OUT 64
+#define RNG_WALK 128
+#define RNG_TOT 160
+
+extern "C" uint64_t ambc_range_workspace_bytes(uint64_t range_len, uint64_t n_cand)
+{
+    return rng_layout(range_len, n_cand).bytes;
+}
+
+extern "C" uint64_t ambc_range_out_offset(const ambc_range_state *s, uint64_t lo, uint64_t orig_size, uint32_t mb,
+                                          uint32_t known_mask)
+{
+    return s ? rng_out_offset(*s, lo, orig_size, mb, known_mask) : 0;
+}
+
+static RngGeo rng_geo(const ambc_range *r)
+{
+    RngGeo g;
+    g.lo = r->lo; g.hi = r->hi; g.body_len = r->body_len; g.orig_size = r->orig_size; g.mb = r->marker_bytes;
+    g.known_mask = r->known_mask;
+    return g;
+}
+
+extern "C" int ambc_range_index(const void *buf_dev, uint64_t buf_len, uint64_t lo, uint64_t hi, uint64_t body_len,
+                                const uint8_t *marker, uint32_t mb, uint64_t orig_size, uint32_t known_mask, void *work_dev,
+                                uint64_t work_bytes, ambc_range *r, void *stream_)
+{
+    cudaStream_t s = (cudaStream_t)stream_;
+    if (!r || !marker || mb < 1 || mb > 4 || lo > hi || hi > body_len || (buf_len && !buf_dev))
+        return ambc_fail(AMBC_E_ARG, "ambc_range_index: bad argument");
+    const uint64_t halo_end = rng_min(hi + mb + 13, body_len);
+    if (lo + buf_len < halo_end) return ambc_fail(AMBC_E_ARG, "ambc_range_index: buffer ends before the header halo");
+    r->lo = lo; r->hi = hi; r->body_len = body_len; r->orig_size = orig_size; r->n_cand = 0;
+    r->work_dev = work_dev; r->marker_bytes = mb; r->known_mask = known_mask; r->levels = 1; r->reserved = 0;
+    const uint64_t R = hi - lo;
+    RngLayout l = rng_layout(R, 0);
+    r->work_bytes = l.bytes;
+    if (!work_dev || work_bytes < l.bytes) return ambc_fail(AMBC_E_CAPACITY, "ambc_range_index: workspace too small");
+    uint32_t marker_word = 0;
+    for (uint32_t k = 0; k < mb; k++) marker_word |= (uint32_t)marker[k] << (8 * k);
+    const uint8_t *buf = (const uint8_t *)buf_dev;
+    uint8_t *W = (uint8_t *)work_dev;
+    // candidates: marker occurrences that start in [lo, hi)
+    const uint64_t scan_len = R ? rng_min(buf_len, R + mb - 1) : 0, n_tiles = (scan_len + IDX_TILE - 1) / IDX_TILE;
+    unsigned long long *tile_cnt = (unsigned long long *)(W + l.tile_cnt), *tile_base = (unsigned long long *)(W + l.tile_base);
+    uint64_t M64 = 0;
+    int rc;
+    if (n_tiles) {
+        k_idx_scan<false><<<(unsigned)n_tiles, IDX_THREADS, 0, s>>>(buf, scan_len, marker_word, mb, tile_cnt, nullptr, nullptr);
+        ambc_count_launch();
+        unsigned long long *d_total = (unsigned long long *)(W + l.total);
+        if ((rc = dev_excl_scan(tile_cnt, n_tiles, tile_base, (unsigned long long *)(W + l.sc), d_total, s))) return rc;
+        unsigned long long h_total = 0;
+        CUDA_TRY(cudaMemcpyAsync(&h_total, d_total, 8, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(cudaStreamSynchronize(s));
+        M64 = h_total;
+    }
+    if (M64 > 0x7FFFFFF0ull) return ambc_fail(AMBC_E_CAPACITY, "ambc_range_index: too many marker occurrences");
+    l = rng_layout(R, M64);
+    r->n_cand = M64;
+    r->work_bytes = l.bytes;
+    r->levels = (uint32_t)l.K;
+    if (work_bytes < l.bytes) return ambc_fail(AMBC_E_CAPACITY, "ambc_range_index: workspace too small (%llu bytes)", (unsigned long long)l.bytes);
+    const uint32_t M = (uint32_t)M64, n = l.n;
+    unsigned long long *cand = (unsigned long long *)(W + l.cand), *S = (unsigned long long *)(W + l.S);
+    uint32_t *J = (uint32_t *)(W + l.J);
+    if (M) {
+        k_idx_scan<true><<<(unsigned)n_tiles, IDX_THREADS, 0, s>>>(buf, scan_len, marker_word, mb, nullptr, tile_base, cand);
+        ambc_count_launch();
+    }
+    k_rng_link<<<(n + 255) / 256, 256, 0, s>>>(buf, rng_geo(r), cand, M, (IdxRec *)(W + l.rec), J, S);
+    ambc_count_launch();
+    for (int k = 1; k < l.K; k++) {
+        k_rng_jump<<<(n + 255) / 256, 256, 0, s>>>(J + (uint64_t)(k - 1) * n, S + (uint64_t)(k - 1) * n, J + (uint64_t)k * n,
+                                                    S + (uint64_t)k * n, n);
+        ambc_count_launch();
+    }
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaStreamSynchronize(s));
+    return AMBC_OK;
+}
+
+// the fold step on the device; leaves the walk record in the info area
+static int rng_fold(const ambc_range *r, const ambc_range_state *in, ambc_range_state *out, unsigned long long *walk,
+                    cudaStream_t s)
+{
+    if (!r || !in || !r->work_dev) return ambc_fail(AMBC_E_ARG, "ambc_range: bad argument");
+    const RngLayout l = rng_layout(r->hi - r->lo, r->n_cand);
+    uint8_t *W = (uint8_t *)r->work_dev;
+    ambc_range_state *d_in = (ambc_range_state *)(W + l.info + RNG_IN), *d_out = (ambc_range_state *)(W + l.info + RNG_OUT);
+    unsigned long long *d_walk = (unsigned long long *)(W + l.info + RNG_WALK);
+    CUDA_TRY(cudaMemcpyAsync(d_in, in, sizeof(ambc_range_state), cudaMemcpyHostToDevice, s));
+    k_rng_fold<<<1, 1, 0, s>>>((const unsigned long long *)(W + l.cand), (const IdxRec *)(W + l.rec), (const uint32_t *)(W + l.J),
+                               (const unsigned long long *)(W + l.S), l.n, l.K, (uint32_t)r->n_cand, rng_geo(r), d_in, d_out, d_walk);
+    ambc_count_launch();
+    CUDA_TRY(cudaGetLastError());
+    if (out) CUDA_TRY(cudaMemcpyAsync(out, d_out, sizeof(ambc_range_state), cudaMemcpyDeviceToHost, s));
+    if (walk) CUDA_TRY(cudaMemcpyAsync(walk, d_walk, 32, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    return AMBC_OK;
+}
+
+extern "C" int ambc_range_fold(const ambc_range *r, const ambc_range_state *in, ambc_range_state *out, void *stream_)
+{
+    if (!out) return ambc_fail(AMBC_E_ARG, "ambc_range_fold: bad argument");
+    return rng_fold(r, in, out, nullptr, (cudaStream_t)stream_);
+}
+
+extern "C" int ambc_range_table(const ambc_range *r, const ambc_range_state *entry, ambc_pkg *table_dev, uint64_t table_cap,
+                                uint64_t *n_entries, uint64_t *out_lo, uint64_t *out_hi, uint64_t *need, void *stream_)
+{
+    cudaStream_t s = (cudaStream_t)stream_;
+    if (n_entries) *n_entries = 0;
+    if (need) *need = 0;
+    ambc_range_state ex;
+    unsigned long long walk[4] = {0, 0, 0, 0};
+    int rc = rng_fold(r, entry, &ex, walk, s);
+    if (rc) return rc;
+    const RngGeo g = rng_geo(r);
+    const uint64_t hdr = g.mb + 14, lo = g.lo;
+    const uint64_t o_lo = rng_out_offset(*entry, lo, g.orig_size, g.mb, g.known_mask);
+    if (out_lo) *out_lo = o_lo;
+    if (out_hi) *out_hi = rng_out_offset(ex, g.hi, g.orig_size, g.mb, g.known_mask);
+    // a copied-through package whose payload began in an earlier range
+    uint64_t n_in = 0, in_pay = 0;
+    RngShare in_sh = {0, 0};
+    if (entry->pkg_pos != AMBC_RANGE_NO_PKG && rng_copied(entry->pkg_type, g.known_mask)) {
+        in_pay = entry->pkg_pos + hdr;
+        const uint64_t emit = rng_emit(rng_nominal(entry->pkg_type, g.known_mask, entry->pkg_comp, entry->pkg_orig), entry->pkg_out,
+                                       g.orig_size);
+        in_sh = rng_share(in_pay, entry->pkg_comp, emit, lo, g.hi, false);
+        n_in = (in_sh.b - in_sh.a + IDX_RAW_PIECE - 1) / IDX_RAW_PIECE;
+    }
+    const uint64_t chain_len = walk[0];
+    const RngLayout l = rng_layout(g.hi - lo, r->n_cand);
+    uint8_t *W = (uint8_t *)r->work_dev;
+    const IdxRec *rec = (const IdxRec *)(W + l.rec);
+    const unsigned long long *cand = (const unsigned long long *)(W + l.cand);
+    uint32_t *chain = (uint32_t *)(W + l.chain);
+    unsigned long long *nominal = (unsigned long long *)(W + l.nom), *obefore = (unsigned long long *)(W + l.ob);
+    unsigned long long *ecount = (unsigned long long *)(W + l.ec), *ebase = (unsigned long long *)(W + l.eb);
+    unsigned long long *sct = (unsigned long long *)(W + l.sct), *tot = (unsigned long long *)(W + l.info + RNG_TOT);
+    uint64_t n_chain = 0;
+    const unsigned cgrid = (unsigned)((chain_len + 255) / 256);
+    if (chain_len) {
+        k_rng_chain<<<cgrid, 256, 0, s>>>((const uint32_t *)(W + l.J), l.n, l.K, (uint32_t)walk[1], chain_len, chain);
+        k_idx_nominal<<<cgrid, 256, 0, s>>>(rec, chain, chain_len, g.known_mask, nominal);
+        ambc_count_launch(); ambc_count_launch();
+        if ((rc = dev_excl_scan(nominal, chain_len, obefore, sct, tot, s))) return rc;
+        k_rng_entries<false><<<cgrid, 256, 0, s>>>(rec, chain, cand, nominal, obefore, chain_len, entry->out_before, g, ecount,
+                                                    nullptr, 0, 0, nullptr);
+        ambc_count_launch();
+        if ((rc = dev_excl_scan(ecount, chain_len, ebase, sct, tot + 1, s))) return rc;
+        unsigned long long h_tot = 0, h_last = 0;
+        IdxRec last;
+        CUDA_TRY(cudaMemcpyAsync(&h_tot, tot + 1, 8, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(cudaMemcpyAsync(&last, rec + walk[2], sizeof(IdxRec), cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(cudaMemcpyAsync(&h_last, cand + walk[2], 8, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(cudaStreamSynchronize(s));
+        n_chain = h_tot;
+        // a decoded package needs its whole payload, also the part behind the halo
+        if (need && last.kind == 0 && !rng_copied(last.type, g.known_mask) &&
+            rng_emit(rng_nominal(last.type, g.known_mask, last.comp, last.orig), walk[3], g.orig_size)) {
+            const uint64_t end = lo + h_last + hdr + last.comp, have = rng_min(g.hi + g.mb + 13, g.body_len);
+            *need = end > have ? end - have : 0;
+        }
+    }
+    const uint64_t ne = n_in + n_chain;
+    if (n_entries) *n_entries = ne;
+    if (table_dev && ne) {
+        if (ne > table_cap) return ambc_fail(AMBC_E_CAPACITY, "ambc_range_table: table too small (%llu entries)", (unsigned long long)ne);
+        if (n_in) {
+            k_rng_inbound<<<(unsigned)((n_in + 255) / 256), 256, 0, s>>>(in_pay, entry->pkg_comp, in_sh, entry->pkg_out, lo, o_lo, table_dev);
+            ambc_count_launch();
+        }
+        if (n_chain) {
+            k_rng_entries<true><<<cgrid, 256, 0, s>>>(rec, chain, cand, nominal, obefore, chain_len, entry->out_before, g, nullptr,
+                                                       ebase, n_in, o_lo, table_dev);
+            ambc_count_launch();
+        }
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(cudaStreamSynchronize(s));
+    }
+    return AMBC_OK;
+}

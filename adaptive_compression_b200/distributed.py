@@ -1,6 +1,6 @@
 """Multi-GPU sharding of the chunk path (SURVEY.md §8e): contiguous chunk ranges per rank, one
-process per GPU, torch.distributed (NCCL over NVLink; gloo in the CPU tests) for the two tiny
-exchanges the path has:
+process per GPU, torch.distributed (NCCL over NVLink; gloo in the CPU tests) for the tiny exchanges
+the path has:
 
   place_shards        all-gather of one 16-byte record per rank -> every rank folds the
                       "rest of file raw" monoid left to right (adaptive_compressor.py:586-590) and
@@ -8,6 +8,14 @@ exchanges the path has:
                       the raw tail.
   merge_marker_flags  byte-wise MAX all-reduce of the per-shard n-gram presence flags
                       (NCCL has no bitwise OR; flags are 0/1 bytes).
+  decompress_sharded  the way back: every rank holds one byte range of an assembled body
+                      (body_ranges, scatter_body), indexes it on its own GPU (ambc_range_index),
+                      and the package walk (adaptive_compressor.py:396-454) is folded across the
+                      ranges in rank order, one 48-byte state per hop (R - 1 point-to-point
+                      messages).  One all-gather of the entry states tells every rank where its
+                      output slice lies and which copied-through package runs into its range; a
+                      second one of the per-rank tail needs plans the payload bytes a rank fetches
+                      from the next ranks (tail_fetch_plan).  Then every rank decodes its own slice.
 
 A rank compresses its range as if no earlier rank had hit a chunk without a winner; shard_fragment()
 then turns the local body into the bytes this rank contributes to the global body."""
@@ -239,3 +247,158 @@ def find_marker_sharded(t_shard, max_len=32, levels=(16, 24, 32)):
         if rc != L.E_NO_MARKER or Lb == max_len:
             L.check(rc)
     raise ValueError("Could not find a marker of length <= %d bits" % min(max_len, levels[-1]))
+
+
+# ---- sharded decode of one assembled body ---------------------------------------------------------------
+STATE_WORDS = 8  # ambc_range_state as int64 words
+
+
+def body_ranges(body_len, world):
+    """[(lo, hi)] per rank: contiguous byte ranges of about equal size covering [0, body_len)"""
+    return [(body_len * r // world, body_len * (r + 1) // world) for r in range(world)]
+
+
+def range_halo(marker_bytes=4):
+    """header bytes a rank holds behind its range (a header starting at hi - 1 ends at hi + marker_bytes + 13)"""
+    return marker_bytes + 13
+
+
+def buffer_span(lo, hi, body_len, marker_bytes=4):
+    """body bytes [b0, b1) a rank holds for its range [lo, hi): the range and the header halo behind it"""
+    return lo, min(hi + range_halo(marker_bytes), body_len)
+
+
+def tail_fetch_plan(ranges, needs, body_len, marker_bytes=4):
+    """needs[r] = payload bytes rank r's last decoded package needs behind its buffer.  -> [(src, dst, g0, g1)]:
+    rank src sends body[g0, g1) (inside its own range) to rank dst, in a fixed order every rank computes alike"""
+    plan = []
+    for r, ((lo, hi), need) in enumerate(zip(ranges, needs)):
+        if not need:
+            continue
+        f0 = buffer_span(lo, hi, body_len, marker_bytes)[1]
+        f1 = f0 + int(need)
+        for q in range(r + 1, len(ranges)):
+            qlo, qhi = ranges[q]
+            g0, g1 = max(f0, qlo), min(f1, qhi)
+            if g1 > g0:
+                plan.append((q, r, g0, g1))
+    return plan
+
+
+def output_slices(entry_states, ranges, orig_size, marker_bytes=4, known_mask=None):
+    """[(o0, o1)] per rank: the output bytes rank r decodes, from the states the fold handed to every rank.
+    Slices are contiguous in rank order; the last one ends at orig_size (it owns the zero tail)."""
+    from . import _lib as L
+    from . import engine
+    km = L.NATIVE_MASK if known_mask is None else known_mask
+    starts = [engine.range_out_offset(s, lo, orig_size, marker_bytes, km) for s, (lo, _) in zip(entry_states, ranges)]
+    return [(starts[r], starts[r + 1] if r + 1 < len(starts) else orig_size) for r in range(len(starts))]
+
+
+def state_to_words(s):
+    return [int(s.next_pos), int(s.out_before), int(s.pkg_pos) - (1 << 64) if s.pkg_pos >= 1 << 63 else int(s.pkg_pos),
+            int(s.pkg_out), int(s.pkg_type), int(s.pkg_orig), int(s.pkg_comp), int(s.status)]
+
+
+def state_from_words(w):
+    from . import _lib as L
+    return L.RangeState(*[int(x) & ((1 << 64) - 1) for x in w[:4]], *[int(x) & 0xFFFFFFFF for x in w[4:8]])
+
+
+def scatter_body(body, body_len, src=0, marker_bytes=4, device=None):
+    """rank `src` holds the assembled body (None elsewhere); every rank receives buffer_span() of its
+    body_ranges() range (dist.send / recv, as assemble_body).  -> this rank's buffer"""
+    rank, world = dist.get_rank(), dist.get_world_size()
+    ranges = body_ranges(body_len, world)
+    if rank == src:
+        reqs = []
+        for r, (lo, hi) in enumerate(ranges):
+            b0, b1 = buffer_span(lo, hi, body_len, marker_bytes)
+            if r != src and b1 > b0:
+                reqs.append(dist.isend(body[b0:b1].contiguous(), r))
+        for q in reqs:
+            q.wait()
+        b0, b1 = buffer_span(*ranges[rank], body_len, marker_bytes)
+        return body[b0:b1]
+    b0, b1 = buffer_span(*ranges[rank], body_len, marker_bytes)
+    buf = torch.empty(b1 - b0, dtype=torch.uint8, device=device if device is not None else _device())
+    if b1 > b0:
+        dist.recv(buf, src)
+    return buf
+
+
+def decompress_sharded(buf, lo, hi, body_len, orig_size, marker=b"\xff\xff\x00\x00", known_mask=None, gather_to=None):
+    """Decode one .ambc body whose byte ranges are spread over the ranks (body_ranges() order; buf =
+    body[buffer_span(lo, hi)] on this rank's GPU).  Phase 1 indexes the range locally, the fold walks the
+    package chain across the ranges in rank order, every rank fetches the payload bytes its last decoded
+    package needs from the next ranks, lists and decodes its own part.
+    -> (out_offset, output slice, status [codec errors, length mismatches]) of this rank.
+    gather_to=dst: the slices are also sent to rank dst, which returns (0, the whole output, summed status).
+    A marker mismatch the serial walk would hit raises ValueError("Marker mismatch in chunk header.") on
+    every rank."""
+    from . import _lib as L
+    from . import engine
+    km = L.NATIVE_MASK if known_mask is None else known_mask
+    rank, world = dist.get_rank(), dist.get_world_size()
+    mb = len(marker)
+    dev = buf.device
+    ranges = body_ranges(body_len, world)
+    assert ranges[rank] == (lo, hi), "ranges follow body_ranges(body_len, world)"
+    ri = engine.range_index(buf, lo, hi, body_len, orig_size, marker, km)
+    # fold: rank r - 1 -> rank r
+    w = torch.empty(STATE_WORDS, dtype=torch.int64, device=dev)
+    if rank == 0:
+        entry = engine.range_init_state()
+    else:
+        dist.recv(w, rank - 1)
+        entry = state_from_words(w.cpu().tolist())
+    exit_ = engine.range_fold(ri, entry)
+    if rank + 1 < world:
+        dist.send(torch.tensor(state_to_words(exit_), dtype=torch.int64, device=dev), rank + 1)
+    # every rank learns every entry state and the walk's final state
+    mine = torch.tensor(state_to_words(entry) + state_to_words(exit_), dtype=torch.int64, device=dev)
+    allw = torch.empty(2 * STATE_WORDS * world, dtype=torch.int64, device=dev)
+    dist.all_gather_into_tensor(allw, mine)
+    rows = allw.view(world, 2 * STATE_WORDS).cpu().tolist()
+    if int(rows[-1][2 * STATE_WORDS - 1]) == L.RANGE_MARKER:
+        raise ValueError("Marker mismatch in chunk header.")  # adaptive_compressor.py:407
+    entries = [state_from_words(r[:STATE_WORDS]) for r in rows]
+    slices = output_slices(entries, ranges, orig_size, mb, km)
+    o0, o1 = slices[rank]
+    # payload bytes behind the halo
+    _, _, _, _, need = engine.range_table(ri, entry, count_only=True)
+    needs = torch.empty(world, dtype=torch.int64, device=dev)
+    dist.all_gather_into_tensor(needs, torch.tensor([need], dtype=torch.int64, device=dev))
+    plan = tail_fetch_plan(ranges, needs.cpu().tolist(), body_len, mb)
+    if need:
+        grown = torch.empty(buf.numel() + need, dtype=torch.uint8, device=dev)
+        grown[:buf.numel()].copy_(buf)
+        buf = grown
+    reqs = []
+    for src, dst, g0, g1 in plan:
+        if src == rank:
+            reqs.append(dist.isend(buf[g0 - lo:g1 - lo].contiguous(), dst))
+        elif dst == rank:
+            reqs.append(dist.irecv(buf[g0 - lo:g1 - lo], src))
+    for q in reqs:
+        q.wait()
+    t_table, n, _, _, _ = engine.range_table(ri, entry)
+    out, status = engine.range_decode(buf, t_table, n, o1 - o0, km)
+    if gather_to is None:
+        return o0, out, status
+    st = torch.tensor(status, dtype=torch.int64, device=dev)
+    dist.all_reduce(st)
+    if rank != gather_to:
+        if o1 > o0:
+            dist.send(out.contiguous(), gather_to)
+        return o0, out, status
+    whole = torch.empty(max(orig_size, 1), dtype=torch.uint8, device=dev)[:orig_size]
+    reqs = []
+    for r, (a, b) in enumerate(slices):
+        if r == rank:
+            whole[a:b].copy_(out)
+        elif b > a:
+            reqs.append(dist.irecv(whole[a:b], r))
+    for q in reqs:
+        q.wait()
+    return 0, whole, [int(x) for x in st.cpu().tolist()]

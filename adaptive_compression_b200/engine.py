@@ -180,6 +180,82 @@ def decompress_device(t_body, orig_size, marker=FIXED_MARKER, known_mask=L.NATIV
     return out[:orig_size], status.cpu().tolist()
 
 
+# ---- range-local index (ambc_range_*): one byte range [lo, hi) of a body per rank -------------------------
+class RangeIndex:
+    """the phase-1 tables of one range (ambc_range_index) and the workspace that holds them"""
+    __slots__ = ("r", "work", "marker")
+
+
+def range_index(t_buf, lo, hi, body_len, orig_size, marker=FIXED_MARKER, known_mask=L.NATIVE_MASK, work=None):
+    """phase 1 on body[lo, hi): t_buf = body[lo, min(hi + len(marker) + 13, body_len)) (the range and the header
+    halo, distributed.buffer_span) as a device tensor -> RangeIndex"""
+    lib = require_cuda()
+    r = L.Range()
+    guess = int(lib.ambc_range_workspace_bytes(hi - lo, (hi - lo) // 2048 + 64))
+    if work is None or work.numel() < guess:
+        work = torch.empty(guess, dtype=torch.uint8, device="cuda")
+    while True:
+        rc = lib.ambc_range_index(C.c_void_p(t_buf.data_ptr() if t_buf.numel() else 0), t_buf.numel(), lo, hi, body_len,
+                                  marker, len(marker), orig_size, known_mask, C.c_void_p(work.data_ptr()), work.numel(),
+                                  C.byref(r), _stream_ptr())
+        if rc == L.E_CAPACITY and r.work_bytes > work.numel():
+            work = torch.empty(int(r.work_bytes), dtype=torch.uint8, device="cuda")
+            continue
+        L.check(rc)
+        break
+    ri = RangeIndex()
+    ri.r, ri.work, ri.marker = r, work, marker
+    return ri
+
+
+def range_init_state():
+    """the walk's state before body position 0"""
+    return L.RangeState(0, 0, L.RANGE_NO_PKG, 0, 0, 0, 0, L.RANGE_RUNNING)
+
+
+def range_fold(ri, state):
+    """phase 2, one step: the walk's state behind this range given the state before it"""
+    out = L.RangeState()
+    L.check(require_cuda().ambc_range_fold(C.byref(ri.r), C.byref(state), C.byref(out), _stream_ptr()))
+    return out
+
+
+def range_table(ri, entry, count_only=False):
+    """phase 3: -> (uint8 device tensor of 32-byte ambc_pkg entries, n entries, out_lo, out_hi, need).
+    src_off is relative to the range's buffer, dst_off to out_lo; `need` = payload bytes past the halo
+    that the buffer must hold before decoding"""
+    lib = require_cuda()
+    ne, olo, ohi, need = C.c_uint64(0), C.c_uint64(0), C.c_uint64(0), C.c_uint64(0)
+    L.check(lib.ambc_range_table(C.byref(ri.r), C.byref(entry), None, 0, C.byref(ne), C.byref(olo), C.byref(ohi),
+                                 C.byref(need), _stream_ptr()))
+    t_table = torch.empty(max(ne.value, 1) * 32, dtype=torch.uint8, device="cuda")
+    if ne.value and not count_only:
+        L.check(lib.ambc_range_table(C.byref(ri.r), C.byref(entry), C.c_void_p(t_table.data_ptr()), ne.value, C.byref(ne),
+                                     C.byref(olo), C.byref(ohi), C.byref(need), _stream_ptr()))
+    return t_table, ne.value, olo.value, ohi.value, need.value
+
+
+def range_out_offset(state, lo, orig_size, marker_bytes=4, known_mask=L.NATIVE_MASK):
+    """first output byte owned by the range starting at body position lo, given the state the fold handed to it
+    (host arithmetic, no device needed)"""
+    return int(L.lib().ambc_range_out_offset(C.byref(state), lo, orig_size, marker_bytes, known_mask))
+
+
+def range_decode(t_buf, t_table, n_entries, out_len, known_mask=L.NATIVE_MASK, out=None):
+    """decode a range's table into its output slice of out_len bytes -> (slice, status [codec errors, length
+    mismatches]); the zero tail is written when the slice reaches past the last entry"""
+    lib = require_cuda()
+    if out is None or out.numel() < out_len:
+        out = torch.empty(max(out_len, 1), dtype=torch.uint8, device="cuda")
+    status = torch.zeros(2, dtype=torch.int32, device="cuda")
+    L.check(lib.ambc_decompress_dev_mask(C.c_void_p(t_buf.data_ptr() if t_buf.numel() else 0), t_buf.numel(),
+                                         C.c_void_p(t_table.data_ptr() if n_entries else 0), n_entries,
+                                         C.c_void_p(out.data_ptr()), out_len, known_mask, C.c_void_p(status.data_ptr()),
+                                         _stream_ptr()))
+    torch.cuda.current_stream().synchronize()
+    return out[:out_len], status.cpu().tolist()
+
+
 def _pack_items(items):
     offs = np.zeros(len(items) + 1, dtype=np.uint64)
     for i, it in enumerate(items):

@@ -170,6 +170,81 @@ int ambc_index_dev(const void *body_dev, uint64_t body_len, const uint8_t *marke
                    uint64_t *n_entries, uint64_t *out_bytes, void *stream);
 
 /*
+ * Range-local index: the same walk (adaptive_compressor.py:396-454) split across ranks that each
+ * hold one byte range [lo, hi) of the body, so that every GPU indexes and decodes its own range.
+ *
+ *   1. ambc_range_index  (no communication) finds the header candidates in [lo, hi) of the rank's
+ *      buffer, parses them, links every candidate to its successor and builds jump and output-sum
+ *      tables.  A successor at or beyond hi is an exit of the range.
+ *   2. ambc_range_fold   runs once per rank in rank order on the state the previous rank returned
+ *      (the first rank starts from AMBC_RANGE_INIT): a rank whose range holds the next header walks
+ *      its chain to the exit or to the walk's end, every other rank passes the state on unchanged.
+ *   3. ambc_range_table  lists the rank's part of the walk from its entry state (the state the fold
+ *      handed to it) as ambc_pkg entries for ambc_decompress_dev_mask: src_off relative to the rank's
+ *      buffer (= body position - lo), dst_off relative to out_lo.
+ *
+ * Ownership: a decoded package belongs to the rank that holds its header; a copied-through payload
+ * (type 255 and types without a known_mask bit) belongs to whoever holds its bytes, in 64 KiB pieces,
+ * and the zero pad behind it to the rank holding its last payload byte; the zero tail
+ * [covered, orig_size) belongs to the last rank.  Rank r's output slice is [out_lo_r, out_lo_{r+1})
+ * with out_lo_R = orig_size; decode it with ambc_decompress_dev_mask(orig_size = slice length).
+ */
+typedef struct {
+    uint64_t next_pos;   /* body position of the next header on the chain                               */
+    uint64_t out_before; /* output bytes of the walk before it (>= orig_size once complete)           */
+    uint64_t pkg_pos;    /* header position of the package whose payload runs past the range that      */
+                         /* listed it, AMBC_RANGE_NO_PKG if none                                         */
+    uint64_t pkg_out;    /* its output offset                                                         */
+    uint32_t pkg_type, pkg_orig, pkg_comp;
+    uint32_t status;     /* AMBC_RANGE_*                                                              */
+} ambc_range_state;
+#define AMBC_RANGE_NO_PKG (~0ull)
+#define AMBC_RANGE_RUNNING 0   /* the walk continues at next_pos                                        */
+#define AMBC_RANGE_END 1       /* END package (:422-424)                                                */
+#define AMBC_RANGE_TRUNCATED 2 /* out of body: header or payload cut off, or the body's end (:400-403, :425-427) */
+#define AMBC_RANGE_COMPLETE 3  /* output complete (:444-445)                                            */
+#define AMBC_RANGE_MARKER 4    /* "Marker mismatch in chunk header." (:405-407)                          */
+#define AMBC_RANGE_INIT {0, 0, AMBC_RANGE_NO_PKG, 0, 0, 0, 0, AMBC_RANGE_RUNNING}
+
+/* what one rank holds; ambc_range_index fills it, the later calls read it */
+typedef struct {
+    uint64_t lo, hi;        /* body range of this rank                                                 */
+    uint64_t body_len;      /* length of the whole body                                                */
+    uint64_t orig_size;
+    uint64_t n_cand;        /* header candidates (marker occurrences) starting in [lo, hi)             */
+    uint64_t work_bytes;    /* workspace this range needs (also set when AMBC_E_CAPACITY is returned)  */
+    void *work_dev;
+    uint32_t marker_bytes, known_mask, levels, reserved;
+} ambc_range;
+
+/* device workspace for a range of range_len bytes with n_cand candidates */
+uint64_t ambc_range_workspace_bytes(uint64_t range_len, uint64_t n_cand);
+/*
+ * Phase 1.  buf_dev holds body[lo, lo + buf_len) with buf_len >= min(hi + marker_bytes + 13, body_len) - lo
+ * (the range plus the header halo behind hi).  Counts the candidates first; when work_bytes is too
+ * small returns AMBC_E_CAPACITY with r->n_cand and r->work_bytes set (allocate and call again).  The
+ * tables stay in work_dev for the other calls; the buffer is not read again.  Synchronises `stream`.
+ */
+int ambc_range_index(const void *buf_dev, uint64_t buf_len, uint64_t lo, uint64_t hi, uint64_t body_len,
+                     const uint8_t *marker, uint32_t marker_bytes, uint64_t orig_size, uint32_t known_mask,
+                     void *work_dev, uint64_t work_bytes, ambc_range *r, void *stream);
+/* Phase 2, one fold step: *out = the walk's state behind this range given *in (host structs).
+ * Synchronises `stream`. */
+int ambc_range_fold(const ambc_range *r, const ambc_range_state *in, ambc_range_state *out, void *stream);
+/*
+ * Phase 3: the rank's table from its entry state (table_dev NULL: count only).  *out_lo / *out_hi =
+ * output offsets of its first and behind its last entry (out_hi excludes the zero tail);
+ * *need = payload bytes a decoded package of this range needs beyond body position
+ * min(hi + marker_bytes + 13, body_len): the buffer must hold them before decoding.  Synchronises `stream`.
+ */
+int ambc_range_table(const ambc_range *r, const ambc_range_state *entry, ambc_pkg *table_dev, uint64_t table_cap,
+                     uint64_t *n_entries, uint64_t *out_lo, uint64_t *out_hi, uint64_t *need, void *stream);
+/* output offset of the first byte a range starting at body position `lo` owns, given the state the
+ * fold handed to it (pure host arithmetic) */
+uint64_t ambc_range_out_offset(const ambc_range_state *s, uint64_t lo, uint64_t orig_size, uint32_t marker_bytes,
+                               uint32_t known_mask);
+
+/*
  * Decode every table entry into out_dev (orig_size bytes; zero padded / truncated
  * as adaptive_compressor.py:447-452).  status_dev (optional, uint32[2]):
  * [0] = entries whose codec raised (output zero-filled, :440-442),

@@ -248,7 +248,8 @@ uint64_t ambc_range_out_offset(const ambc_range_state *s, uint64_t lo, uint64_t 
  * Decode every table entry into out_dev (orig_size bytes; zero padded / truncated
  * as adaptive_compressor.py:447-452).  status_dev (optional, uint32[2]):
  * [0] = entries whose codec raised (output zero-filled, :440-442),
- * [1] = entries whose decoded length differed from out_len (malformed stream).
+ * [1] = entries whose decoded length differed from the package's nominal length (malformed
+ *       stream; nominal: orig_len, min(comp_len, orig_len) for Delta, 0 for an empty payload).
  * Entries of types 6 (BZIP2) and 7 (LZMA) are left to ambc_decompress_dev_mask.
  */
 int ambc_decompress_dev(const void *body_dev, uint64_t body_len, const ambc_pkg *table_dev, uint64_t n_entries,

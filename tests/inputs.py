@@ -268,6 +268,21 @@ def malformed_payloads():
     return out
 
 
+def corrupt(payload, r):
+    """1 to 3 random edits of a payload drawn from RandomState r: a byte overwritten, the tail cut off, or a few
+    random bytes appended"""
+    a = bytearray(payload)
+    for _ in range(int(r.randint(1, 4))):
+        what = r.randint(3)
+        if what == 0 and len(a) > 2:
+            a[r.randint(len(a))] = r.randint(256)
+        elif what == 1 and len(a) > 4:
+            del a[r.randint(len(a)):]
+        else:
+            a += bytes(r.randint(0, 256, size=r.randint(1, 5)).astype(np.uint8))
+    return bytes(a)
+
+
 def gate_case(i):
     """i-th should_use probe: a seeded input blended with random bytes so that the
     sampled ratios / entropy land near the reference's thresholds."""

@@ -160,16 +160,7 @@ def test_decode_corrupted_fuzz(eng):
             p = O.compress(mid, d, lz_fast=True)
             if isinstance(p, int):
                 continue
-            a = bytearray(p)
-            for _ in range(int(r.randint(1, 4))):
-                what = r.randint(3)
-                if what == 0 and len(a) > 2:
-                    a[r.randint(len(a))] = r.randint(256)
-                elif what == 1 and len(a) > 4:
-                    del a[r.randint(len(a)):]
-                else:
-                    a += bytes(r.randint(0, 256, size=r.randint(1, 5)).astype(np.uint8))
-            payloads.append(bytes(a))
+            payloads.append(inputs.corrupt(p, r))
             origs.append(len(d))
         got = eng.codec_decode_batch(mid, payloads, origs)
         for i, (p, o, g) in enumerate(zip(payloads, origs, got)):

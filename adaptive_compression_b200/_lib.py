@@ -59,6 +59,22 @@ class Range(C.Structure):
                 ("marker_bytes", C.c_uint32), ("known_mask", C.c_uint32), ("levels", C.c_uint32), ("reserved", C.c_uint32)]
 
 
+class DynEntry(C.Structure):
+    """ambc_dyn_entry: where the multi-candidate chain goes from one possible entry of a rank's input range"""
+    _fields_ = [("entry", C.c_uint64), ("exit", C.c_uint64), ("stop", C.c_uint64), ("status", C.c_uint32),
+                ("reserved", C.c_uint32)]
+
+
+class DynRange(C.Structure):
+    """ambc_dyn_range: what one rank holds after ambc_dyn_range_walk"""
+    _fields_ = [("lo", C.c_uint64), ("hi", C.c_uint64), ("n", C.c_uint64), ("work_bytes", C.c_uint64),
+                ("work_dev", C.c_void_p), ("host", C.c_void_p), ("n_entries", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+DYN_JOIN, DYN_LEAVE, DYN_STOP, DYN_UNRESOLVED = 0, 1, 2, 3
+DYN_MAX_ENTRIES = 32
+DYN_NONE = (1 << 64) - 1
+
 RANGE_NO_PKG = (1 << 64) - 1
 RANGE_RUNNING, RANGE_END, RANGE_TRUNCATED, RANGE_COMPLETE, RANGE_MARKER = 0, 1, 2, 3, 4
 
@@ -81,6 +97,15 @@ _SIGS = {
     "ambc_compress_dynamic_dev": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32,
                                             C.c_char_p, C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64,
                                             C.POINTER(CompressResult), C.c_void_p, C.c_uint64, C.c_void_p]),
+    "ambc_dyn_range_workspace_bytes": (C.c_uint64, [C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_uint32]),
+    "ambc_dyn_range_walk": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_uint32,
+                                      C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_uint64, C.POINTER(DynRange),
+                                      C.POINTER(DynEntry), C.c_uint32, C.POINTER(C.c_uint32), C.c_void_p]),
+    "ambc_dyn_range_resolve": (C.c_int, [C.POINTER(DynRange), C.c_uint64, C.POINTER(DynEntry), C.c_void_p]),
+    "ambc_dyn_range_encode": (C.c_int, [C.POINTER(DynRange), C.c_void_p, C.c_uint64, C.c_char_p, C.c_uint32, C.c_void_p,
+                                        C.c_uint64, C.POINTER(CompressResult), C.c_void_p, C.c_uint64,
+                                        C.POINTER(C.c_uint64), C.c_void_p]),
+    "ambc_dyn_range_free": (None, [C.POINTER(DynRange)]),
     "ambc_index_host": (C.c_int, [C.c_void_p, C.c_uint64, C.c_char_p, C.c_uint32, C.c_uint64, C.c_uint32,
                                   C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "ambc_index_dev": (C.c_int, [C.c_void_p, C.c_uint64, C.c_char_p, C.c_uint32, C.c_uint64, C.c_uint32,

@@ -629,6 +629,9 @@ static uint64_t gcd64(uint64_t a, uint64_t b) { while (b) { uint64_t t = a % b; 
 struct WalkRec { unsigned long long pos; uint32_t size; uint32_t type_len; };   // type << 24 | payload length
 struct WalkSeg { unsigned long long exit; unsigned long long stop; uint32_t count; uint32_t merged; uint32_t pad[2]; };
 struct WalkCands { uint32_t n; uint32_t c[32]; };
+// PER_ITEM = false: ambc_compress_dynamic_dev; true: the list-mode walks of ambc_dyn_range_* (a range's candidate
+// entries all lie in its segment 0, so their records are stored per item)
+template <bool PER_ITEM>
 __global__ void __launch_bounds__(SF_T, 3)
 k_dynamic_walk(const uint8_t *__restrict__ in, uint64_t total, WalkCands cands, uint32_t mask, uint32_t ovh, uint32_t pcr,
                uint32_t g, const unsigned long long *__restrict__ list, uint64_t n_items,
@@ -636,7 +639,8 @@ k_dynamic_walk(const uint8_t *__restrict__ in, uint64_t total, WalkCands cands, 
                WalkRec *__restrict__ recs, WalkSeg *__restrict__ segs)
 {
     // list == nullptr: item i = segment i entered at its first byte; else item i = (segment, entry position) and the
-    // walk stops where it meets the segment's speculative chain (spec_recs / spec_segs)
+    // walk stops where it meets the segment's speculative chain (spec_recs / spec_segs).  Records go to
+    // recs[segment * DYN_SEGU], or with PER_ITEM to recs[item * DYN_SEGU] (several items may share a segment)
     extern __shared__ uint4 smem4[];
     SfCtx<8192> c;
     sf_carve<8192>(c, (uint8_t *)smem4);
@@ -692,7 +696,7 @@ k_dynamic_walk(const uint8_t *__restrict__ in, uint64_t total, WalkCands cands, 
             if (threadIdx.x == 0) {
                 WalkRec r;
                 r.pos = pos; r.size = best_c; r.type_len = (best_t << 24) | best_len;
-                recs[sg * DYN_SEGU + count] = r;
+                recs[(PER_ITEM ? it : sg) * DYN_SEGU + count] = r;
             }
             count++;
             pos += best_c;
@@ -710,7 +714,9 @@ struct DynLayout {
     uint64_t slots, spans, type, comp, offs, tiles, state, walk_recs, walk_segs, walk_list, total;
     uint64_t n_pos, n_tiles, g, n_seg;
 };
-static int dyn_layout(uint64_t n, const uint32_t *cands, uint32_t n_cands, DynLayout &L)
+// n: the bytes whose chain is walked (the file, or a range [lo, hi)); items > 0: a range, whose list-mode walks store
+// their records per item (up to `items` of them) and whose last packages may run up to 8192 bytes past its end
+static int dyn_layout(uint64_t n, const uint32_t *cands, uint32_t n_cands, DynLayout &L, uint64_t items = 0)
 {
     if (!cands || n_cands < 1 || n_cands > 32) return ambc_fail(AMBC_E_ARG, "need 1..32 candidate sizes");
     uint64_t g = 0;
@@ -730,7 +736,7 @@ static int dyn_layout(uint64_t n, const uint32_t *cands, uint32_t n_cands, DynLa
     L.n_tiles = (L.n_pos + SCAN_TILE - 1) / SCAN_TILE;
     uint64_t o = 0;
     auto take = [&](uint64_t bytes) { uint64_t r = o; o += (bytes + 255) & ~255ull; return r; };
-    L.slots = take(n + 64);
+    L.slots = take(n + (items ? AMBC_NMAX : 0) + 64);
     L.spans = take(L.n_pos * sizeof(ChunkSpan) + 16);
     L.type = take(L.n_pos + 16);
     L.comp = take(L.n_pos * 4 + 16);
@@ -738,9 +744,9 @@ static int dyn_layout(uint64_t n, const uint32_t *cands, uint32_t n_cands, DynLa
     L.tiles = take(L.n_tiles * 8 + 16);
     L.state = take(sizeof(ScanState));
     L.n_seg = (L.n_pos + DYN_SEGU - 1) / DYN_SEGU;
-    L.walk_recs = take(2 * L.n_pos * sizeof(WalkRec) + 64);   // speculative chains | re-entered chains
-    L.walk_segs = take(2 * L.n_seg * sizeof(WalkSeg) + 64);
-    L.walk_list = take(L.n_seg * 16 + 64);
+    L.walk_recs = take((L.n_pos + (items ? items * DYN_SEGU : L.n_pos)) * sizeof(WalkRec) + 64); // speculative | re-entered
+    L.walk_segs = take((L.n_seg + (items ? items : L.n_seg)) * sizeof(WalkSeg) + 64);
+    L.walk_list = take((items ? items : L.n_seg) * 16 + 64);
     L.total = o;
     return AMBC_OK;
 }
@@ -750,6 +756,282 @@ extern "C" uint64_t ambc_compress_dynamic_workspace_bytes(uint64_t n, const uint
     DynLayout L;
     if (dyn_layout(n, cands, n_cands, L)) return 0;
     return L.total;
+}
+
+// ---- the chain stitch of one walked span: the whole file, or a range [lo, hi) with positions relative to lo --------
+struct DynStitch {
+    const uint8_t *in;
+    uint64_t total, len;  // bytes from position 0 to the end of the file; bytes whose chain is walked
+    WalkCands wc;
+    uint32_t mask, ovh, pcr;
+    bool per_item;        // list-mode walks store their records per item (k_dynamic_walk<true>)
+    uint64_t g, seglen, n_seg, n_pos;
+    WalkRec *d_spec, *d_fix;
+    WalkSeg *d_sseg, *d_fseg;
+    unsigned long long *d_list;
+    std::vector<WalkRec> h_spec, h_fix;
+    std::vector<WalkSeg> h_sseg, fixseg;
+    std::vector<uint64_t> fix_entry; // entry position the stored re-entered chain of a segment belongs to
+    std::vector<WalkRec> extra_recs; // the walks of the extra items of the first round (a range's candidate entries)
+    std::vector<WalkSeg> extra_segs;
+};
+
+static void dyn_stitch_init(DynStitch &S, const void *in, uint64_t total, uint64_t len, const uint32_t *cands,
+                            uint32_t n_cands, uint32_t mask, uint32_t ovh, bool pcr, bool per_item, const DynLayout &L,
+                            uint8_t *W)
+{
+    S.in = (const uint8_t *)in;
+    S.total = total; S.len = len;
+    S.wc.n = n_cands;
+    for (uint32_t i = 0; i < n_cands; i++) S.wc.c[i] = cands[i];
+    S.mask = mask; S.ovh = ovh; S.pcr = pcr ? 1u : 0u; S.per_item = per_item;
+    S.g = L.g; S.seglen = (uint64_t)DYN_SEGU * L.g; S.n_seg = L.n_seg; S.n_pos = L.n_pos;
+    S.d_spec = (WalkRec *)(W + L.walk_recs); S.d_fix = S.d_spec + L.n_pos;
+    S.d_sseg = (WalkSeg *)(W + L.walk_segs); S.d_fseg = S.d_sseg + L.n_seg;
+    S.d_list = (unsigned long long *)(W + L.walk_list);
+    S.h_spec.assign(L.n_pos, WalkRec());
+    S.h_fix.assign(L.n_pos, WalkRec());
+    S.h_sseg.assign(L.n_seg, WalkSeg());
+    S.fixseg.assign(L.n_seg, WalkSeg());
+    S.fix_entry.assign(L.n_seg, ~0ull);
+}
+
+static int dyn_launch(const DynStitch &S, const unsigned long long *list, uint64_t n_items, WalkRec *recs, WalkSeg *segs,
+                      cudaStream_t stream)
+{
+    const size_t wsmem = SfCfg<8192>::SMEM;
+    const unsigned grid = (unsigned)min<uint64_t>(n_items, 0x7fffffffull);
+    const WalkRec *sr = list ? S.d_spec : nullptr;
+    const WalkSeg *ss = list ? S.d_sseg : nullptr;
+    if (list && S.per_item) {
+        CUDA_TRY(cudaFuncSetAttribute(k_dynamic_walk<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
+        k_dynamic_walk<true><<<grid, SF_T, wsmem, stream>>>(S.in, S.total, S.wc, S.mask, S.ovh, S.pcr, (uint32_t)S.g, list,
+                                                            n_items, sr, ss, recs, segs);
+    } else {
+        CUDA_TRY(cudaFuncSetAttribute(k_dynamic_walk<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
+        k_dynamic_walk<false><<<grid, SF_T, wsmem, stream>>>(S.in, S.total, S.wc, S.mask, S.ovh, S.pcr, (uint32_t)S.g, list,
+                                                             n_items, sr, ss, recs, segs);
+    }
+    ambc_count_launch();
+    CUDA_TRY(cudaGetLastError());
+    return AMBC_OK;
+}
+
+// the speculative chain of every segment, entered at its first byte
+static int dyn_spec_walk(DynStitch &S, cudaStream_t stream)
+{
+    int rc = dyn_launch(S, nullptr, S.n_seg, S.d_spec, S.d_sseg, stream);
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(S.h_spec.data(), S.d_spec, S.n_pos * sizeof(WalkRec), cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaMemcpyAsync(S.h_sseg.data(), S.d_sseg, S.n_seg * sizeof(WalkSeg), cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    return AMBC_OK;
+}
+
+// follows the chain from e through the segments with what is known and appends the (segment, entry) pairs that still
+// have to be walked (unknown ones are assumed to meet their speculative chain).  With none appended, *exit (the first
+// position at or past len) or *stop (no winner there, strict mode) is where the chain leaves the span.
+static void dyn_follow(const DynStitch &S, uint64_t e, std::vector<unsigned long long> &list, uint64_t *exit, uint64_t *stop)
+{
+    *stop = ~0ull;
+    for (uint64_t sg = e / S.seglen; sg < S.n_seg && e < S.len; sg++) {
+        const uint64_t s0 = sg * S.seglen, s1 = min<uint64_t>(S.len, s0 + S.seglen);
+        if (e >= s1) continue;
+        const WalkSeg &sp = S.h_sseg[sg];
+        if (e == s0) { if (sp.stop != ~0ull) { *stop = sp.stop; break; } e = sp.exit; continue; }
+        if (S.fix_entry[sg] == e) {
+            const WalkSeg &last = S.fixseg[sg].merged ? sp : S.fixseg[sg];
+            if (last.stop != ~0ull) { *stop = last.stop; break; }
+            e = last.exit;
+            continue;
+        }
+        list.push_back(sg); list.push_back(e);
+        if (sp.stop != ~0ull) { *stop = sp.stop; break; }
+        e = sp.exit;
+    }
+    *exit = e;
+}
+
+// re-enters segments (one launch per round) until the chain from e0 is known to where it leaves the span; the first
+// round also walks `extra` (segment, entry) items, whose records land in S.extra_recs / S.extra_segs
+static int dyn_stitch(DynStitch &S, uint64_t e0, const std::vector<unsigned long long> &extra, uint64_t *exit,
+                      uint64_t *stop, cudaStream_t stream)
+{
+    std::vector<unsigned long long> list;
+    std::vector<WalkSeg> h_fseg;
+    std::vector<WalkRec> h_items;
+    for (int round = 0;; round++) {
+        list.clear();
+        dyn_follow(S, e0, list, exit, stop);
+        const uint64_t n_local = list.size() / 2;
+        if (round == 0) list.insert(list.end(), extra.begin(), extra.end());
+        if (list.empty()) break;
+        if (round > (int)S.n_seg + 2) return ambc_fail(AMBC_E_CUDA, "internal: the chain stitch does not settle");
+        const uint64_t ni = list.size() / 2;
+        CUDA_TRY(cudaMemcpyAsync(S.d_list, list.data(), list.size() * 8, cudaMemcpyHostToDevice, stream));
+        int rc = dyn_launch(S, S.d_list, ni, S.d_fix, S.d_fseg, stream);
+        if (rc) return rc;
+        h_fseg.resize(ni);
+        CUDA_TRY(cudaMemcpyAsync(h_fseg.data(), S.d_fseg, ni * sizeof(WalkSeg), cudaMemcpyDeviceToHost, stream));
+        CUDA_TRY(cudaStreamSynchronize(stream));
+        if (S.per_item) {
+            h_items.resize(ni * DYN_SEGU);
+            CUDA_TRY(cudaMemcpyAsync(h_items.data(), S.d_fix, ni * DYN_SEGU * sizeof(WalkRec), cudaMemcpyDeviceToHost, stream));
+            CUDA_TRY(cudaStreamSynchronize(stream));
+            for (uint64_t k = 0; k < n_local; k++)
+                std::copy(h_items.begin() + k * DYN_SEGU, h_items.begin() + k * DYN_SEGU + h_fseg[k].count,
+                          S.h_fix.begin() + list[2 * k] * DYN_SEGU);
+            if (round == 0 && ni > n_local) {
+                S.extra_recs.assign(h_items.begin() + n_local * DYN_SEGU, h_items.end());
+                S.extra_segs.assign(h_fseg.begin() + n_local, h_fseg.end());
+            }
+        } else {
+            // (one copy of the whole record buffer: thousands of short copies cost more than the 16 bytes per g bytes)
+            const uint64_t lo = list[0] * DYN_SEGU, hi = min<uint64_t>(S.n_pos, (list[2 * (ni - 1)] + 1) * DYN_SEGU);
+            CUDA_TRY(cudaMemcpyAsync(S.h_fix.data() + lo, S.d_fix + lo, (hi - lo) * sizeof(WalkRec), cudaMemcpyDeviceToHost, stream));
+            CUDA_TRY(cudaStreamSynchronize(stream));
+        }
+        for (uint64_t k = 0; k < n_local; k++) {
+            const uint64_t sg = list[2 * k];
+            S.fixseg[sg] = h_fseg[k];
+            S.fix_entry[sg] = list[2 * k + 1];
+        }
+    }
+    return AMBC_OK;
+}
+
+// the chain from e, once dyn_stitch has run from it, as spans (positions relative to the span's start).  on_spec: e
+// lies on the speculative chain of its segment (a walk met it there).  *raw_from = the strict stop, or untouched.
+struct DynChain {
+    std::vector<ChunkSpan> spans;
+    std::vector<uint8_t> type;
+    std::vector<uint32_t> len;
+    void push(const WalkRec &r)
+    {
+        ChunkSpan sp; sp.pos = r.pos; sp.size = r.size; sp.pad = 0;
+        spans.push_back(sp); type.push_back((uint8_t)(r.type_len >> 24)); len.push_back(r.type_len & 0xFFFFFFu);
+    }
+};
+static int dyn_chain(const DynStitch &S, uint64_t e, bool on_spec, DynChain &C, uint64_t *raw_from)
+{
+    for (uint64_t sg = e / S.seglen; sg < S.n_seg && e < S.len; sg++) {
+        const uint64_t s0 = sg * S.seglen, s1 = min<uint64_t>(S.len, s0 + S.seglen);
+        if (e >= s1) continue;
+        const WalkSeg &sp = S.h_sseg[sg];
+        const WalkRec *spec = S.h_spec.data() + sg * DYN_SEGU;
+        uint32_t from = 0; // first speculative record that belongs to the true chain
+        bool use_spec = true;
+        if (e != s0 && on_spec) {
+            while (from < sp.count && spec[from].pos != e) from++;
+            if (from == sp.count) return ambc_fail(AMBC_E_CUDA, "internal: meeting point not on the speculative chain");
+        } else if (e != s0) {
+            const WalkSeg &f = S.fixseg[sg];
+            if (S.fix_entry[sg] != e) return ambc_fail(AMBC_E_CUDA, "internal: segment %llu not walked from its entry", (unsigned long long)sg);
+            for (uint32_t k = 0; k < f.count; k++) C.push(S.h_fix[sg * DYN_SEGU + k]);
+            if (f.merged) {
+                while (from < sp.count && spec[from].pos != f.exit) from++;
+                if (from == sp.count) return ambc_fail(AMBC_E_CUDA, "internal: meeting point not on the speculative chain");
+            } else {
+                use_spec = false;
+                if (f.stop != ~0ull) { *raw_from = f.stop; break; }
+                e = f.exit;
+            }
+        }
+        on_spec = false;
+        if (use_spec) {
+            for (uint32_t k = from; k < sp.count; k++) C.push(spec[k]);
+            if (sp.stop != ~0ull) { *raw_from = sp.stop; break; }
+            e = sp.exit;
+        }
+    }
+    return AMBC_OK;
+}
+
+// per-chunk-raw extension without a native method: raw pieces of the smallest candidate size from `from` (a multiple of
+// it) up to the first piece that starts at or past `to`; `base` is subtracted from the positions
+static void dyn_raw_pieces(uint64_t from, uint64_t to, uint64_t n, uint32_t cmin, uint64_t base, DynChain &C)
+{
+    for (uint64_t pos = from; pos < to;) {
+        WalkRec r;
+        r.pos = pos - base; r.size = (uint32_t)min<uint64_t>(cmin, n - pos); r.type_len = (255u << 24) | r.size;
+        C.push(r);
+        pos += r.size;
+    }
+}
+
+// encode + frame the chosen chunks (span mode): packages only, body bytes [0, *body) of out_dev
+static int dyn_encode(const uint8_t *in, uint64_t total, const DynLayout &L, uint8_t *W, const DynChain &C,
+                      uint32_t method_mask, uint32_t ovh, uint32_t marker_word, uint32_t marker_bytes, void *out_dev,
+                      uint64_t out_cap, uint64_t body, cudaStream_t stream)
+{
+    const uint64_t n_list = C.spans.size();
+    if (!n_list) return AMBC_OK;
+    ChunkSpan *d_spans = (ChunkSpan *)(W + L.spans);
+    uint8_t *type = W + L.type;
+    uint32_t *comp = (uint32_t *)(W + L.comp);
+    unsigned long long *offs = (unsigned long long *)(W + L.offs);
+    unsigned long long *tiles = (unsigned long long *)(W + L.tiles);
+    ScanState *st = (ScanState *)(W + L.state);
+    ScanState h_st;
+    memset(&h_st, 0, sizeof h_st);
+    h_st.first_raw = ~0ull;
+    CUDA_TRY(cudaMemcpyAsync(st, &h_st, sizeof h_st, cudaMemcpyHostToDevice, stream));
+    CUDA_TRY(cudaMemcpyAsync(d_spans, C.spans.data(), n_list * sizeof(ChunkSpan), cudaMemcpyHostToDevice, stream));
+    uint32_t maxsz = 0;
+    for (uint64_t k = 0; k < n_list; k++) maxsz = max(maxsz, C.spans[k].size);
+    if (maxsz > AMBC_NMAX) { // only per-chunk-raw pieces can be this large
+        return ambc_fail(AMBC_E_ARG, "per-chunk-raw pieces larger than 8192 bytes are not supported");
+    }
+    unsigned grid = (unsigned)min<uint64_t>(n_list, 0x7fffffffull);
+    int rc;
+    if ((rc = launch_select_span(grid, stream, in, total, maxsz, method_mask, ovh, 0, d_spans, W + L.slots, type, comp,
+                                 n_list))) return rc;
+    const unsigned gt = (unsigned)((n_list + SCAN_TILE - 1) / SCAN_TILE);
+    const uint32_t sflags = 1u | 2u; // every entry is a package; no END (appended by the caller)
+    k_sizes<<<gt, 256, 0, stream>>>(type, comp, 0, n_list, maxsz, total, ovh, sflags, st, tiles);
+    ambc_count_launch();
+    k_scan_tiles<<<1, 1024, 0, stream>>>(tiles, 0, gt, 1, type, comp, n_list, maxsz, total, ovh, sflags, st, (uint8_t *)out_dev,
+                                         out_cap, marker_word, marker_bytes);
+    ambc_count_launch();
+    k_offsets<<<gt, 256, 0, stream>>>(type, comp, 0, n_list, maxsz, total, ovh, sflags, st, tiles, offs);
+    ambc_count_launch();
+    size_t psmem = 32 + (((size_t)maxsz + 15) & ~(size_t)15) + 32;
+    CUDA_TRY(cudaFuncSetAttribute(k_pack_span, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem));
+    k_pack_span<<<grid, PACK_BLOCK, psmem, stream>>>(in, d_spans, W + L.slots, type, comp, offs, marker_word, marker_bytes,
+                                                    (uint8_t *)out_dev, n_list);
+    ambc_count_launch();
+    CUDA_TRY(cudaGetLastError());
+    // the second evaluation must agree with the trial the chain was built from
+    std::vector<uint8_t> chk_t(n_list);
+    std::vector<uint32_t> chk_l(n_list);
+    CUDA_TRY(cudaMemcpyAsync(chk_t.data(), type, n_list, cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaMemcpyAsync(chk_l.data(), comp, n_list * 4, cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaMemcpyAsync(&h_st, st, sizeof h_st, cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    for (uint64_t k = 0; k < n_list; k++)
+        if (chk_t[k] != C.type[k] || chk_l[k] != C.len[k])
+            return ambc_fail(AMBC_E_CUDA, "internal: span encode disagrees with its trial at chunk %llu", (unsigned long long)k);
+    if (h_st.body_len != body) return ambc_fail(AMBC_E_CUDA, "internal: span body length mismatch");
+    return AMBC_OK;
+}
+
+// usage, payload bytes and the package map of a chain (map positions shifted by `base`)
+static void dyn_result(const DynChain &C, uint64_t base, ambc_compress_result *res, ambc_chunk_info *map_out, uint64_t map_cap)
+{
+    const uint64_t n_list = C.spans.size();
+    for (uint64_t k = 0; k < n_list; k++) {
+        const int t = C.type[k];
+        if (t >= 1 && t <= 4) { res->usage[t]++; res->payload_bytes += C.len[k]; }
+        else res->usage[0]++;
+        if (map_out && k < map_cap) { map_out[k].pos = base + C.spans[k].pos; map_out[k].orig_len = C.spans[k].size; map_out[k].comp_len = C.len[k]; map_out[k].type = (uint32_t)t; }
+    }
+}
+
+static uint32_t marker_word_of(const uint8_t *marker, uint32_t marker_bytes)
+{
+    uint32_t w = 0;
+    for (uint32_t k = 0; k < marker_bytes; k++) w |= (uint32_t)marker[k] << (8 * k);
+    return w;
 }
 
 extern "C" int ambc_compress_dynamic_dev(const void *in_dev, uint64_t n, const uint32_t *cands, uint32_t n_cands,
@@ -766,8 +1048,7 @@ extern "C" int ambc_compress_dynamic_dev(const void *in_dev, uint64_t n, const u
     if (rc) return rc;
     if (work_bytes < L.total) return ambc_fail(AMBC_E_CAPACITY, "ambc_compress_dynamic_dev: workspace too small");
     const uint32_t ovh = marker_bytes + 14;
-    uint32_t marker_word = 0;
-    for (uint32_t k = 0; k < marker_bytes; k++) marker_word |= (uint32_t)marker[k] << (8 * k);
+    const uint32_t marker_word = marker_word_of(marker, marker_bytes);
     memset(res, 0, sizeof(*res));
     res->first_raw = -1;
     uint8_t endp[16], hdr[18];
@@ -777,167 +1058,32 @@ extern "C" int ambc_compress_dynamic_dev(const void *in_dev, uint64_t n, const u
     const bool pcr = flags & AMBC_F_PER_CHUNK_RAW;
 
     const bool native = (method_mask & AMBC_NATIVE_MASK) != 0;
-    std::vector<ChunkSpan> spans;
-    std::vector<uint8_t> s_type;
-    std::vector<uint32_t> s_len;
+    DynChain C;
     uint64_t raw_from = n; // raw_from < n: one raw package [raw_from, n)
     if (n && native) {
-        // ---- the chain, walked on the GPU segment by segment (k_dynamic_walk) ------------------------------------
-        WalkCands wc;
-        wc.n = n_cands;
-        for (uint32_t i = 0; i < n_cands; i++) wc.c[i] = cands[i];
-        const uint64_t seglen = (uint64_t)DYN_SEGU * L.g, n_seg = L.n_seg;
-        WalkRec *d_spec = (WalkRec *)(W + L.walk_recs), *d_fix = d_spec + L.n_pos;
-        WalkSeg *d_sseg = (WalkSeg *)(W + L.walk_segs), *d_fseg = d_sseg + n_seg;
-        unsigned long long *d_list = (unsigned long long *)(W + L.walk_list);
-        const size_t wsmem = SfCfg<8192>::SMEM;
-        CUDA_TRY(cudaFuncSetAttribute(k_dynamic_walk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
-        k_dynamic_walk<<<(unsigned)min<uint64_t>(n_seg, 0x7fffffffull), SF_T, wsmem, stream>>>(
-            (const uint8_t *)in_dev, n, wc, method_mask, ovh, pcr ? 1u : 0u, (uint32_t)L.g, nullptr, n_seg, nullptr, nullptr, d_spec, d_sseg);
-        ambc_count_launch();
-        CUDA_TRY(cudaGetLastError());
-        std::vector<WalkRec> h_spec(L.n_pos), h_fix(L.n_pos);
-        std::vector<WalkSeg> h_sseg(n_seg), h_fseg(n_seg), fixseg(n_seg);
-        std::vector<uint64_t> fix_entry(n_seg, ~0ull); // entry position the stored re-entered chain of a segment belongs to
-        CUDA_TRY(cudaMemcpyAsync(h_spec.data(), d_spec, L.n_pos * sizeof(WalkRec), cudaMemcpyDeviceToHost, stream));
-        CUDA_TRY(cudaMemcpyAsync(h_sseg.data(), d_sseg, n_seg * sizeof(WalkSeg), cudaMemcpyDeviceToHost, stream));
-        CUDA_TRY(cudaStreamSynchronize(stream));
-        std::vector<unsigned long long> list;
-        for (int round = 0;; round++) {
-            // follow the true chain through the segments with what is known; collect the (segment, entry) pairs that
-            // still have to be walked (unknown ones are assumed to meet their speculative chain)
-            list.clear();
-            uint64_t e = 0;
-            for (uint64_t sg = 0; sg < n_seg && e < n; sg++) {
-                const uint64_t s0 = sg * seglen, s1 = min<uint64_t>(n, s0 + seglen);
-                if (e >= s1) continue;
-                if (e == s0) { if (h_sseg[sg].stop != ~0ull) break; e = h_sseg[sg].exit; continue; }
-                if (fix_entry[sg] == e) {
-                    const WalkSeg &f = fixseg[sg];
-                    if (f.merged) { if (h_sseg[sg].stop != ~0ull) break; e = h_sseg[sg].exit; }
-                    else { if (f.stop != ~0ull) break; e = f.exit; }
-                    continue;
-                }
-                list.push_back(sg); list.push_back(e);
-                if (h_sseg[sg].stop != ~0ull) break;
-                e = h_sseg[sg].exit;
-            }
-            if (list.empty()) break;
-            if (round > (int)n_seg + 2) return ambc_fail(AMBC_E_CUDA, "internal: the chain stitch does not settle");
-            const uint64_t ni = list.size() / 2;
-            CUDA_TRY(cudaMemcpyAsync(d_list, list.data(), list.size() * 8, cudaMemcpyHostToDevice, stream));
-            k_dynamic_walk<<<(unsigned)min<uint64_t>(ni, 0x7fffffffull), SF_T, wsmem, stream>>>(
-                (const uint8_t *)in_dev, n, wc, method_mask, ovh, pcr ? 1u : 0u, (uint32_t)L.g, d_list, ni, d_spec, d_sseg, d_fix, d_fseg);
-            ambc_count_launch();
-            CUDA_TRY(cudaGetLastError());
-            CUDA_TRY(cudaMemcpyAsync(h_fseg.data(), d_fseg, ni * sizeof(WalkSeg), cudaMemcpyDeviceToHost, stream));
-            CUDA_TRY(cudaStreamSynchronize(stream));
-            // (one copy of the whole record buffer: thousands of short copies cost more than the 16 bytes per g bytes)
-            const uint64_t lo = list[0] * DYN_SEGU, hi = min<uint64_t>(L.n_pos, (list[2 * (ni - 1)] + 1) * DYN_SEGU);
-            CUDA_TRY(cudaMemcpyAsync(h_fix.data() + lo, d_fix + lo, (hi - lo) * sizeof(WalkRec), cudaMemcpyDeviceToHost, stream));
-            CUDA_TRY(cudaStreamSynchronize(stream));
-            for (uint64_t k = 0; k < ni; k++) {
-                const uint64_t sg = list[2 * k];
-                fixseg[sg] = h_fseg[k];
-                fix_entry[sg] = list[2 * k + 1];
-            }
-        }
-        // the chain itself
-        auto push = [&](const WalkRec &r) {
-            ChunkSpan sp; sp.pos = r.pos; sp.size = r.size; sp.pad = 0;
-            spans.push_back(sp); s_type.push_back((uint8_t)(r.type_len >> 24)); s_len.push_back(r.type_len & 0xFFFFFFu);
-        };
-        uint64_t e = 0;
-        for (uint64_t sg = 0; sg < n_seg && e < n; sg++) {
-            const uint64_t s0 = sg * seglen, s1 = min<uint64_t>(n, s0 + seglen);
-            if (e >= s1) continue;
-            uint32_t from = 0; // first speculative record that belongs to the true chain
-            bool use_spec = true;
-            if (e != s0) {
-                const WalkSeg &f = fixseg[sg];
-                for (uint32_t k = 0; k < f.count; k++) push(h_fix[sg * DYN_SEGU + k]);
-                if (f.merged) {
-                    while (from < h_sseg[sg].count && h_spec[sg * DYN_SEGU + from].pos != f.exit) from++;
-                    if (from == h_sseg[sg].count) return ambc_fail(AMBC_E_CUDA, "internal: meeting point not on the speculative chain");
-                } else {
-                    use_spec = false;
-                    if (f.stop != ~0ull) { raw_from = f.stop; break; }
-                    e = f.exit;
-                }
-            }
-            if (use_spec) {
-                for (uint32_t k = from; k < h_sseg[sg].count; k++) push(h_spec[sg * DYN_SEGU + k]);
-                if (h_sseg[sg].stop != ~0ull) { raw_from = h_sseg[sg].stop; break; }
-                e = h_sseg[sg].exit;
-            }
-        }
+        // ---- the chain, walked on the GPU segment by segment (k_dynamic_walk), stitched from position 0 ----------
+        DynStitch S;
+        dyn_stitch_init(S, in_dev, n, n, cands, n_cands, method_mask, ovh, pcr, false, L, W);
+        uint64_t exit, stop;
+        if ((rc = dyn_spec_walk(S, stream))) return rc;
+        if ((rc = dyn_stitch(S, 0, {}, &exit, &stop, stream))) return rc;
+        if ((rc = dyn_chain(S, 0, false, C, &raw_from))) return rc;
     } else if (!pcr) {
         raw_from = 0; // no native method: the whole file is one raw package (:586-590)
     } else {
-        // per-chunk-raw extension without a native method: raw pieces of the smallest candidate size
-        for (uint64_t pos = 0; pos < n;) {
-            ChunkSpan sp; sp.pos = pos; sp.size = (uint32_t)min<uint64_t>(cands[n_cands - 1], n - pos); sp.pad = 0;
-            spans.push_back(sp); s_type.push_back(255); s_len.push_back(sp.size);
-            pos += sp.size;
-        }
+        dyn_raw_pieces(0, n, n, cands[n_cands - 1], 0, C);
     }
-    const uint64_t n_list = spans.size();
+    const uint64_t n_list = C.spans.size();
     if (n_list > L.n_pos) return ambc_fail(AMBC_E_ARG, "internal: chain longer than the position table");
     uint64_t body = 0;
-    for (uint64_t k = 0; k < n_list; k++) body += ovh + s_len[k];
+    for (uint64_t k = 0; k < n_list; k++) body += ovh + C.len[k];
     const uint64_t raw_len = raw_from < n ? n - raw_from : 0;
     if (raw_len > 0xFFFFFFFFull) return ambc_fail(AMBC_E_ARG, "raw package over 4 GiB cannot be framed (u32 fields)");
     const uint64_t total_body = body + (raw_len ? ovh + raw_len : 0) + marker_bytes + 12;
     if (total_body > out_cap) return ambc_fail(AMBC_E_CAPACITY, "ambc_compress_dynamic_dev: out_cap too small");
 
-    // ---- encode + frame the chosen chunks ---------------------------------------------------------
-    if (n_list) {
-        ChunkSpan *d_spans = (ChunkSpan *)(W + L.spans);
-        uint8_t *type = W + L.type;
-        uint32_t *comp = (uint32_t *)(W + L.comp);
-        unsigned long long *offs = (unsigned long long *)(W + L.offs);
-        unsigned long long *tiles = (unsigned long long *)(W + L.tiles);
-        ScanState *st = (ScanState *)(W + L.state);
-        ScanState h_st;
-        memset(&h_st, 0, sizeof h_st);
-        h_st.first_raw = ~0ull;
-        CUDA_TRY(cudaMemcpyAsync(st, &h_st, sizeof h_st, cudaMemcpyHostToDevice, stream));
-        CUDA_TRY(cudaMemcpyAsync(d_spans, spans.data(), n_list * sizeof(ChunkSpan), cudaMemcpyHostToDevice, stream));
-        uint32_t maxsz = 0;
-        for (uint64_t k = 0; k < n_list; k++) maxsz = max(maxsz, spans[k].size);
-        if (maxsz > AMBC_NMAX) { // only per-chunk-raw pieces can be this large
-            return ambc_fail(AMBC_E_ARG, "per-chunk-raw pieces larger than 8192 bytes are not supported");
-        }
-        unsigned grid = (unsigned)min<uint64_t>(n_list, 0x7fffffffull);
-        if ((rc = launch_select_span(grid, stream, (const uint8_t *)in_dev, n, maxsz, method_mask, ovh, 0, d_spans,
-                                     W + L.slots, type, comp, n_list))) return rc;
-        const unsigned gt = (unsigned)((n_list + SCAN_TILE - 1) / SCAN_TILE);
-        const uint32_t sflags = 1u | 2u; // every entry is a package; no END (appended below)
-        k_sizes<<<gt, 256, 0, stream>>>(type, comp, 0, n_list, maxsz, n, ovh, sflags, st, tiles);
-        ambc_count_launch();
-        k_scan_tiles<<<1, 1024, 0, stream>>>(tiles, 0, gt, 1, type, comp, n_list, maxsz, n, ovh, sflags, st, (uint8_t *)out_dev,
-                                             out_cap, marker_word, marker_bytes);
-        ambc_count_launch();
-        k_offsets<<<gt, 256, 0, stream>>>(type, comp, 0, n_list, maxsz, n, ovh, sflags, st, tiles, offs);
-        ambc_count_launch();
-        size_t psmem = 32 + (((size_t)maxsz + 15) & ~(size_t)15) + 32;
-        CUDA_TRY(cudaFuncSetAttribute(k_pack_span, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem));
-        k_pack_span<<<grid, PACK_BLOCK, psmem, stream>>>((const uint8_t *)in_dev, d_spans, W + L.slots, type, comp, offs,
-                                                        marker_word, marker_bytes, (uint8_t *)out_dev, n_list);
-        ambc_count_launch();
-        CUDA_TRY(cudaGetLastError());
-        // the second evaluation must agree with the trial the chain was built from
-        std::vector<uint8_t> chk_t(n_list);
-        std::vector<uint32_t> chk_l(n_list);
-        CUDA_TRY(cudaMemcpyAsync(chk_t.data(), type, n_list, cudaMemcpyDeviceToHost, stream));
-        CUDA_TRY(cudaMemcpyAsync(chk_l.data(), comp, n_list * 4, cudaMemcpyDeviceToHost, stream));
-        CUDA_TRY(cudaMemcpyAsync(&h_st, st, sizeof h_st, cudaMemcpyDeviceToHost, stream));
-        CUDA_TRY(cudaStreamSynchronize(stream));
-        for (uint64_t k = 0; k < n_list; k++)
-            if (chk_t[k] != s_type[k] || chk_l[k] != s_len[k])
-                return ambc_fail(AMBC_E_CUDA, "internal: span encode disagrees with its trial at chunk %llu", (unsigned long long)k);
-        if (h_st.body_len != body) return ambc_fail(AMBC_E_CUDA, "internal: span body length mismatch");
-    }
+    if ((rc = dyn_encode((const uint8_t *)in_dev, n, L, W, C, method_mask, ovh, marker_word, marker_bytes, out_dev, out_cap,
+                         body, stream))) return rc;
     // ---- raw tail package (if any) and END ---------------------------------------------------------
     uint8_t *o = (uint8_t *)out_dev + body;
     if (raw_len) {
@@ -956,15 +1102,208 @@ extern "C" int ambc_compress_dynamic_dev(const void *in_dev, uint64_t n, const u
     res->n_chunks = n_list + (raw_len ? 1 : 0);
     res->n_packages = res->n_chunks;
     res->first_raw = raw_len ? (int64_t)n_list : -1;
-    for (uint64_t k = 0; k < n_list; k++) {
-        const int t = s_type[k];
-        if (t >= 1 && t <= 4) { res->usage[t]++; res->payload_bytes += s_len[k]; }
-        else res->usage[0]++;
-        if (map_out && k < map_cap) { map_out[k].pos = spans[k].pos; map_out[k].orig_len = spans[k].size; map_out[k].comp_len = s_len[k]; map_out[k].type = (uint32_t)t; }
-    }
+    dyn_result(C, 0, res, map_out, map_cap);
     if (raw_len) {
         res->usage[0]++;
         if (map_out && n_list < map_cap) { map_out[n_list].pos = raw_from; map_out[n_list].orig_len = (uint32_t)raw_len; map_out[n_list].comp_len = (uint32_t)raw_len; map_out[n_list].type = 255; }
     }
     return AMBC_OK;
+}
+
+// ---- one rank's input range of the multi-candidate mode (ambc_dyn_range_*) ------------------------------------------
+// The rank walks [lo, hi) with positions relative to lo on a buffer holding [lo, min(n, hi + 8192)): the winner at p
+// depends on data[p, p + 8192) and on n - p only.  lo and hi are whole segments, so the range's segments are the
+// file's.  The chain enters the range at a multiple of g in [lo, lo + S), S = min(8192, cands[0]) (a non-raw package
+// is at most S bytes, a per-chunk-raw piece cands[-1]): those entries are walked in segment 0 with the first round.
+struct DynRangeHost {
+    DynLayout L;
+    DynStitch S;
+    uint64_t lo, hi, n;
+    uint32_t cands[32], n_cands, mask, flags, ovh;
+    bool native, pcr;
+    const uint8_t *buf;
+    std::vector<ambc_dyn_entry> tab;
+    uint64_t lo_exit, lo_stop; // the chain from lo (relative positions)
+    std::vector<uint8_t> resolved; // tab[k] resolved by ambc_dyn_range_resolve: its chain was stitched past segment 0
+};
+
+static uint64_t dyn_max_entries(uint64_t g, const uint32_t *cands)
+{
+    return min<uint64_t>(AMBC_NMAX, cands[0]) / g;
+}
+
+extern "C" uint64_t ambc_dyn_range_workspace_bytes(uint64_t lo, uint64_t hi, uint64_t n, const uint32_t *cands,
+                                                   uint32_t n_cands)
+{
+    DynLayout L;
+    if (hi < lo || hi > n || dyn_layout(hi - lo, cands, n_cands, L)) return 0;
+    if (dyn_layout(hi - lo, cands, n_cands, L, L.n_seg + dyn_max_entries(L.g, cands))) return 0;
+    return L.total;
+}
+
+extern "C" int ambc_dyn_range_walk(const void *buf_dev, uint64_t buf_len, uint64_t lo, uint64_t hi, uint64_t n,
+                                   const uint32_t *cands, uint32_t n_cands, uint32_t method_mask, uint32_t flags,
+                                   uint32_t marker_bytes, void *work_dev, uint64_t work_bytes, ambc_dyn_range *r,
+                                   ambc_dyn_entry *tab, uint32_t cap, uint32_t *n_tab, void *stream_)
+{
+    cudaStream_t stream = (cudaStream_t)stream_;
+    if (!r || !n_tab || marker_bytes < 1 || marker_bytes > 4 || hi < lo || hi > n)
+        return ambc_fail(AMBC_E_ARG, "ambc_dyn_range_walk: bad argument");
+    memset(r, 0, sizeof(*r));
+    DynLayout L;
+    int rc = dyn_layout(hi - lo, cands, n_cands, L);
+    if (rc) return rc;
+    const uint64_t max_e = dyn_max_entries(L.g, cands);
+    if ((rc = dyn_layout(hi - lo, cands, n_cands, L, L.n_seg + max_e))) return rc;
+    const uint64_t seglen = (uint64_t)DYN_SEGU * L.g;
+    if ((lo % seglen && lo != n) || (hi % seglen && hi != n))
+        return ambc_fail(AMBC_E_ARG, "ambc_dyn_range_walk: lo and hi must be multiples of %llu bytes or n", (unsigned long long)seglen);
+    if (hi > lo && (!buf_dev || ((uintptr_t)buf_dev & 15) || buf_len < min<uint64_t>(n, hi + AMBC_NMAX) - lo))
+        return ambc_fail(AMBC_E_ARG, "ambc_dyn_range_walk: the buffer must be 16-byte aligned and hold [lo, min(n, hi + 8192))");
+    r->lo = lo; r->hi = hi; r->n = n; r->work_bytes = L.total;
+    if (hi > lo && (!work_dev || work_bytes < L.total)) return ambc_fail(AMBC_E_CAPACITY, "ambc_dyn_range_walk: workspace too small");
+    const uint64_t rlen = hi - lo;
+    // the chain enters the first range at 0; any other range at one of n_e positions
+    const uint64_t n_e = lo ? min<uint64_t>(max_e, (rlen + L.g - 1) / L.g) : (rlen ? 1 : 0);
+    if (cap < n_e || (n_e && !tab)) return ambc_fail(AMBC_E_CAPACITY, "ambc_dyn_range_walk: entry table too small");
+
+    DynRangeHost *H = new DynRangeHost();
+    r->host = H;
+    r->work_dev = work_dev;
+    H->L = L; H->lo = lo; H->hi = hi; H->n = n;
+    for (uint32_t i = 0; i < n_cands; i++) H->cands[i] = cands[i];
+    H->n_cands = n_cands; H->mask = method_mask; H->flags = flags; H->ovh = marker_bytes + 14;
+    H->native = (method_mask & AMBC_NATIVE_MASK) != 0;
+    H->pcr = flags & AMBC_F_PER_CHUNK_RAW;
+    H->buf = (const uint8_t *)buf_dev;
+    H->tab.assign(n_e, ambc_dyn_entry());
+    H->resolved.assign(n_e, 0);
+    for (uint64_t k = 0; k < n_e; k++) {
+        ambc_dyn_entry &t = H->tab[k];
+        t.entry = lo + k * L.g; t.exit = ~0ull; t.stop = ~0ull;
+    }
+    if (n_e && H->native) {
+        DynStitch &S = H->S;
+        dyn_stitch_init(S, buf_dev, n - lo, rlen, cands, n_cands, method_mask, H->ovh, H->pcr, true, L, (uint8_t *)work_dev);
+        if ((rc = dyn_spec_walk(S, stream))) return rc;
+        std::vector<unsigned long long> extra;
+        for (uint64_t k = 1; k < n_e; k++) { extra.push_back(0); extra.push_back(k * L.g); }
+        if ((rc = dyn_stitch(S, 0, extra, &H->lo_exit, &H->lo_stop, stream))) return rc;
+        for (uint64_t k = 0; k < n_e; k++) {
+            ambc_dyn_entry &t = H->tab[k];
+            const WalkSeg *w = k ? &S.extra_segs[k - 1] : nullptr;
+            if (!k || w->merged) { // the chain from lo
+                t.status = AMBC_DYN_JOIN;
+                if (H->lo_stop != ~0ull) t.stop = lo + H->lo_stop;
+                else t.exit = lo + H->lo_exit;
+            } else if (w->stop != ~0ull) {
+                t.status = AMBC_DYN_STOP; t.stop = lo + w->stop;
+            } else if (w->exit >= rlen) {
+                t.status = AMBC_DYN_LEAVE; t.exit = lo + w->exit;
+            } else {
+                t.status = AMBC_DYN_UNRESOLVED; t.exit = lo + w->exit;
+            }
+        }
+    } else {
+        // no native method: the rest of the file is raw from the entry on, or per-chunk-raw pieces of cands[-1]
+        const uint64_t cmin = cands[n_cands - 1];
+        for (uint64_t k = 0; k < n_e; k++) {
+            ambc_dyn_entry &t = H->tab[k];
+            if (!H->pcr) { t.status = AMBC_DYN_STOP; t.stop = t.entry; continue; }
+            t.status = AMBC_DYN_LEAVE;
+            t.exit = min<uint64_t>(n, t.entry + (hi - t.entry + cmin - 1) / cmin * cmin);
+        }
+    }
+    for (uint64_t k = 0; k < n_e; k++) tab[k] = H->tab[k];
+    *n_tab = (uint32_t)n_e;
+    r->n_entries = (uint32_t)n_e;
+    return AMBC_OK;
+}
+
+static int dyn_find_entry(const ambc_dyn_range *r, uint64_t entry, uint64_t *k)
+{
+    const DynRangeHost *H = r ? (const DynRangeHost *)r->host : nullptr;
+    if (!H) return ambc_fail(AMBC_E_ARG, "ambc_dyn_range: not walked");
+    for (uint64_t i = 0; i < H->tab.size(); i++)
+        if (H->tab[i].entry == entry) { *k = i; return AMBC_OK; }
+    return ambc_fail(AMBC_E_ARG, "ambc_dyn_range: %llu is not an entry of [%llu, %llu)", (unsigned long long)entry,
+                     (unsigned long long)H->lo, (unsigned long long)H->hi);
+}
+
+extern "C" int ambc_dyn_range_resolve(ambc_dyn_range *r, uint64_t entry, ambc_dyn_entry *out, void *stream_)
+{
+    uint64_t k;
+    int rc = dyn_find_entry(r, entry, &k);
+    if (rc) return rc;
+    DynRangeHost *H = (DynRangeHost *)r->host;
+    ambc_dyn_entry &t = H->tab[k];
+    if (t.status == AMBC_DYN_UNRESOLVED) {
+        uint64_t exit, stop;
+        if ((rc = dyn_stitch(H->S, t.exit - H->lo, {}, &exit, &stop, (cudaStream_t)stream_))) return rc;
+        if (stop != ~0ull) { t.status = AMBC_DYN_STOP; t.stop = H->lo + stop; t.exit = ~0ull; }
+        else { t.status = AMBC_DYN_LEAVE; t.exit = H->lo + exit; }
+        H->resolved[k] = 1;
+    }
+    if (out) *out = t;
+    return AMBC_OK;
+}
+
+extern "C" int ambc_dyn_range_encode(ambc_dyn_range *r, const void *buf_dev, uint64_t entry, const uint8_t *marker,
+                                     uint32_t marker_bytes, void *out_dev, uint64_t out_cap, ambc_compress_result *res,
+                                     ambc_chunk_info *map_out, uint64_t map_cap, uint64_t *stop, void *stream_)
+{
+    cudaStream_t stream = (cudaStream_t)stream_;
+    if (!r || !res || !stop || !marker || marker_bytes < 1 || marker_bytes > 4)
+        return ambc_fail(AMBC_E_ARG, "ambc_dyn_range_encode: bad argument");
+    DynRangeHost *H = (DynRangeHost *)r->host;
+    if (!H) return ambc_fail(AMBC_E_ARG, "ambc_dyn_range_encode: not walked");
+    if (marker_bytes + 14 != H->ovh) return ambc_fail(AMBC_E_ARG, "ambc_dyn_range_encode: marker length differs from the walk's");
+    memset(res, 0, sizeof(*res));
+    res->first_raw = -1;
+    *stop = ~0ull;
+    DynChain C;
+    uint64_t raw_from = ~0ull; // relative
+    if (entry < H->hi) {
+        uint64_t k;
+        int rc = dyn_find_entry(r, entry, &k);
+        if (rc) return rc;
+        const uint64_t e = entry - H->lo;
+        if (!H->native) {
+            if (H->pcr) dyn_raw_pieces(entry, H->hi, H->n, H->cands[H->n_cands - 1], H->lo, C);
+            else raw_from = e;
+        } else if (k == 0) {
+            if ((rc = dyn_chain(H->S, 0, false, C, &raw_from))) return rc;
+        } else {
+            // the candidate's own walk in segment 0, then the chain it met, or its own stitched continuation
+            const WalkSeg &w = H->S.extra_segs[k - 1];
+            for (uint32_t i = 0; i < w.count; i++) C.push(H->S.extra_recs[(k - 1) * DYN_SEGU + i]);
+            if (w.merged) rc = dyn_chain(H->S, w.exit, true, C, &raw_from);
+            else if (w.stop != ~0ull) raw_from = w.stop;
+            else if (w.exit < H->hi - H->lo) {
+                if (!H->resolved[k]) return ambc_fail(AMBC_E_ARG, "ambc_dyn_range_encode: entry %llu is unresolved", (unsigned long long)entry);
+                rc = dyn_chain(H->S, w.exit, false, C, &raw_from);
+            }
+            if (rc) return rc;
+        }
+    }
+    const uint64_t n_list = C.spans.size();
+    if (n_list > H->L.n_pos) return ambc_fail(AMBC_E_ARG, "internal: chain longer than the position table");
+    uint64_t body = 0;
+    for (uint64_t k = 0; k < n_list; k++) body += H->ovh + C.len[k];
+    if (body > out_cap || (body && !out_dev)) return ambc_fail(AMBC_E_CAPACITY, "ambc_dyn_range_encode: out_cap too small");
+    int rc = dyn_encode((const uint8_t *)buf_dev, H->n - H->lo, H->L, (uint8_t *)r->work_dev, C, H->mask, H->ovh,
+                        marker_word_of(marker, marker_bytes), marker_bytes, out_dev, out_cap, body, stream);
+    if (rc) return rc;
+    res->body_len = body;
+    res->n_chunks = res->n_packages = n_list;
+    dyn_result(C, H->lo, res, map_out, map_cap);
+    if (raw_from != ~0ull) *stop = H->lo + raw_from;
+    return AMBC_OK;
+}
+
+extern "C" void ambc_dyn_range_free(ambc_dyn_range *r)
+{
+    if (!r) return;
+    delete (DynRangeHost *)r->host;
+    r->host = nullptr;
 }

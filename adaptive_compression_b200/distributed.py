@@ -17,6 +17,13 @@ the path has:
                       second one of the per-rank tail needs plans the payload bytes a rank fetches
                       from the next ranks (tail_fetch_plan).  Then every rank decodes its own slice.
 
+  compress_dynamic_sharded  the multi-candidate mode (adaptive_compressor.py:537-590): every rank walks the
+                      chunk chain of its own input range (whole segments of 64 * g bytes, dyn_shard_ranges)
+                      from every position the chain can enter it at; an all-gather of the fixed-size entry
+                      tables and a host fold (fold_dyn_entries) find the true entries, a rank whose true
+                      entry is still open stitches it further, then every rank encodes its own packages
+                      and one all-gather of (fragment bytes, stop) places them (dyn_fragment_plan).
+
 A rank compresses its range as if no earlier rank had hit a chunk without a winner; shard_fragment()
 then turns the local body into the bytes this rank contributes to the global body."""
 import struct
@@ -161,8 +168,14 @@ def assemble_body(frag, records, total_bytes, chunk, marker_bytes=4, dst=0, out=
     """Gather every rank's fragment into ONE body on rank `dst` (NCCL send / recv straight into the placed
     slice of the destination buffer -- NVLink peer copies; gloo on CPU).  Returns the body tensor on `dst`
     (None elsewhere).  `out`: optional preallocated destination on `dst` (>= body length)."""
-    rank, world = dist.get_rank(), dist.get_world_size()
     plan, body_len = fragment_plan(records, total_bytes, chunk, marker_bytes)
+    return gather_fragments(frag, plan, body_len, dst, out)
+
+
+def gather_fragments(frag, plan, body_len, dst=0, out=None):
+    """send every rank's fragment to its place [offset, offset + length) of the plan in ONE body on rank `dst`;
+    -> the body on `dst`, None elsewhere"""
+    rank = dist.get_rank()
     if rank != dst:
         if frag.numel():
             dist.send(frag.contiguous(), dst)
@@ -402,3 +415,176 @@ def decompress_sharded(buf, lo, hi, body_len, orig_size, marker=b"\xff\xff\x00\x
     for q in reqs:
         q.wait()
     return 0, whole, [int(x) for x in st.cpu().tolist()]
+
+
+# ---- the multi-candidate mode across ranks ------------------------------------------------------------------------
+DYN_SEGU = 64      # positions (multiples of g) per segment of the chain walk
+DYN_HALO = 8192    # the winner at p depends on input[p, p + 8192) (and on n - p)
+DYN_TABLE_WORDS = 4 * 32 + 1
+
+
+def _gcd_of(candidates):
+    import math
+    g = 0
+    for c in candidates:
+        g = math.gcd(g, int(c))
+    return g
+
+
+def dyn_shard_ranges(n, candidates, world):
+    """[(lo, hi)] per rank: whole segments of 64 * g input bytes, the last non-empty range ends at n; trailing
+    ranks are empty (n, n) when there are fewer segments than ranks"""
+    seglen = DYN_SEGU * _gcd_of(candidates)
+    n_seg = -(-n // seglen)
+    per = -(-n_seg // world) if world else 0
+    return [(min(n, r * per * seglen), min(n, (r + 1) * per * seglen)) for r in range(world)]
+
+
+def dyn_buffer_span(lo, hi, n):
+    """input bytes [b0, b1) a rank holds for its range: the range and the 8192-byte halo behind it"""
+    return lo, min(n, hi + DYN_HALO) if hi > lo else lo
+
+
+def fold_dyn_entries(tables, n):
+    """tables[r] = rank r's entry rows [(entry, status, exit, stop)] (exit / stop None when absent), rank order.
+    Follows the chain from position 0 through the ranks -> (entries, stuck, stop): entries[r] = the true entry
+    into rank r (None: the chain ended or stopped before it), stuck = the first rank whose true entry is
+    unresolved (None once the fold is complete), stop = where the rest of the file becomes one raw package (None)"""
+    from . import _lib as L
+    entries, e = [None] * len(tables), 0
+    for r, tab in enumerate(tables):
+        if e >= n:
+            break
+        if not tab:
+            continue  # an empty range
+        row = next((t for t in tab if t[0] == e), None)
+        if row is None:
+            raise RuntimeError("the chain enters rank %d at %d, which its entry table does not hold" % (r, e))
+        entries[r] = e
+        _, status, exit_, stop = row
+        if status == L.DYN_UNRESOLVED:
+            return entries, r, None
+        if stop is not None:
+            return entries, None, stop
+        e = exit_
+    return entries, None, None
+
+
+def dyn_fragment_plan(records, ranges, n, marker_bytes=4):
+    """records[r] = (bytes of rank r's encoded packages, stop or -1); ranges = dyn_shard_ranges().
+    -> ([(offset, length, state)] per rank, body length): the first rank whose chain stops writes the raw
+    header and its input bytes [stop, hi), later ranks their input [lo, hi) verbatim, the last rank the END
+    package.  A raw package of 4 GiB or more cannot be framed (adaptive_compressor.py:617-619)."""
+    from . import _lib as L
+    ovh, end = marker_bytes + 14, marker_bytes + 12
+    stop = next((int(st) for _, st in records if st >= 0), -1)
+    if stop >= 0 and n - stop > 0xFFFFFFFF:
+        raise L.AmbcError(L.E_ARG, "raw package over 4 GiB cannot be framed (u32 fields)")
+    plan, off, raw_seen = [], 0, False
+    for r, ((nbytes, st), (lo, hi)) in enumerate(zip(records, ranges)):
+        if raw_seen:
+            state, length = "in_raw_tail", hi - lo
+        elif st >= 0:
+            state, length, raw_seen = "raw_starts_here", nbytes + ovh + (hi - st), True
+        else:
+            state, length = "packed", nbytes
+        if r == len(records) - 1:
+            length += end
+        plan.append((off, length, state))
+        off += length
+    return plan, off
+
+
+def _all_rows(tab, dev):
+    """all-gather of every rank's entry table (fixed size) -> list of row lists"""
+    from . import _lib as L
+    world = dist.get_world_size()
+    words = [len(tab)]
+    for e, st, ex, sp in tab:
+        words += [e, st, -1 if ex is None else ex, -1 if sp is None else sp]
+    words += [0] * (DYN_TABLE_WORDS - len(words))
+    allw = torch.empty(DYN_TABLE_WORDS * world, dtype=torch.int64, device=dev)
+    dist.all_gather_into_tensor(allw, torch.tensor(words, dtype=torch.int64, device=dev))
+    out = []
+    for row in allw.view(world, DYN_TABLE_WORDS).cpu().tolist():
+        k = int(row[0])
+        out.append([(int(row[1 + 4 * i]), int(row[2 + 4 * i]), None if row[3 + 4 * i] < 0 else int(row[3 + 4 * i]),
+                     None if row[4 + 4 * i] < 0 else int(row[4 + 4 * i])) for i in range(k)])
+    assert all(len(t) <= L.DYN_MAX_ENTRIES for t in out)
+    return out
+
+
+def settle_dyn_entries(table, n, resolve, dev):
+    """the fold loop: all-gather every rank's entry table, fold, let the first rank whose true entry is unresolved
+    resolve it (resolve(entry) -> its updated table), repeat; at most one round per rank.
+    -> (entries, stop, rounds) as fold_dyn_entries gives them once complete"""
+    rank, world = dist.get_rank(), dist.get_world_size()
+    for rounds in range(1, world + 1):
+        entries, stuck, stop = fold_dyn_entries(_all_rows(table, dev), n)
+        if stuck is None:
+            return entries, stop, rounds
+        if stuck == rank:
+            table = resolve(entries[rank])
+    raise RuntimeError("the fold of the entry tables does not settle within %d rounds" % world)
+
+
+def dyn_fragment(frag, stop, state, t_buf, lo, hi, n, marker, last):
+    """the bytes a rank contributes to the body (dyn_fragment_plan state): its packages, then the raw header and its
+    input bytes [stop, hi) when its chain stops there, or its input [lo, hi) inside the raw tail; END on the last
+    rank.  t_buf = input[lo, ...) on the rank's device."""
+    dev = t_buf.device
+    parts = [frag]
+    if state == "raw_starts_here":
+        raw = n - stop
+        hdr = marker + bytes([255, 0]) + struct.pack("<III", raw, raw, raw)
+        parts += [torch.tensor(list(hdr), dtype=torch.uint8, device=dev), t_buf[stop - lo:hi - lo]]
+    elif state == "in_raw_tail":
+        parts = [t_buf[:hi - lo]]
+    if last:
+        parts.append(torch.tensor(list(marker + bytes(12)), dtype=torch.uint8, device=dev))
+    return torch.cat(parts) if len(parts) > 1 else parts[0]
+
+
+def compress_dynamic_sharded(t_buf, lo, hi, n, candidates, mask=None, flags=0, marker=b"\xff\xff\x00\x00", dst=0):
+    """Multi-candidate compression of an input whose ranges are spread over the ranks (dyn_shard_ranges() order;
+    t_buf = input[dyn_buffer_span(lo, hi, n)] on this rank's GPU).  -> (body on `dst` (None elsewhere), the package
+    list [(type, orig, comp)], usage [raw, 1..4], payload bytes): what engine.compress_dynamic_device gives for the
+    whole input.  Raises AmbcError(E_ARG) on every rank where the single-GPU call would."""
+    from . import _lib as L
+    from . import engine
+    mask = L.NATIVE_MASK if mask is None else mask
+    rank, world = dist.get_rank(), dist.get_world_size()
+    ranges = dyn_shard_ranges(n, candidates, world)
+    assert ranges[rank] == (lo, hi), "ranges follow dyn_shard_ranges(n, candidates, world)"
+    dev = t_buf.device
+    mb = len(marker)
+    dr = engine.dyn_range_walk(t_buf, lo, hi, n, candidates, mask, flags, mb)
+
+    def resolve(entry):
+        engine.dyn_range_resolve(dr, entry)
+        return dr.table
+    entries, _, _ = settle_dyn_entries(dr.table, n, resolve, dev)
+    mine = entries[rank]
+    if mine is not None and mine < hi:
+        frag, my_stop, pk, usage, payload = engine.dyn_range_encode(dr, mine, marker)
+    else:
+        frag, my_stop, pk, usage, payload = t_buf[:0], None, [], [0] * 5, 0
+    rec = torch.tensor([frag.numel(), -1 if my_stop is None else my_stop], dtype=torch.int64, device=dev)
+    allr = torch.empty(2 * world, dtype=torch.int64, device=dev)
+    dist.all_gather_into_tensor(allr, rec)
+    records = [tuple(int(x) for x in r) for r in allr.view(world, 2).cpu().tolist()]
+    plan, body_len = dyn_fragment_plan(records, ranges, n, mb)
+    _, _, state = plan[rank]
+    local = dyn_fragment(frag, my_stop, state, t_buf, lo, hi, n, marker, rank == world - 1)
+    body = gather_fragments(local, plan, body_len, dst)
+    # the package list and the counters, with the raw tail package of the rank that stops
+    if state == "raw_starts_here":
+        pk = pk + [(my_stop, 255, n - my_stop, n - my_stop)]
+        usage = [usage[0] + 1] + usage[1:]
+    lists = [None] * world
+    dist.all_gather_object(lists, pk)
+    cnt = torch.tensor(list(usage) + [payload], dtype=torch.int64, device=dev)
+    dist.all_reduce(cnt)
+    cnt = cnt.cpu().tolist()
+    packages = [(t, o, c) for part in lists for _, t, o, c in part]
+    return body, packages, [int(x) for x in cnt[:5]], int(cnt[5])

@@ -107,6 +107,80 @@ def compress_dynamic_device(t_in, candidates, mask=L.NATIVE_MASK, flags=0, marke
     return o
 
 
+# ---- one rank's input range of the multi-candidate mode (ambc_dyn_range_*) -------------------------------------
+def _cands(candidates):
+    cands = sorted({int(c) for c in candidates}, reverse=True)
+    return cands, (C.c_uint32 * len(cands))(*cands)
+
+
+class DynRange:
+    """a rank's walked range (ambc_dyn_range_walk): the workspace, the buffer it was walked on and the entry table
+    [(entry, status, exit, stop)] (exit / stop None when absent)"""
+    __slots__ = ("r", "work", "buf", "table", "__weakref__")
+
+    def __del__(self):
+        if getattr(self, "r", None) is not None and L._lib is not None:
+            L._lib.ambc_dyn_range_free(C.byref(self.r))
+
+
+def _dyn_row(e):
+    none = lambda v: None if v == L.DYN_NONE else int(v)  # noqa: E731
+    return (int(e.entry), int(e.status), none(e.exit), none(e.stop))
+
+
+def dyn_range_walk(t_buf, lo, hi, n, candidates, mask=L.NATIVE_MASK, flags=0, marker_bytes=4, work=None):
+    """phase 1 on input [lo, hi): t_buf = input[lo, min(n, hi + 8192)) as a device tensor -> DynRange"""
+    lib = require_cuda()
+    _, arr = _cands(candidates)
+    wbytes = lib.ambc_dyn_range_workspace_bytes(lo, hi, n, arr, len(arr))
+    if wbytes == 0:
+        raise L.AmbcError(L.E_ARG, lib.ambc_last_error().decode("utf-8", "replace"))
+    if work is None or work.numel() < wbytes:
+        work = torch.empty(int(wbytes), dtype=torch.uint8, device="cuda")
+    dr = DynRange()
+    dr.r = L.DynRange()
+    tab = (L.DynEntry * L.DYN_MAX_ENTRIES)()
+    nt = C.c_uint32(0)
+    rc = lib.ambc_dyn_range_walk(C.c_void_p(t_buf.data_ptr() if t_buf.numel() else 0), t_buf.numel(), lo, hi, n, arr,
+                                 len(arr), mask, flags, marker_bytes, C.c_void_p(work.data_ptr()), work.numel(),
+                                 C.byref(dr.r), tab, L.DYN_MAX_ENTRIES, C.byref(nt), _stream_ptr())
+    L.check(rc)
+    dr.work, dr.buf = work, t_buf
+    dr.table = [_dyn_row(tab[k]) for k in range(nt.value)]
+    return dr
+
+
+def dyn_range_resolve(dr, entry):
+    """phase 2: stitch the chain from an unresolved entry until it leaves the range or stops -> its updated row
+    (also stored in dr.table)"""
+    out = L.DynEntry()
+    L.check(require_cuda().ambc_dyn_range_resolve(C.byref(dr.r), entry, C.byref(out), _stream_ptr()))
+    row = _dyn_row(out)
+    dr.table = [row if t[0] == entry else t for t in dr.table]
+    return row
+
+
+def dyn_range_encode(dr, entry, marker=FIXED_MARKER, out=None):
+    """phase 3: the rank's packages of the chain from its true entry -> (fragment device tensor, stop or None,
+    [(pos, type, orig, comp)] with global positions, usage [raw, 1..4], payload bytes)"""
+    lib = require_cuda()
+    r = dr.r
+    n_pos = max((r.hi - r.lo) // 256 + 2, 1)
+    bound = (r.hi - r.lo) + 8192 + n_pos * (len(marker) + 14) + 64
+    if out is None or out.numel() < bound:
+        out = torch.empty(bound, dtype=torch.uint8, device="cuda")
+    info = (L.ChunkInfo * n_pos)()
+    res = L.CompressResult()
+    stop = C.c_uint64(0)
+    L.check(lib.ambc_dyn_range_encode(C.byref(r), C.c_void_p(dr.buf.data_ptr() if dr.buf.numel() else 0), entry, marker,
+                                      len(marker), C.c_void_p(out.data_ptr()), out.numel(), C.byref(res), info, n_pos,
+                                      C.byref(stop), _stream_ptr()))
+    pk = [(int(info[k].pos), int(info[k].type), int(info[k].orig_len), int(info[k].comp_len))
+          for k in range(int(res.n_packages))]
+    return (out[:res.body_len], None if stop.value == L.DYN_NONE else int(stop.value), pk, list(res.usage),
+            int(res.payload_bytes))
+
+
 def package_map(o, n, chunk, per_chunk_raw=False):
     """[(type, orig, comp)] per package, as the reference's package walk would list them"""
     types = o.types.cpu().numpy()

@@ -132,6 +132,59 @@ int ambc_compress_dynamic_dev(const void *in_dev, uint64_t n, const uint32_t *ca
                               void *out_dev, uint64_t out_cap, void *work_dev, uint64_t work_bytes,
                               ambc_compress_result *res, ambc_chunk_info *map_out, uint64_t map_cap, void *stream);
 
+/*
+ * The multi-candidate mode across ranks: every rank holds one input range [lo, hi) and walks its chain; the fold of
+ * the ranks' entry tables is host arithmetic (adaptive_compression_b200/distributed.py).  lo and hi are multiples of
+ * 64 * g (g = gcd of the candidates), except that the last rank's hi is n.  The chain enters a range at a multiple of
+ * g in [lo, lo + min(8192, cands[0])): a non-raw package is at most that long.
+ *
+ *   1. ambc_dyn_range_walk    (no communication) walks the range's segments, stitches the chain from lo, and in the
+ *      first re-entry launch walks every other possible entry lo + k * g until it meets the chain from lo in the
+ *      range's first segment.  Fills one ambc_dyn_entry per possible entry (lo first).
+ *   2. ambc_dyn_range_resolve runs more stitch rounds from an entry the walk left AMBC_DYN_UNRESOLVED, until the
+ *      chain from it leaves the range or stops.
+ *   3. ambc_dyn_range_encode  encodes and frames the rank's packages of the chain from its true entry with the
+ *      records already walked: no raw tail, no END; map positions are global.  *stop = the position the chain
+ *      stops at (the rest of the file is one raw package), ~0 if it leaves the range.
+ *
+ * buf_dev holds input bytes [lo, min(n, hi + 8192)), 16-byte aligned, and stays valid until the last call; the
+ * host side of the walk lives in r->host until ambc_dyn_range_free.
+ */
+typedef struct {
+    uint64_t entry;    /* input position the chain enters the range at                                       */
+    uint64_t exit;     /* first position of the chain at or past hi (>= n: the chain is complete), ~0 if none */
+    uint64_t stop;     /* strict mode: no winner there, the rest of the file is raw; ~0 if none              */
+    uint32_t status;   /* AMBC_DYN_*                                                                          */
+    uint32_t reserved;
+} ambc_dyn_entry;
+#define AMBC_DYN_JOIN 0       /* meets the chain from lo: exit / stop are that chain's                           */
+#define AMBC_DYN_LEAVE 1      /* leaves the range at exit without meeting it                                     */
+#define AMBC_DYN_STOP 2       /* stops at stop without meeting it                                                */
+#define AMBC_DYN_UNRESOLVED 3 /* left the first segment at exit without meeting it: ambc_dyn_range_resolve       */
+#define AMBC_DYN_MAX_ENTRIES 32
+
+typedef struct {
+    uint64_t lo, hi, n;   /* the rank's input range and the input length                                      */
+    uint64_t work_bytes;  /* device workspace the range needs (also set when AMBC_E_CAPACITY is returned)     */
+    void *work_dev;
+    void *host;           /* the walk's records on the host (ambc_dyn_range_free)                             */
+    uint32_t n_entries, reserved;
+} ambc_dyn_range;
+
+uint64_t ambc_dyn_range_workspace_bytes(uint64_t lo, uint64_t hi, uint64_t n, const uint32_t *cands, uint32_t n_cands);
+/* Phase 1 (synchronises `stream`); tab gets r->n_entries <= AMBC_DYN_MAX_ENTRIES entries (cap of them at most) */
+int ambc_dyn_range_walk(const void *buf_dev, uint64_t buf_len, uint64_t lo, uint64_t hi, uint64_t n,
+                        const uint32_t *cands, uint32_t n_cands, uint32_t method_mask, uint32_t flags,
+                        uint32_t marker_bytes, void *work_dev, uint64_t work_bytes, ambc_dyn_range *r,
+                        ambc_dyn_entry *tab, uint32_t cap, uint32_t *n_tab, void *stream);
+/* Phase 2: *out = the entry's row, resolved (a no-op for an entry the walk resolved).  Synchronises `stream`. */
+int ambc_dyn_range_resolve(ambc_dyn_range *r, uint64_t entry, ambc_dyn_entry *out, void *stream);
+/* Phase 3: the rank's packages into out_dev (res->body_len bytes); entry >= hi: none.  Synchronises `stream`. */
+int ambc_dyn_range_encode(ambc_dyn_range *r, const void *buf_dev, uint64_t entry, const uint8_t *marker,
+                          uint32_t marker_bytes, void *out_dev, uint64_t out_cap, ambc_compress_result *res,
+                          ambc_chunk_info *map_out, uint64_t map_cap, uint64_t *stop, void *stream);
+void ambc_dyn_range_free(ambc_dyn_range *r);
+
 /* ------------------------------------------------------------------ */
 /* decompress: AdaptiveCompressor._adaptive_decompress                  */
 /*   adaptive_compressor.py:396-454                                     */

@@ -17,8 +17,12 @@ What differs, on purpose:
     out of scope.
   * per_chunk_raw=True and use_marker_search=True are labelled extensions (files stay readable by
     the reference decoder)."""
+import ctypes as C
 import hashlib
 import os
+import secrets
+import shutil
+import stat
 import struct
 import threading
 import time
@@ -27,7 +31,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
-from . import engine
+from . import engine, windowed
 from .compression_methods import (BZip2Compression, DeflateCompression, DeltaCompression, DictionaryCompression,
                                   HuffmanCompression, LZMACompression, NoCompression, RLECompression)
 from .marker_finder import MarkerFinder
@@ -40,6 +44,48 @@ METHOD_CHUNK_PREFS = {1: (32, 4096), 2: (128, 8192), 3: (32, 8192), 4: (32, 4096
 
 
 REFERENCE_CANDIDATES = (131072, 65536, 32768, 16384, 8192, 4096, 2048, 1024)  # adaptive_compressor.py:61-62
+
+WINDOW_CAP = 4 << 30      # largest window of the windowed path (DESIGN.md §4.6)
+WINDOW_MIN = 16 << 20
+MEMORY_MARGIN = 2 << 30   # device memory left free for the allocator's rounding, other streams and library scratch
+
+
+def window_bytes(need, device_bytes):
+    """The path of one compress / decompress call.  need = device bytes the in-memory path allocates for this file,
+    device_bytes(W) = those of the windowed path with windows of W bytes.  -> None when `need` fits the free device
+    memory with a margin (the in-memory path runs), else the window size: the largest power of two up to WINDOW_CAP
+    whose windowed path fits."""
+    free = torch.cuda.mem_get_info()[0] + torch.cuda.memory_reserved() - torch.cuda.memory_allocated()
+    if need + MEMORY_MARGIN <= free:
+        return None
+    w = WINDOW_CAP
+    while w > WINDOW_MIN and device_bytes(w) + MEMORY_MARGIN > free:
+        w //= 2
+    return w
+
+
+def _temp_beside(path):
+    """-> (temporary file, final file): an empty file beside the file `path` names (through a symlink, which is
+    kept), with the mode of the file it will replace, or else the mode a new file gets there (0o666 less the
+    umask, applied by open)"""
+    target = os.path.realpath(path)
+    try:
+        mode = stat.S_IMODE(os.stat(target).st_mode)
+    except FileNotFoundError:
+        mode = None
+    while True:
+        tmp = os.path.join(os.path.dirname(target), ".%s.%s.tmp" % (os.path.basename(target), secrets.token_hex(6)))
+        try:
+            fd = os.open(tmp, os.O_WRONLY | os.O_CREAT | os.O_EXCL, 0o666)
+            break
+        except FileExistsError:
+            continue
+    try:
+        if mode is not None:
+            os.fchmod(fd, mode)
+    finally:
+        os.close(fd)
+    return tmp, target
 
 
 class AdaptiveCompressor:
@@ -207,11 +253,35 @@ class AdaptiveCompressor:
             return h.digest()
         return buf[:n], join
 
+    def _compress_need(self, n, chunk):
+        """device bytes of the in-memory compress of n bytes, from the library's own size functions (marker of at
+        most 4 bytes; the host-buffer path adds 1/8 to each cached buffer)"""
+        lib = L.lib()
+        if chunk is None:
+            cands = sorted({int(c) for c in self.CHUNK_SIZE_CANDIDATES}, reverse=True)
+            g = windowed.D._gcd_of(cands)
+            need = 2 * n + (n // g + 3) * 18 + 80 + int(lib.ambc_compress_dynamic_workspace_bytes(
+                n, (C.c_uint32 * len(cands))(*cands), len(cands)))
+        else:
+            need = (n + 64 + int(lib.ambc_compress_bound(n, chunk, 4)) + int(lib.ambc_compress_workspace_bytes(n, chunk)))
+            need += need // 8
+        if self.use_marker_search:  # the input, the 2^32 flags and the pick's scratch of the 32-bit level
+            need = max(need, n + (2 << 32))
+        return need
+
     def compress(self, input_file, output_file):
         start_t = time.time()
         engine.require_cuda()
         chunk = self._fixed_chunk()
         mask = self._method_mask()
+        n = os.path.getsize(input_file)
+        if chunk is None:
+            W = window_bytes(self._compress_need(n, None),
+                             lambda w: windowed.dynamic_device_bytes(w, self.CHUNK_SIZE_CANDIDATES))
+        else:
+            W = window_bytes(self._compress_need(n, chunk), lambda w: windowed.fixed_device_bytes(w, chunk))
+        if W is not None:
+            return self._compress_windowed(input_file, output_file, n, chunk, mask, W, start_t)
         file_data, md5_join = self._read_with_md5(input_file, "in")
         n = int(file_data.size)
         t_read = time.time()
@@ -252,6 +322,59 @@ class AdaptiveCompressor:
         self.last_timing = {"read_s": t_read - start_t, "gpu_s": t_gpu - t_read, "total_s": time.time() - start_t}
         return stats
 
+    def _compress_windowed(self, input_file, output_file, n, chunk, mask, W, start_t):
+        """compress() through windows of W bytes (windowed.py): the same file and stats; the output appears by a
+        rename once complete"""
+        if self.use_marker_search:
+            marker_bytes, marker_len = windowed.find_marker(input_file, n, W, min(int(self.marker_finder.max_marker_length), 32))
+        else:
+            marker_bytes, marker_len = b"\xff\xff\x00\x00", 32
+        self._init_marker(marker_bytes, marker_len)
+        t_read = time.time()
+        flags = L.F_PER_CHUNK_RAW if self.per_chunk_raw else 0
+        tmp, target = _temp_beside(output_file)
+        try:
+            with open(tmp, "wb") as f:
+                header = self._build_header(marker_bytes[:self.marker_byte_length], marker_len, b"\0" * 16, n, 0)
+                f.write(header)
+                if chunk is None:
+                    body_len, md5, cnt = windowed.compress_dynamic(input_file, f, n, self.CHUNK_SIZE_CANDIDATES, W, mask,
+                                                                   flags, self.marker_bytes_aligned)
+                else:
+                    body_len, md5, cnt = windowed.compress_fixed(input_file, f, n, chunk, W, mask, flags,
+                                                                 self.marker_bytes_aligned)
+                final_size = len(header) + body_len
+                if final_size <= n:
+                    f.seek(0)
+                    f.write(self._build_header(marker_bytes[:self.marker_byte_length], marker_len, md5, n, body_len))
+            t_gpu = time.time()
+            self._store_chunk_stats(cnt.n_packages, cnt.n_comp, cnt.usage, cnt.saved, cnt.payload, n)
+            if final_size > n:
+                print("Compression bigger than original => store raw.")
+                shutil.copyfile(input_file, tmp)
+                stats = self._build_stats_raw(n, time.time() - start_t)
+            else:
+                stats = self._calculate_compression_stats(n, final_size, time.time() - start_t)
+            os.replace(tmp, target)
+        except BaseException:
+            os.unlink(tmp)
+            raise
+        self.last_timing = {"read_s": t_read - start_t, "gpu_s": t_gpu - t_read, "total_s": time.time() - start_t}
+        return stats
+
+    def _store_chunk_stats(self, n_packages, n_comp, usage_counts, saved, payload, n):
+        """chunk_stats as _init_stats/_update_stats (:457-480) leave them; usage_counts = [raw, 1, 2, 3, 4]"""
+        ovh = self.marker_byte_length + 14
+        usage = {m.type_id: 0 for m in self.compression_methods}
+        for mid in (1, 2, 3, 4):
+            if mid in usage:
+                usage[mid] = int(usage_counts[mid])
+        self.chunk_stats = {
+            "total_chunks": int(n_packages), "compressed_chunks": int(n_comp), "raw_chunks": int(n_packages) - int(n_comp),
+            "method_usage": usage, "bytes_saved": int(saved), "original_size": n,
+            "compressed_size_without_overhead": int(payload), "overhead_bytes": ovh * int(n_comp) + self.marker_byte_length + 12,
+        }
+
     def _fill_chunk_stats(self, out, types, comps, n, chunk):
         """same numbers as _init_stats/_update_stats (:457-480) + the END overhead (:393); out = CompressResult,
         types / comps = the per-chunk method map"""
@@ -265,40 +388,16 @@ class AdaptiveCompressor:
         origs = np.full(limit, chunk, dtype=np.int64)
         if limit and limit == int(out.n_chunks):
             origs[-1] = n - (limit - 1) * chunk
-        usage = {m.type_id: 0 for m in self.compression_methods}
-        for mid in (1, 2, 3, 4):
-            c = int((t == mid).sum())
-            if mid in usage:
-                usage[mid] = c
-        n_comp = int(comp_mask.sum())
-        self.chunk_stats = {
-            "total_chunks": int(out.n_packages),
-            "compressed_chunks": n_comp,
-            "raw_chunks": int(out.n_packages) - n_comp,
-            "method_usage": usage,
-            "bytes_saved": int((origs[comp_mask] - comps[:limit][comp_mask] - ovh).sum()),
-            "original_size": n,
-            "compressed_size_without_overhead": int(comps[:limit][comp_mask].sum()),
-            "overhead_bytes": ovh * n_comp + self.marker_byte_length + 12,
-        }
+        usage = {mid: int((t == mid).sum()) for mid in (1, 2, 3, 4)}
+        self._store_chunk_stats(out.n_packages, int(comp_mask.sum()), [0] + [usage.get(mid, 0) for mid in (1, 2, 3, 4)],
+                                (origs[comp_mask] - comps[:limit][comp_mask] - ovh).sum(),
+                                comps[:limit][comp_mask].sum(), n)
 
     def _fill_chunk_stats_packages(self, packages, n):
         """_init_stats/_update_stats (:457-480) from a package list [(type, orig, comp)]"""
-        ovh = self.marker_byte_length + 14
-        usage = {m.type_id: 0 for m in self.compression_methods}
-        n_comp = saved = payload = 0
-        for t, orig, comp in packages:
-            if t != 255:
-                n_comp += 1
-                saved += orig - comp - ovh
-                payload += comp
-                if t in usage:
-                    usage[t] += 1
-        self.chunk_stats = {
-            "total_chunks": len(packages), "compressed_chunks": n_comp, "raw_chunks": len(packages) - n_comp,
-            "method_usage": usage, "bytes_saved": saved, "original_size": n,
-            "compressed_size_without_overhead": payload, "overhead_bytes": ovh * n_comp + self.marker_byte_length + 12,
-        }
+        cnt = windowed.Counters()
+        cnt.add_packages(packages, self.marker_byte_length + 14)
+        self._store_chunk_stats(cnt.n_packages, cnt.n_comp, cnt.usage, cnt.saved, cnt.payload, n)
 
     def _build_stats_raw(self, original_size, elapsed):
         tput = original_size / (1024 * 1024 * elapsed) if elapsed > 0 else 0.0
@@ -334,6 +433,16 @@ class AdaptiveCompressor:
         start_t = time.time()
         engine.require_cuda()
         size = os.path.getsize(input_file)
+        with open(input_file, "rb") as f:
+            hdr = self._parse_header(f.read(64))
+        body_len = max(size - hdr["header_size"], 0)
+        # ambc_decompress_host caches the body, the output and a table ring, each with 1/8 on top
+        need = (body_len + hdr["original_size"] + (4 << 20)) * 9 // 8
+        # one package's payload behind a halo and its output piece may each reach 2^32 - 1 bytes
+        W = window_bytes(need, lambda w: windowed.decompress_device_bytes(w, w, (hdr["marker_length"] + 7) // 8,
+                                                                         big=2 * 0xFFFFFFFF))
+        if W is not None:
+            return self._decompress_windowed(input_file, output_file, size, hdr, W, start_t)
         cdata = engine.pinned("cin", max(size, 1))[:size]
         with open(input_file, "rb", buffering=0) as f:
             pos = 0
@@ -363,3 +472,27 @@ class AdaptiveCompressor:
         dsize = int(decompressed.size)
         return {"compressed_size": int(cdata.size), "decompressed_size": dsize, "elapsed_time": elapsed,
                 "throughput_mb_per_sec": dsize / (1024 * 1024 * elapsed) if elapsed > 0 else 0.0}
+
+    def _decompress_windowed(self, input_file, output_file, size, hdr, W, start_t):
+        """decompress() through body windows of W bytes (windowed.py), the output bounded by W too.  Errors as in
+        the reference: on a marker mismatch no output appears; on a checksum mismatch the output is written first"""
+        self._init_marker(hdr["marker_bytes"], hdr["marker_length"])
+        known = engine.method_mask([m.type_id for m in self.compression_methods if m.type_id != 255])
+        orig = hdr["original_size"]
+        tmp, target = _temp_beside(output_file)
+        try:
+            with open(tmp, "wb") as f:
+                md5, status = windowed.decompress(input_file, f, hdr["header_size"], max(size - hdr["header_size"], 0),
+                                                  orig, W, self.marker_bytes_aligned, known)
+            os.replace(tmp, target)
+        except BaseException:
+            os.unlink(tmp)
+            raise
+        self.last_status = status
+        if md5 != hdr["checksum"]:
+            raise ValueError("Checksum mismatch => possibly corrupted file.")
+        if status != [0, 0]:
+            print("Warning: %d package(s) failed to decode, %d with a length mismatch" % (status[0], status[1]))
+        elapsed = time.time() - start_t
+        return {"compressed_size": size, "decompressed_size": orig, "elapsed_time": elapsed,
+                "throughput_mb_per_sec": orig / (1024 * 1024 * elapsed) if elapsed > 0 else 0.0}

@@ -34,6 +34,24 @@ import torch.distributed as dist
 NO_RAW = -1
 
 
+def raw_package_header(marker, rawlen):
+    """the header of the raw package that holds the rest of the file (adaptive_compressor.py:586-590, :609-621);
+    struct.error for 4 GiB or more, as the reference's struct.pack at :617-619"""
+    return marker + bytes([255, 0]) + struct.pack("<III", rawlen, rawlen, rawlen)
+
+
+def end_package(marker):
+    """the END package (adaptive_compressor.py:595-607)"""
+    return marker + bytes(12)
+
+
+def refuse_dyn_raw(n, stop):
+    """the multi-candidate mode refuses a raw package of 4 GiB or more as ambc_compress_dynamic_dev does"""
+    from . import _lib as L
+    if stop >= 0 and n - stop > 0xFFFFFFFF:
+        raise L.AmbcError(L.E_ARG, "raw package over 4 GiB cannot be framed (u32 fields)")
+
+
 def shard_range(total_bytes, chunk, rank, world):
     """contiguous chunk range of `rank`: (first_chunk, byte_begin, byte_end)"""
     n_chunks = (total_bytes + chunk - 1) // chunk
@@ -142,7 +160,7 @@ def shard_fragment(local_body, local_input, first_raw_local, first_chunk_global,
     n_local = local_input.numel()
     pk = packed_bytes(local_body.numel(), n_local, first_raw_local, chunk, mb)
     last = rank == len(records) - 1
-    end_pkg = torch.tensor(list(marker + bytes(12)), dtype=torch.uint8, device=local_body.device)
+    end_pkg = torch.tensor(list(end_package(marker)), dtype=torch.uint8, device=local_body.device)
     g = next((fr for _, fr in records if fr >= 0), NO_RAW)  # global first raw chunk
     if state == "packed":
         if last and first_raw_local < 0:  # the local body ends with the same END package: no copy
@@ -153,8 +171,7 @@ def shard_fragment(local_body, local_input, first_raw_local, first_chunk_global,
         rawlen = total_bytes - g * chunk
         if rawlen > 0xFFFFFFFF:
             raise struct.error("'I' format requires 0 <= number <= 4294967295")  # adaptive_compressor.py:617-619
-        hdr = marker + bytes([255, 0]) + struct.pack("<III", rawlen, rawlen, rawlen)
-        hdr_t = torch.tensor(list(hdr), dtype=torch.uint8, device=local_body.device)
+        hdr_t = torch.tensor(list(raw_package_header(marker, rawlen)), dtype=torch.uint8, device=local_body.device)
         frag = torch.cat([local_body[:pk], hdr_t, local_input[first_raw_local * chunk:]])
     else:
         frag = local_input
@@ -457,9 +474,7 @@ def fold_dyn_entries(tables, n):
             break
         if not tab:
             continue  # an empty range
-        row = next((t for t in tab if t[0] == e), None)
-        if row is None:
-            raise RuntimeError("the chain enters rank %d at %d, which its entry table does not hold" % (r, e))
+        row = entry_row(tab, e, "rank %d" % r)
         entries[r] = e
         _, status, exit_, stop = row
         if status == L.DYN_UNRESOLVED:
@@ -470,16 +485,21 @@ def fold_dyn_entries(tables, n):
     return entries, None, None
 
 
+def entry_row(tab, e, where):
+    """the row of entry e in a walked range's entry table [(entry, status, exit, stop)]"""
+    row = next((t for t in tab if t[0] == e), None)
+    if row is None:
+        raise RuntimeError("the chain enters %s at %d, which its entry table does not hold" % (where, e))
+    return row
+
+
 def dyn_fragment_plan(records, ranges, n, marker_bytes=4):
     """records[r] = (bytes of rank r's encoded packages, stop or -1); ranges = dyn_shard_ranges().
     -> ([(offset, length, state)] per rank, body length): the first rank whose chain stops writes the raw
     header and its input bytes [stop, hi), later ranks their input [lo, hi) verbatim, the last rank the END
     package.  A raw package of 4 GiB or more cannot be framed (adaptive_compressor.py:617-619)."""
-    from . import _lib as L
     ovh, end = marker_bytes + 14, marker_bytes + 12
-    stop = next((int(st) for _, st in records if st >= 0), -1)
-    if stop >= 0 and n - stop > 0xFFFFFFFF:
-        raise L.AmbcError(L.E_ARG, "raw package over 4 GiB cannot be framed (u32 fields)")
+    refuse_dyn_raw(n, next((int(st) for _, st in records if st >= 0), -1))
     plan, off, raw_seen = [], 0, False
     for r, ((nbytes, st), (lo, hi)) in enumerate(zip(records, ranges)):
         if raw_seen:
@@ -535,13 +555,12 @@ def dyn_fragment(frag, stop, state, t_buf, lo, hi, n, marker, last):
     dev = t_buf.device
     parts = [frag]
     if state == "raw_starts_here":
-        raw = n - stop
-        hdr = marker + bytes([255, 0]) + struct.pack("<III", raw, raw, raw)
-        parts += [torch.tensor(list(hdr), dtype=torch.uint8, device=dev), t_buf[stop - lo:hi - lo]]
+        parts += [torch.tensor(list(raw_package_header(marker, n - stop)), dtype=torch.uint8, device=dev),
+                  t_buf[stop - lo:hi - lo]]
     elif state == "in_raw_tail":
         parts = [t_buf[:hi - lo]]
     if last:
-        parts.append(torch.tensor(list(marker + bytes(12)), dtype=torch.uint8, device=dev))
+        parts.append(torch.tensor(list(end_package(marker)), dtype=torch.uint8, device=dev))
     return torch.cat(parts) if len(parts) > 1 else parts[0]
 
 

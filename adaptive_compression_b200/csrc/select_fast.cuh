@@ -206,6 +206,9 @@ template <int NMAX> __device__ inline void sf_load(SfCtx<NMAX> &c, const uint8_t
 }
 
 // ---- run-boundary bitmap, RLE gate and pair count (compression_methods.py:95-109, 165-180) ---------------
+// bits 0, s, 2 s, ... of a 32-bit word, by s = 1..8
+static __constant__ uint32_t sf_step_mask[9] = {0x00000000u, 0xFFFFFFFFu, 0x55555555u, 0x49249249u, 0x11111111u,
+                                                0x42108421u, 0x41041041u, 0x10204081u, 0x01010101u};
 // bmask bit p = (p == 0 || sd[p] != sd[p-1]).  rep = sampled positions i with sd[i] == sd[i+1].
 // Returns rep (block-wide); *pairs = number of (byte, count) pairs RLE emits -- computed only when the gate holds.
 template <int NMAX> __device__ inline bool sf_rle_features(SfCtx<NMAX> &c, int *pairs_out)
@@ -214,6 +217,13 @@ template <int NMAX> __device__ inline bool sf_rle_features(SfCtx<NMAX> &c, int *
     const int nw = (n + 31) >> 5;
     const int ss = min(1000, n);
     const int step = n < 4 ? 1 : max(1, n / ss);
+    // sampled positions i = 0, step, 2 step, ...: bits 0, step, 2 step, ... of a word (sf_step_mask, step <= 8 for
+    // n <= 8192), shifted to the word's first sample.  Keep this branch-free: the equivalent C++ with a branch per
+    // step value (S = ~0u for step 1, 0x11111111 for step 4, a bit loop otherwise) was mis-compiled by the CUDA 12.9
+    // ptxas for sm_100a -- the `step == 1` branch was taken on the predicate of the VIMNMX that forms
+    // max(1, n / ss), so S was ~0u for every step: rep counted all positions, and k_select_fast<4096> opened the gate
+    // on 2000..4096-byte chunks the reference rejects.
+    const uint32_t Sp = sf_step_mask[step];
     int rep = 0;
     for (int wd = tid; wd < nw; wd += SF_T) {
         const uint4 a = *(const uint4 *)(c.sd + 32 * wd);
@@ -239,14 +249,7 @@ template <int NMAX> __device__ inline bool sf_rle_features(SfCtx<NMAX> &c, int *
         uint32_t eq = ~((mask >> 1) | (nextb << 31));
         const int m1 = min(32, n - 1 - 32 * wd); // positions with a successor
         eq &= m1 >= 32 ? 0xFFFFFFFFu : (m1 <= 0 ? 0u : ((1u << m1) - 1u));
-        uint32_t S;
-        if (step == 1) S = 0xFFFFFFFFu;
-        else if (step == 4) S = 0x11111111u;
-        else {
-            S = 0;
-            int first = (step - (32 * wd) % step) % step;
-            for (int j = first; j < 32; j += step) S |= 1u << j;
-        }
+        const uint32_t S = Sp << ((step - (32 * wd) % step) % step);
         rep += __popc(eq & S);
     }
     rep = sf_block_sum(rep, c.red); // (also publishes bmask)
